@@ -6,6 +6,7 @@
     python bench.py --workload infer                                     # C5: configs[4], predict.py-style inference
     python bench.py --impl reference --gpus N --steps K ...              # reference arm: its CPU fp32 path
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...   # N > 1 (C4 = configs[3])
+    python bench.py ... --dump-outputs DIR                               # + the last timed step's outputs as .npy
 
 train: one step = forward + loss (CE + dice + 0.2*boundary_loss, the train.py:137-147 form) + backward (+ NCCL
 gradient all-reduce when N > 1) + clip_grad_norm_ + RMSprop step (train.py:80,153-159) on 16 synthetic 1x512x512
@@ -66,7 +67,12 @@ def parse():
                     help="torch.optim.RMSprop + clip_grad_norm_ instead of the fused multi-tensor kernels (A/B)")
     ap.add_argument("--graph", default="auto", choices=["auto", "on", "off"],
                     help="replay the whole step as one CUDA graph (auto: try, fall back to eager launches)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32; "
+                         "at most 64 MB in all, larger arrays as a fixed seeded sample) to compare two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.batch is None:
         a.batch = 16 if a.workload == "train" else 8
     if a.size is None:
@@ -113,6 +119,40 @@ def measured_peaks():
         except Exception:  # noqa: BLE001
             pass
     return dict(hbm_gbs=6650.0, tflops_burst=1590.0, tflops_sustained=1400.0, source="fallback")
+
+
+DUMP_BYTES = 64 << 20          # --dump-outputs writes at most this much
+
+
+def step_outputs(a, result, params, buffers):
+    """What a caller of one step receives.  train: the loss, and the parameters, gradients and floating-point
+    buffers (BatchNorm running statistics) the step left behind, each flattened and concatenated in module order;
+    infer: the label map."""
+    if a.workload == "infer":
+        return {"labels": result}
+
+    def flat(ts):
+        return torch.cat([t.detach().float().reshape(-1) for t in ts])
+    return {"loss": result.detach().reshape(1), "params": flat(params),
+            "grads": flat(p.grad for p in params),
+            "buffers": flat(b for b in buffers if b.is_floating_point())}
+
+
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy per array, float64 data as float64 and everything else as float32.  An array larger than an
+    even share of DUMP_BYTES is replaced by a sample of its flattened elements at fixed, seeded indices (the same for
+    every run with the same arguments)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        cap = share // t.element_size()
+        if t.numel() > cap:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, f"{name}.npy"), t.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------
@@ -216,10 +256,16 @@ class ReferenceStep:
     def step(self, img, msk):
         return self.train_step(img, msk) if self.a.workload == "train" else self.infer_step(img)
 
+    def buffers(self):
+        if self.model is not None:
+            return list(self.model.buffers())
+        return [v for k, v in self.state.items() if k not in self.names]
 
-def cpu_reference_rate(a, steps, warmup, budget_s, batch):
+
+def cpu_reference_rate(a, steps, warmup, budget_s, batch, dump=None):
     """img/s of the reference's CPU fp32 step, all host threads; `batch` images per step (a bounded sample of the
-    workload), at most `budget_s` seconds, at least one timed step."""
+    workload), at most `budget_s` seconds, at least one timed step.  `dump`: a directory for the outputs of the last
+    timed step (--dump-outputs)."""
     torch.set_num_threads(os.cpu_count() or 1)
     ref = ReferenceStep(a, "cpu", amp=False)
     img, msk = synthetic(a, 0, batch)
@@ -227,7 +273,7 @@ def cpu_reference_rate(a, steps, warmup, budget_s, batch):
     t_start = time.perf_counter()
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        ref.step(img, msk)
+        out = ref.step(img, msk)
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
@@ -240,6 +286,8 @@ def cpu_reference_rate(a, steps, warmup, budget_s, batch):
             warmup = done_warm                   # cut the warm-up short: keep at least one timed step
     if not times:
         times = [dt]
+    if dump:
+        dump_outputs(dump, step_outputs(a, out, ref.params, ref.buffers()))
     med = statistics.median(times)
     return batch / med, len(times), done_warm, med, ref.kind
 
@@ -248,12 +296,14 @@ def run_reference(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # one timed step = a bounded sample of the workload: 2 images.  Measured on the GPU box's 16 host cores
+    # one timed step = a bounded sample of the workload: 2 images.  Measured on the 16 host cores of a B200 machine
     # (profiles/r2_bench_reference_b16.json): 2 images take 1.44 s/step (1.39 img/s), but the full batch of 16 took
     # 596 s for ONE step (0.027 img/s: the fp32 activations + autograd state of B=16 at 512x512 no longer fit the
-    # box's memory comfortably), so the full batch would neither finish the driver's --steps 20 nor flatter the CPU.
+    # host's memory comfortably), so the full batch would neither finish a run of 20 steps nor flatter the CPU.
+    # --steps sets the number of timed steps exactly: no time budget here.
     batch = min(a.batch, 2)
-    rate, n, nw, med, kind = cpu_reference_rate(a, a.steps, min(a.warmup, 1), budget_s=170.0, batch=batch)
+    rate, n, nw, med, kind = cpu_reference_rate(a, a.steps, min(a.warmup, 1), budget_s=float("inf"), batch=batch,
+                                                dump=a.dump_outputs)
     cores = os.cpu_count() or 1
     src = ("unmodified reference modules (baseline/_ref: unet, utils.dice_score, utils.boundary_loss)" if kind == "reference"
            else "oracle port of the reference step (torch-CPU fp32 restatement; baseline/_ref did not travel)")
@@ -658,8 +708,15 @@ def bench_train(ctx):
             step(img_d, msk_d)
     _sync_all(ctx)
     sampler = ClockSampler(ctx["local"]) if rank == 0 else None
-    ms = _timed(ctx, lambda: step(img_d, msk_d), a.steps)
+    last = [None]
+
+    def timed_step():
+        last[0] = step(img_d, msk_d)
+    ms = _timed(ctx, timed_step, a.steps)
     clocks = sampler.stop() if sampler else {}
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, step_outputs(a, last[0], list(model.parameters()), list(model.buffers())))
+    last[0] = None                  # a live loss keeps its autograd graph alive (see the warm-up above)
     e2e_steps(2)
     ms_e2e = _timed(ctx, lambda: e2e_steps(a.steps), 1)
     last_loss = float(step(img_d, msk_d).detach())
@@ -740,8 +797,14 @@ def bench_infer(ctx):
         run()
     _sync_all(ctx)
     sampler = ClockSampler(ctx["local"]) if rank == 0 else None
-    ms = _timed(ctx, run, a.steps)
+    last = [None]
+
+    def timed_step():
+        last[0] = run()
+    ms = _timed(ctx, timed_step, a.steps)
     clocks = sampler.stop() if sampler else {}
+    if a.dump_outputs and rank == 0:             # a graph replay returns nothing: its label map is static_out
+        dump_outputs(a.dump_outputs, step_outputs(a, static_out if replay is not None else last[0], None, None))
 
     # end to end through the reference-facing call: predict_img(model, host images, device) -> label map on the host
     copy_stream = torch.cuda.Stream(device=dev)

@@ -1,9 +1,9 @@
-"""Generate tests/golden/*.pt by running the UNMODIFIED reference (imported read-only from
-/root/reference) on seeded synthetic inputs.  Run in the build container only:
+"""Generate tests/golden/*.pt by running the UNMODIFIED reference (imported read-only from the checkout that
+UNETB200_REFERENCE_DIR names) on seeded synthetic inputs:
 
-    python tests/golden/make_golden.py
+    UNETB200_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden.py
 
-The GPU box has no /root/reference; tests read the committed fixtures instead.  The script also
+The tests read the committed fixtures and never need the reference.  The script also
 asserts, bit for bit, that oracle.build_state() draws the same weights as the reference
 constructor, and that the oracle reproduces every fixture it writes (so a fixture can never be
 committed that the oracle disagrees with).
@@ -16,7 +16,7 @@ import torch
 import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = "/root/reference"
+REF = os.environ.get("UNETB200_REFERENCE_DIR") or sys.exit("set UNETB200_REFERENCE_DIR to a checkout of the reference")
 sys.path.insert(0, ROOT)
 
 # import the reference's own modules under private names so they cannot shadow anything

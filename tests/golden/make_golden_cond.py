@@ -1,13 +1,13 @@
 """Pin oracle.conditioned_state / structured_batch / Rounding against the UNMODIFIED reference.
 
-    python tests/golden/make_golden_cond.py          (build container only: needs /root/reference)
+    UNETB200_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden_cond.py
 
 The reference's own ``UNet`` module is trained for the same number of steps with ``torch.optim.RMSprop`` on the same
 structured batch; the script asserts the oracle's recipe lands on the same state BIT FOR BIT (the recipe restates the
 optimizer's single-tensor update op for op: the trajectory is chaotic, a one-ulp difference grows to 1e-1 in ten
 steps), then commits a small fingerprint (``golden_cond_v1.pt``: per-tensor sums of the conditioned state, logits
 samples, loss, accuracy and gradient norms of one further step on a fresh batch) that ``tests/test_oracle_cond.py``
-re-checks on every run without /root/reference.
+re-checks on every run without the reference.
 """
 import os
 import sys

@@ -1,7 +1,7 @@
 """Generate tests/golden/golden_io_v1.pt by running the UNMODIFIED reference code either side of the
-UNet step (SURVEY.md section 8(f) N1, N3) on seeded synthetic bytes.  Build container only:
+UNet step (SURVEY.md section 8(f) N1, N3) on seeded synthetic bytes:
 
-    python tests/golden/make_golden_io.py
+    UNETB200_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden_io.py
 
   * utils/data_loading.py: BasicDataset.preprocess + rotate_image_and_mask (through PIL, as __getitem__ does)
   * utils/dice_score.py:   dice_coeff, applied to the literal tail expressions of evaluate.py:56-66,111-117
@@ -19,7 +19,7 @@ import torch.nn.functional as F
 from PIL import Image
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-REF = "/root/reference"
+REF = os.environ.get("UNETB200_REFERENCE_DIR") or sys.exit("set UNETB200_REFERENCE_DIR to a checkout of the reference")
 sys.path.insert(0, ROOT)
 
 
@@ -106,6 +106,12 @@ def main():
         assert agree >= (1.0 if tag.startswith("same") else 0.999), tag
         G["predict"].append(dict(tag=tag, logits=logits, size=(H, W), idx=idx))
 
+    for cases in G.values():                    # label maps (values < 256) as uint8: the loaders widen them to int64
+        for c in cases:
+            for k in ("out_msk", "idx"):
+                if k in c:
+                    assert 0 <= int(c[k].min()) and int(c[k].max()) < 256, (c["tag"], k)
+                    c[k] = c[k].to(torch.uint8)
     out = os.path.join(ROOT, "tests", "golden", "golden_io_v1.pt")
     torch.save(G, out)
     print("wrote", out, os.path.getsize(out), "bytes")

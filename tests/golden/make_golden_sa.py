@@ -1,13 +1,13 @@
 """Pin the oracle's SpatialAttention / UNet_SA restatement against the UNMODIFIED reference.
 
-    python tests/golden/make_golden_sa.py          (build container only: needs /root/reference)
+    UNETB200_REFERENCE_DIR=<reference checkout> python tests/golden/make_golden_sa.py
 
 Builds the reference's ``UNet_SA`` (unet_model.py:140-189; ``Up(..., use_attention=True)``, unet_parts.py:62-98 with the
 ``SpatialAttention`` gate of :39-60) under a fixed seed, runs one training step (CE + dice, train.py:137-142) on the
 oracle's synthetic batch, asserts the oracle agrees (its ``up`` applies the gate exactly when the state holds the 7x7
 weight), and commits ``golden_sa_v1.pt``: per-tensor sums of the seeded state, logits, loss, gradient norms and samples, plus one
 stand-alone gate case (x * attention(x) forward / backward) -- re-checked by tests/test_oracle_sa.py without
-/root/reference and used by the -m gpu gate of the CUDA kernels.
+the reference and used by the -m gpu gate of the CUDA kernels.
 """
 import os
 import sys

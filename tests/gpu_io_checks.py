@@ -24,7 +24,15 @@ DEV = "cuda"
 
 
 def load_golden_io():
-    return torch.load(os.path.join(ROOT, "tests", "golden", "golden_io_v1.pt"), weights_only=False)
+    """The label maps (`out_msk`, `idx`) are stored as uint8 to keep the file small; they are int64 in the reference
+    and are widened back here."""
+    g = torch.load(os.path.join(ROOT, "tests", "golden", "golden_io_v1.pt"), weights_only=False)
+    for cases in g.values():
+        for c in cases:
+            for k in ("out_msk", "idx"):
+                if k in c:
+                    c[k] = c[k].long()
+    return g
 
 
 def ndiff(a, b):

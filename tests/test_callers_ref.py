@@ -1,6 +1,7 @@
 """-m gpu: the reference's own train.py / evaluate.py / predict.py, UNMODIFIED (baseline/_ref, staged by
 __graft_entry__.build()), run on the drop-in modules and -- same files, same seeds, same data -- on stock PyTorch.
-See tests/callers_ref_worker.py.  Skipped when the reference copy did not travel with the snapshot."""
+See tests/callers_ref_worker.py.  Those scripts are not part of this repository: the test skips unless build() ran with
+UNETB200_REFERENCE_DIR naming a checkout of the reference, which stages them under baseline/_ref."""
 import json
 import os
 import subprocess
@@ -26,7 +27,8 @@ def _run(mode, tmp):
         return json.load(f), np.load(out + ".mask.npy")
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "train.py")), reason="baseline/_ref not staged")
+@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "train.py")),
+                    reason="needs the reference's own scripts in baseline/_ref (build() with UNETB200_REFERENCE_DIR set)")
 def test_reference_callers_run_unchanged_on_the_dropin(tmp_path):
     ours, mask_o = _run("dropin", str(tmp_path))
     ref, mask_r = _run("stock", str(tmp_path))

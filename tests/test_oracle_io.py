@@ -1,6 +1,6 @@
 """CPU: oracle/io_oracle.py (input pipeline, evaluate / predict tails) against the fixtures generated from the
 reference itself by tests/golden/make_golden_io.py, plus the host-side argument logic of unetb200.data /
-unetb200.eval_tail.  No access to /root/reference, no compute calls into the CUDA library."""
+unetb200.eval_tail.  Never needs the reference, no compute calls into the CUDA library."""
 import os
 
 import numpy as np
@@ -14,7 +14,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 @pytest.fixture(scope="module")
 def gio():
-    return torch.load(os.path.join(ROOT, "tests", "golden", "golden_io_v1.pt"), weights_only=False)
+    from gpu_io_checks import load_golden_io
+    return load_golden_io()
 
 
 def test_pipeline_matches_reference_arrays(gio):
