@@ -248,6 +248,45 @@ int unetb200_bn_relu_bwd_apply(const void* gz, int64_t ld_gz, const void* y, int
                                int dtype, int B, int H, int W, int C, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * nn.SyncBatchNorm: BatchNorm statistics synchronised over the GPUs of one node (2..16 ranks).
+ * ------------------------------------------------------------------------------------------- */
+/* A peer group is the exception to "the caller owns memory" (like an NCCL communicator): the library
+ * allocates each rank's exchange buffer, exports it with CUDA IPC and maps every peer's buffer; the
+ * exchange kernels move data between GPUs by stores only.  Setup, per rank, on the group's device:
+ *   1. unetb200_bn_peer_group_create -> ipc_handle (UNETB200_IPC_HANDLE_BYTES) and the PCI bus id
+ *      (UNETB200_BUS_ID_BYTES, NUL-terminated) of this rank's buffer;
+ *   2. the caller gathers every rank's handle and bus id (rank order, concatenated);
+ *   3. unetb200_bn_peer_group_open checks cudaDeviceCanAccessPeer for every peer and maps its
+ *      buffer; UNETB200_E_INVALID when a peer's GPU is not visible or not reachable by peer access.
+ * destroy frees this rank's side; call it only after every rank's last exchange has completed
+ * (device synchronise + a barrier of the group).  Exchanges of one group must be stream-ordered
+ * (one stream at a time) and every rank must issue them in the same order. */
+#define UNETB200_IPC_HANDLE_BYTES 64
+#define UNETB200_BUS_ID_BYTES 32
+typedef struct unetb200_bn_peer_group_s unetb200_bn_peer_group_t;
+int unetb200_bn_peer_group_create(int rank, int world, int max_channels, void* ipc_handle, char* bus_id,
+                                  unetb200_bn_peer_group_t** out);
+int unetb200_bn_peer_group_open(unetb200_bn_peer_group_t* g, const void* ipc_handles, const char* bus_ids);
+int unetb200_bn_peer_group_destroy(unetb200_bn_peer_group_t* g);
+/* Host read of the group's timeout word: *missing_rank = -1 while no exchange has timed out, else the
+ * rank whose contribution an exchange waited for in vain (30 s, %globaltimer) and *epoch = that
+ * exchange's epoch.  A timed-out exchange writes no outputs; the group is then unusable. */
+int unetb200_bn_peer_group_status(const unetb200_bn_peer_group_t* g, int64_t* missing_rank, int64_t* epoch);
+/* unetb200_bn_finalize_track on the GLOBAL statistics: one single-CTA launch pushes this rank's
+ * stats[2*C] and `count` to every rank, waits for all of theirs, sums them in rank order in fp64
+ * (bit-identical results on every rank: coefficients, running statistics with the unbiased variance
+ * over the global count) and finalizes. */
+int unetb200_bn_sync_finalize(unetb200_bn_peer_group_t* g, const double* stats, int64_t count,
+                              const float* gamma, const float* beta, float eps, float momentum,
+                              float* running_mean, float* running_var, float* save_mean,
+                              float* save_invstd, float* scale, float* shift,
+                              int64_t* num_batches_tracked, int C, void* stream);
+/* unetb200_bn_bwd_finalize (training) with coef = GLOBAL sums / GLOBAL count; dgamma = sums[1] and
+ * dbeta = sums[0] stay this rank's own (the data-parallel gradient mean averages them). */
+int unetb200_bn_sync_bwd_finalize(unetb200_bn_peer_group_t* g, const double* sums, int64_t count,
+                                  float* dgamma, float* dbeta, float* coef, int C, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * nn.Upsample(scale_factor=2, mode='bilinear', align_corners=True) -- unet_parts.py:70, and the
  * F.pad placement of unet_parts.py:85-88 (output written at (off_y, off_x) of an Hout x Wout grid).
  * ------------------------------------------------------------------------------------------- */

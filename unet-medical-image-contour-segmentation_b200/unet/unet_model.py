@@ -44,12 +44,20 @@ class _UNetBase(nn.Module):
 
     def forward(self, x):
         from unetb200 import functional as UF
-        if self._bn_doubles is None:           # 2 C fp64 accumulators (sum, sum of squares) per BatchNorm layer
-            self._bn_doubles = sum(2 * ((m.num_features + 1) // 2 * 2) for m in self.modules() if isinstance(m, nn.BatchNorm2d))
+        if self._bn_doubles is None:
+            from unetb200 import ddp
+            ddp.sync_bn_process_group(self, self.training)      # raises for mixed process groups
+            self._bn_doubles = self.bn_arena_doubles()
         with UF.zero_arena(self._bn_doubles if self.training else 0, x.device):
             return self._forward(x)
 
     _bn_doubles = None
+
+    def bn_arena_doubles(self):
+        """Size of the fp64 statistics arena of a training forward: 2 C accumulators (sum, sum of squares) per
+        BatchNorm holder -- BatchNorm2d, or the nn.SyncBatchNorm that convert_sync_batchnorm puts in its place."""
+        return sum(2 * ((m.num_features + 1) // 2 * 2) for m in self.modules()
+                   if isinstance(m, nn.modules.batchnorm._BatchNorm))
 
     def _forward(self, x):
         x = _prep(x, type(self).__name__)

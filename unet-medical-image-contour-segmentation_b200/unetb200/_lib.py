@@ -81,6 +81,13 @@ PROTOTYPES = {
     "unetb200_bn_relu_bwd_reduce": (C.c_int, [c_p, c_i64, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_p]),
     "unetb200_bn_bwd_finalize": (C.c_int, [c_p, c_i64, C.c_int, c_p, c_p, c_p, C.c_int, c_p]),
     "unetb200_bn_relu_bwd_apply": (C.c_int, [c_p, c_i64, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_p, c_i64, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_p]),
+    "unetb200_bn_peer_group_create": (C.c_int, [C.c_int, C.c_int, C.c_int, c_p, c_p, C.POINTER(c_p)]),
+    "unetb200_bn_peer_group_open": (C.c_int, [c_p, c_p, c_p]),
+    "unetb200_bn_peer_group_destroy": (C.c_int, [c_p]),
+    "unetb200_bn_peer_group_status": (C.c_int, [c_p, C.POINTER(c_i64), C.POINTER(c_i64)]),
+    "unetb200_bn_sync_finalize": (C.c_int, [c_p, c_p, c_i64, c_p, c_p, C.c_float, C.c_float, c_p, c_p, c_p, c_p, c_p, c_p,
+                                            c_p, C.c_int, c_p]),
+    "unetb200_bn_sync_bwd_finalize": (C.c_int, [c_p, c_p, c_i64, c_p, c_p, c_p, C.c_int, c_p]),
     "unetb200_upsample2x_fwd": (C.c_int, [c_p, c_i64, c_p, c_i64, C.c_int] + [C.c_int] * 8 + [c_p]),
     "unetb200_upsample2x_bwd": (C.c_int, [c_p, c_i64, c_p, c_i64, C.c_int] + [C.c_int] * 8 + [c_p]),
     "unetb200_gather_nhwc": (C.c_int, [c_p, C.c_int, c_i64, c_i64, c_i64, c_i64, c_p, C.c_int, c_i64, C.c_int, C.c_int, C.c_int, C.c_int, c_p]),

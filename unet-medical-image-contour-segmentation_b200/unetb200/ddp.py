@@ -63,6 +63,121 @@ def sync_buffers(module, src=0):
             dist.broadcast(t.data, src=src)
 
 
+# ------------------------------------------------------------------------------------------------
+# synchronised BatchNorm (nn.SyncBatchNorm holders): statistics exchanged over NVLink by kernel stores
+# ------------------------------------------------------------------------------------------------
+SYNC_BN_MAX_CHANNELS = 4096        # exchange-buffer capacity per layer (UNet's widest layer has 1024 channels)
+_PEER_GROUPS = {}                  # (device index, process group) -> BNPeerGroup
+
+
+def sync_bn_process_group(module, training=False):
+    """(number of nn.SyncBatchNorm layers in `module`, the process group they name: None = WORLD).  Raises ValueError
+    when they name different groups (one peer group serves a model), and for training when one of them has
+    momentum=None (as the forward pass of such a layer does)."""
+    layers = [m for m in module.modules() if isinstance(m, torch.nn.SyncBatchNorm)]
+    groups = {id(m.process_group): m.process_group for m in layers}
+    if len(groups) > 1:
+        raise ValueError("unetb200: the SyncBatchNorm layers of one model must all name the same process group")
+    if training and any(m.momentum is None for m in layers):
+        raise ValueError("unetb200: SyncBatchNorm(momentum=None) (cumulative average) is not supported")
+    return len(layers), (next(iter(groups.values())) if groups else None)
+
+
+def bn_sync_group(bn, device):
+    """The BNPeerGroup a training-mode BatchNorm holder synchronises over, or None when it normalises with its own
+    batch: not an nn.SyncBatchNorm, torch.distributed not initialised, or a group of one rank (torch's rule).
+    Creates the peer group on first use (a collective of the group: every rank's first synchronised forward)."""
+    if not isinstance(bn, torch.nn.SyncBatchNorm) or not (dist.is_available() and dist.is_initialized()):
+        return None
+    group = bn.process_group if bn.process_group is not None else dist.group.WORLD
+    key = (device.index, group)
+    pg = _PEER_GROUPS.get(key)
+    if pg is not None:
+        return pg
+    if dist.get_world_size(group) <= 1:
+        return None
+    if torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("unetb200: the first synchronised BatchNorm forward must run eagerly (it sets up the "
+                           "NVLink peer group, a collective): run one step before capturing a CUDA graph "
+                           "(SegmentedStep's warm-up does)")
+    pg = _PEER_GROUPS[key] = BNPeerGroup(group, device)
+    return pg
+
+
+class BNPeerGroup:
+    """The ranks of one process group on one device, with their mapped exchange buffers (libunetb200's
+    unetb200_bn_peer_group_t).  Created by bn_sync_group, torn down by destroy_peer_groups."""
+
+    def __init__(self, group, device, max_channels=SYNC_BN_MAX_CHANNELS):
+        import ctypes as C
+
+        from . import _lib
+        L = _lib.load()
+        self.group, self.device = group, device
+        self.rank, self.world = dist.get_rank(group), dist.get_world_size(group)
+        handle, bus = C.create_string_buffer(64), C.create_string_buffer(32)
+        h = C.c_void_p()
+        with torch.cuda.device(device):
+            _lib.check(L.unetb200_bn_peer_group_create(self.rank, self.world, max_channels, handle, bus, C.byref(h)),
+                       "bn_peer_group_create")
+            self.handle = h
+            try:
+                parts = [None] * self.world
+                dist.all_gather_object(parts, (handle.raw, bus.raw), group=group)
+                rc = L.unetb200_bn_peer_group_open(h, b"".join(p[0] for p in parts), b"".join(p[1] for p in parts))
+                msg = L.unetb200_last_error().decode("utf-8", "replace") if rc else ""
+                status = [None] * self.world           # every rank learns whether every rank could map its peers
+                dist.all_gather_object(status, (rc, msg), group=group)
+            except BaseException:
+                L.unetb200_bn_peer_group_destroy(h)
+                raise
+        bad = [f"rank {r}: {m}" for r, (rc, m) in enumerate(status) if rc != 0]
+        if bad:
+            L.unetb200_bn_peer_group_destroy(h)
+            self.handle = None
+            raise RuntimeError("unetb200: SyncBatchNorm needs every pair of ranks to reach each other by CUDA peer "
+                               "access (one node): " + "; ".join(bad))
+
+    def check(self):
+        """Raise if an exchange of this group has timed out (a rank stopped taking part)."""
+        import ctypes as C
+
+        from . import _lib
+        if self.handle is None:
+            raise RuntimeError("unetb200: SyncBatchNorm peer group used after destroy_peer_groups()")
+        missing, epoch = C.c_int64(), C.c_int64()
+        _lib.check(_lib.load().unetb200_bn_peer_group_status(self.handle, C.byref(missing), C.byref(epoch)),
+                   "bn_peer_group_status")
+        if missing.value >= 0:
+            raise RuntimeError(f"unetb200: SyncBatchNorm exchange {epoch.value} on rank {self.rank} timed out waiting "
+                               f"for rank {missing.value}; the peer group is unusable (destroy_peer_groups())")
+
+    def destroy(self):
+        from . import _lib
+        if self.handle is None:
+            return
+        with torch.cuda.device(self.device):
+            torch.cuda.synchronize()
+            if dist.is_initialized():
+                dist.barrier(group=self.group)          # no rank still writes into this rank's buffer
+            _lib.load().unetb200_bn_peer_group_destroy(self.handle)
+        self.handle = None
+
+
+def destroy_peer_groups():
+    """Tear down every SyncBatchNorm peer group of this process: a collective of each group, to be called by every
+    rank before dist.destroy_process_group()."""
+    for key in list(_PEER_GROUPS):
+        _PEER_GROUPS.pop(key).destroy()
+
+
+def check_peer_groups():
+    """Raise if an exchange of any SyncBatchNorm peer group has timed out (for graph replays, which have no Python
+    entry per exchange)."""
+    for pg in _PEER_GROUPS.values():
+        pg.check()
+
+
 class GradAllReducer:
     """Bucketed, backward-overlapped mean all-reduce of ``module``'s gradients.
 
@@ -361,6 +476,7 @@ class SegmentedStep:
             s.copy_(a, non_blocking=True)
 
     def replay(self):
+        check_peer_groups()
         self.g_fwd.replay()
         for k, g in enumerate(self.g_bwd):
             g.replay()

@@ -363,8 +363,20 @@ def _eval_coefs(bn, Cout):
     return coefs
 
 
-def conv_bn_relu_fwd(x, w, bn, training, out=None, want_pool=False, fold=False, outconv=None):
+def sync_peer(bn, training, device):
+    """The ddp.BNPeerGroup whose ranks a training-mode nn.SyncBatchNorm holder takes its statistics from, or None:
+    BatchNorm2d holders, eval mode, and SyncBatchNorm without torch.distributed or in a group of one rank run the
+    per-replica path unchanged (no extra launch)."""
+    if not training or not isinstance(bn, torch.nn.SyncBatchNorm):
+        return None
+    from . import ddp
+    return ddp.bn_sync_group(bn, device)
+
+
+def conv_bn_relu_fwd(x, w, bn, training, out=None, want_pool=False, fold=False, outconv=None, peer=None):
     """x NHWC -> (y raw conv output, z = relu(bn(y)), pooled or None, coefs[4,C]).
+
+    peer: the BNPeerGroup of a synchronised BatchNorm (sync_peer): the batch statistics are those of every rank.
 
     outconv = (weight [K, C, 1, 1], bias or None) with fold=True: when the fused kernel covers the shape, z is the
     LOGITS of OutConv applied to the activation ([B, K, H, W] view of a packed NHWC tensor) and the 5th return value
@@ -408,11 +420,15 @@ def conv_bn_relu_fwd(x, w, bn, training, out=None, want_pool=False, fold=False, 
     beta = _f32c(bn.bias) if bn.bias is not None else None
     if use_batch:
         if bn.momentum is None and bn.running_mean is not None and training:
-            raise ValueError("unetb200: BatchNorm2d(momentum=None) (cumulative average) is not supported")
+            raise ValueError(f"unetb200: {type(bn).__name__}(momentum=None) (cumulative average) is not supported")
         update = training and bn.running_mean is not None and not _RECOMPUTE[0]
-        coefs = ops.bn_finalize(stats, B * H * W, gamma, beta, bn.eps, bn.momentum if update else 0.0,
-                                bn.running_mean if update else None, bn.running_var if update else None, Cout,
-                                num_batches_tracked=bn.num_batches_tracked if update else None)
+        args = (stats, B * H * W, gamma, beta, bn.eps, bn.momentum if update else 0.0,
+                bn.running_mean if update else None, bn.running_var if update else None, Cout)
+        nbt = bn.num_batches_tracked if update else None
+        if peer is None:
+            coefs = ops.bn_finalize(*args, num_batches_tracked=nbt)
+        else:
+            coefs = ops.bn_sync_finalize(peer, *args, num_batches_tracked=nbt)
         if update:
             # the kernel moved the running statistics through raw pointers: tell PyTorch (autograd's saved-tensor
             # check, the eval-coefficient cache above)
@@ -456,18 +472,18 @@ def _vec_dst(param, Cc):
 
 
 def conv_bn_relu_bwd(gz, x, y, w, coefs, batch_stats, need_gx, param=None, bn_params=(None, None), sums=None,
-                     below=None, colsum=None):
+                     below=None, colsum=None, peer=None):
     """-> (gx or None, dW [Co,Ci,3,3] fp32, dgamma, dbeta, sums_below).  `param`: the Parameter object behind `w`;
     `bn_params`: the BatchNorm weight / bias Parameter objects (only to look up their gradient sinks); `sums`: the
     BatchNorm-backward reduction of THIS stage if the kernel that produced gz already made it; `below` = (y, coefs)
     of the conv-BN-ReLU stage whose activation is `x`: its reduction is then made by this stage's dgrad epilogue
-    when the fused kernel covers the shape and returned as sums_below (else None)."""
+    when the fused kernel covers the shape and returned as sums_below (else None).  `peer`: as conv_bn_relu_fwd."""
     param = w if param is None else param
     B, Cin, H, W = x.shape
     Cout = w.shape[0]
     cd = x.dtype
     gy, dgamma, dbeta = ops.bn_relu_bwd(gz, y, coefs, batch_stats, _vec_dst(bn_params[0], Cout),
-                                        _vec_dst(bn_params[1], Cout), sums=sums)
+                                        _vec_dst(bn_params[1], Cout), sums=sums, peer=peer)
     # the gradient takes the parameter's own memory layout (OIHW or channels_last): AccumulateGrad then keeps it
     # without a copy, and for channels_last the split reduction writes it coalesced; with a registered sink
     # (data-parallel bucket view) it is written there
@@ -554,10 +570,12 @@ class DoubleConvFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, w1, g1, b1, w2, g2, b2, cfg):
         fold = not cfg.save
-        y1, z1, _, c1, _ = conv_bn_relu_fwd(x, w1, cfg.bn1, cfg.training, fold=fold)
+        ctx.peers = (sync_peer(cfg.bn1, cfg.training, x.device), sync_peer(cfg.bn2, cfg.training, x.device))
+        y1, z1, _, c1, _ = conv_bn_relu_fwd(x, w1, cfg.bn1, cfg.training, fold=fold, peer=ctx.peers[0])
         y2, z2, pooled, c2, fused_out = conv_bn_relu_fwd(z1, w2, cfg.bn2, cfg.training, out=cfg.out,
                                                          want_pool=cfg.want_pool, fold=fold,
-                                                         outconv=getattr(cfg, "outconv", None) if fold else None)
+                                                         outconv=getattr(cfg, "outconv", None) if fold else None,
+                                                         peer=ctx.peers[1])
         cfg.fused_outconv = fused_out          # tells the caller whether z2 already holds OutConv's logits
         ctx.batch_stats = (cfg.training or cfg.bn1.running_mean is None, cfg.training or cfg.bn2.running_mean is None)
         ctx.has_pool = pooled is not None
@@ -604,9 +622,10 @@ class DoubleConvFn(torch.autograd.Function):
         p1, pg1, pb1, p2, pg2, pb2 = getattr(ctx, "param_objs", (w1, None, None, w2, None, None))
         # conv2's dgrad output is the gradient of z1 = relu(bn1(y1)): its epilogue makes bn1's backward reduction
         gz1, dW2, dg2, db2, sums1 = conv_bn_relu_bwd(gz, z1, y2, w2, c2, ctx.batch_stats[1], True, param=p2,
-                                                     bn_params=(pg2, pb2), below=(y1, c1), sums=sums2)
+                                                     bn_params=(pg2, pb2), below=(y1, c1), sums=sums2,
+                                                     peer=ctx.peers[1])
         gx, dW1, dg1, db1, _ = conv_bn_relu_bwd(gz1, x, y1, w1, c1, ctx.batch_stats[0], need[0], param=p1,
-                                                bn_params=(pg1, pb1), sums=sums1, colsum=ctx.colsum)
+                                                bn_params=(pg1, pb1), sums=sums1, colsum=ctx.colsum, peer=ctx.peers[0])
         return (gx, dW1 if need[1] else None, dg1 if need[2] else None, db1 if need[3] else None,
                 dW2 if need[4] else None, dg2 if need[5] else None, db2 if need[6] else None, None)
 

@@ -583,6 +583,30 @@ def bn_finalize(stats, count, gamma, beta, eps, momentum, running_mean, running_
     return coefs
 
 
+def bn_sync_finalize(peer, stats, count, gamma, beta, eps, momentum, running_mean, running_var, Cc,
+                     num_batches_tracked=None):
+    """bn_finalize on the statistics of every rank of `peer` (a ddp.BNPeerGroup): one single-CTA exchange launch."""
+    peer.check()
+    coefs = torch.empty((4, Cc), dtype=torch.float32, device=stats.device)
+    nbt = num_batches_tracked
+    if nbt is not None and not (nbt.dtype == torch.int64 and nbt.is_cuda and nbt.numel() == 1):
+        nbt.add_(1)
+        nbt = None
+    _run("bn_sync_finalize", lib().unetb200_bn_sync_finalize, peer.handle, _p(stats), count, _p(gamma), _p(beta), eps,
+         momentum, _p(running_mean), _p(running_var), _prow(coefs, 0), _prow(coefs, 1), _prow(coefs, 2),
+         _prow(coefs, 3), _p(nbt), Cc, _stream())
+    if nbt is not None:
+        torch._C._increment_version([nbt])
+    return coefs
+
+
+def bn_sync_bwd_finalize(peer, sums, count, dgamma, dbeta, coef):
+    """bn_bwd_finalize (training) with the coefficients from the sums of every rank of `peer`; dgamma / dbeta local."""
+    peer.check()
+    _run("bn_sync_bwd_finalize", lib().unetb200_bn_sync_bwd_finalize, peer.handle, _p(sums), count, _p(dgamma),
+         _p(dbeta), _p(coef), coef.shape[1], _stream())
+
+
 def bn_eval_coeffs(gamma, beta, running_mean, running_var, eps, Cc):
     coefs = torch.empty((4, Cc), dtype=torch.float32, device=running_mean.device)
     _run("bn_eval_coeffs", lib().unetb200_bn_eval_coeffs, _p(gamma), _p(beta), _p(running_mean), _p(running_var),
@@ -629,9 +653,10 @@ def maxpool2_bwd_bnreduce(x, gp, gx, y, coefs):
     return sums
 
 
-def bn_relu_bwd(gz, y, coefs, training, dgamma=None, dbeta=None, sums=None):
+def bn_relu_bwd(gz, y, coefs, training, dgamma=None, dbeta=None, sums=None, peer=None):
     """Returns (gy, dgamma, dbeta) for z = relu(bn(y)); `dgamma` / `dbeta`: optional fp32 [C] destinations; `sums`:
-    the fp64 [2, C] reduction when the kernel that produced gz already made it (gconv_dgrad_bnbwd)."""
+    the fp64 [2, C] reduction when the kernel that produced gz already made it (gconv_dgrad_bnbwd); `peer`: the
+    ddp.BNPeerGroup of a synchronised BatchNorm (its coefficients then come from the sums of every rank)."""
     B, Cc, H, W = y.shape
     dev = y.device
     es = y.element_size()
@@ -646,8 +671,11 @@ def bn_relu_bwd(gz, y, coefs, training, dgamma=None, dbeta=None, sums=None):
     if dbeta is None:
         dbeta = torch.empty(Cc, dtype=torch.float32, device=dev)
     coef = torch.empty((2, Cc), dtype=torch.float32, device=dev)
-    _run("bn_bwd_finalize", L.unetb200_bn_bwd_finalize, _p(sums), B * H * W, 1 if training else 0, _p(dgamma),
-         _p(dbeta), _p(coef), Cc, _stream())
+    if peer is not None:
+        bn_sync_bwd_finalize(peer, sums, B * H * W, dgamma, dbeta, coef)
+    else:
+        _run("bn_bwd_finalize", L.unetb200_bn_bwd_finalize, _p(sums), B * H * W, 1 if training else 0, _p(dgamma),
+             _p(dbeta), _p(coef), Cc, _stream())
     gy = empty_nhwc(B, Cc, H, W, y.dtype, dev)
     _run("bn_relu_bwd_apply", L.unetb200_bn_relu_bwd_apply, _p(gz), nhwc_ld(gz), _p(y), nhwc_ld(y), _prow(coefs, 2),
          _prow(coefs, 3), _prow(coefs, 0), _prow(coefs, 1), _p(coef), _p(gy), nhwc_ld(gy), dt(y), B, H, W, Cc, _stream(),
