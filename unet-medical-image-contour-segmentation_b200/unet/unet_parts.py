@@ -27,6 +27,7 @@ def _to_internal(x, dtype):
 def _prep(x, what):
     """Caller tensor (fp32 NCHW-logical, usually channels_last) -> NHWC of the compute dtype."""
     ops.require_cuda(x, what)
+    UF.begin_forward()
     if x.dim() != 4:
         raise ValueError(f"{what}: expected a [B, C, H, W] tensor, got {tuple(x.shape)}")
     return _to_internal(x, UF.compute_dtype(x))

@@ -406,6 +406,9 @@ class SegmentedStep:
 
     def __init__(self, model, fwd_loss, clip_and_step, example_inputs, warmup=2, group=None):
         self.model = model
+        # the captured graphs write into whatever these close over (an optimizer's state, a step counter): keep them
+        # alive as long as the graphs
+        self.fwd_loss, self.clip_and_step = fwd_loss, clip_and_step
         self.params_by_segment = segment_params(model)
         self.reducer = GradAllReducer(model, group=group, groups=self.params_by_segment, sinks_always=True)
         self.reducer.manual = True
@@ -440,12 +443,21 @@ class SegmentedStep:
         pool = self.g_fwd.pool()
         self.g_bwd = []
         state = {}
+        views = {id(p): v for b in self.reducer.buckets for p, v in zip(b["params"], b["views"])}
+        self.grad_copies = 0           # gradients a kernel could not write into their bucket view (0 for UNet)
 
         def seg_capture(k, outputs, grad_outputs, cut):
             g = torch.cuda.CUDAGraph()
             ps = [p for p in self.params_by_segment[k] if p.requires_grad]
             with torch.cuda.graph(g, pool=pool, **kw):
                 res = torch.autograd.grad(outputs, ps + cut, grad_outputs, allow_unused=True)
+                # a gradient that did not land in its bucket view (a re-layout fallback, a layout the kernel cannot
+                # write) is copied there by the same graph
+                for p, r in zip(ps, res):
+                    v = views[id(p)]
+                    if r is not None and (r.data_ptr() != v.data_ptr() or r.stride() != v.stride()):
+                        v.copy_(r)
+                        self.grad_copies += 1
             self.g_bwd.append(g)
             state[k] = res[:len(ps)]                       # (alias the bucket views: kept alive for clarity)
             return res[len(ps):]
@@ -483,6 +495,9 @@ class SegmentedStep:
             self.reducer.launch_bucket(k)
         self.reducer.wait_all()
         self.g_opt.replay()
+        F = _functional()
+        if F is not None:
+            F.graph_replayed()          # the weights and running statistics moved: drop the cached operands
         return self.static_loss
 
     def __call__(self, *inputs):

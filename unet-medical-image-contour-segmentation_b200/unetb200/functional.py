@@ -117,16 +117,28 @@ def _pack_many(items, dtype):
     return outs
 
 
+# Replaying a captured CUDA graph moves weights and BatchNorm running statistics through raw pointers without
+# touching any version counter.  Every replay advances this generation, and the caches below (packed operands,
+# eval-mode BatchNorm coefficients) include it in their keys.
+_GENERATION = [0]
+
+
+def graph_replayed():
+    """Mark every cached packed weight operand and eval-mode BatchNorm coefficient stale.  GraphedStep.replay and
+    SegmentedStep.replay call it; call it after each replay of a graph captured with torch.cuda.graph directly."""
+    _GENERATION[0] += 1
+
+
 # GEMM operands packed ahead of their use by one launch at the start of a whole-network forward (`prepack`).  An
-# entry is valid while the parameter object, its storage, its version counter, dtype and device are unchanged:
-# FusedRMSprop bumps the version of every tensor it updates through raw pointers, so a cached operand can never
-# outlive its weights (and inference re-uses the operands across calls: no pack launch at all).
-_PRE = {}          # (id(w), kind) -> (packed, dtype, parameter version, weakref(w), data_ptr)
+# entry is valid while the parameter object, its storage, its version counter, dtype, device and the replay
+# generation are unchanged: FusedRMSprop bumps the version of every tensor it updates through raw pointers, so a
+# cached operand can never outlive its weights (and inference re-uses the operands across calls: no pack launch at all).
+_PRE = {}          # (id(w), kind) -> (packed, dtype, parameter version, weakref(w), data_ptr, generation)
 
 
 def _pre_valid(ent, w, dtype):
     return (ent is not None and ent[1] == dtype and ent[2] == w._version and ent[3]() is w
-            and ent[4] == w.data_ptr() and ent[0].device == w.device)
+            and ent[4] == w.data_ptr() and ent[0].device == w.device and ent[5] == _GENERATION[0])
 
 
 def _packed(w, dtype, kind):
@@ -160,7 +172,7 @@ def prepack(model, dtype, need_dgrad):
             del _PRE[key]
     if todo:
         for (w, kind), packed in zip(todo, _pack_many(todo, dtype)):
-            _PRE[(id(w), kind)] = (packed, dtype, w._version, weakref.ref(w), w.data_ptr())
+            _PRE[(id(w), kind)] = (packed, dtype, w._version, weakref.ref(w), w.data_ptr(), _GENERATION[0])
     return True
 
 
@@ -264,6 +276,18 @@ def bn_of(z):
     return y, coefs
 
 
+def begin_forward():
+    """Entry of a drop-in forward pass.  Outside any backward pass, whatever a backward pass left queued or handed
+    off belongs to a pass that raised (train.py's OOM retry takes this route): drop it before it can reach the next
+    pass.  Inside one (re-computation under use_checkpointing) nothing changes."""
+    if _GRAD_SUMS or _GRAD_COLSUM:
+        task = ops.graph_task()
+        if task is not None and task < 0:
+            _GRAD_SUMS.clear()
+            _GRAD_COLSUM.clear()
+    ops.drop_aborted_work_if_idle()
+
+
 def leave_grad_sums(g, sums):
     if len(_GRAD_SUMS) > 64:
         _GRAD_SUMS.clear()
@@ -340,7 +364,7 @@ class recompute_mode:
 
 
 # eval-mode BatchNorm coefficients (scale / shift from the running statistics), cached per module while the four
-# tensors they come from are unchanged: an inference loop (evaluate.py:43-143, predict.py:22-27) then launches none
+# tensors they come from are unchanged and no graph has been replayed since: an inference loop (evaluate.py:43-143, predict.py:22-27) then launches none
 # of the 18 tiny coefficient kernels per forward
 _EVAL_COEFS = {}    # id(bn) -> (weakref(bn), key, coefs)
 
@@ -348,7 +372,8 @@ _EVAL_COEFS = {}    # id(bn) -> (weakref(bn), key, coefs)
 def _eval_coefs(bn, Cout):
     import weakref
     parts = (bn.weight, bn.bias, bn.running_mean, bn.running_var)
-    key = tuple((t.data_ptr(), t._version, t.dtype, t.device) if t is not None else None for t in parts) + (bn.eps,)
+    key = tuple((t.data_ptr(), t._version, t.dtype, t.device) if t is not None else None for t in parts) + (
+        bn.eps, _GENERATION[0])
     ent = _EVAL_COEFS.get(id(bn))
     if ent is not None and ent[0]() is bn and ent[1] == key and not torch.cuda.is_current_stream_capturing():
         return ent[2]
@@ -463,6 +488,19 @@ def _sink_owns(param, dW):
             and not torch.is_grad_enabled())
 
 
+def _defer_mode(param, dW, kept, side):
+    """gconv_wgrad's `defer` for the weight gradient dW of `param`: "pass" when a data-parallel sink owns it (its split
+    reduction joins the one launch at the end of the backward pass); "call" when autograd keeps dW as it is (one
+    launch for the layers of the running Function's backward, before autograd sees dW); else, and on the side stream,
+    the reduction follows its wgrad.  Deferred reductions all run on the multi-tensor kernel, whose per-layer
+    summation order does not depend on how the layers are grouped."""
+    if side:
+        return False
+    if _sink_owns(param, dW):
+        return "pass"
+    return "call" if kept else False
+
+
 def _vec_dst(param, Cc):
     """gradient sink of a [C] parameter (BatchNorm gamma / beta, a bias), if any"""
     if param is None:
@@ -518,9 +556,7 @@ def conv_bn_relu_bwd(gz, x, y, w, coefs, batch_stats, need_gx, param=None, bn_pa
     # (only when AccumulateGrad will simply keep dW: an existing .grad would be accumulated into on the main stream)
     kept = _grad_kept_as_is(param, dW)
     side = kept and ops.wgrad_on_side_stream()
-    # nothing reads dW before the pass ends (AccumulateGrad keeps it as it is, or a data-parallel sink owns it):
-    # its split reduction joins the one multi-tensor launch at the end of the backward pass
-    defer = (kept or _sink_owns(param, dW)) and not side
+    defer = _defer_mode(param, dW, kept, side)
     run = lambda: ops.gconv_wgrad(dw_desc, x, gy, dW, skw, si, so, gy_split=gs, defer=defer)  # noqa: E731
     if side:
         ops.on_side_stream(run, x, gy)      # AccumulateGrad keeps dW as it is (same layout, no other owner)
@@ -592,6 +628,11 @@ class DoubleConvFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gz2, gpooled=None):
+        with ops.reductions_at_return():          # both weight gradients complete before autograd sees them
+            return DoubleConvFn._backward(ctx, gz2, gpooled)
+
+    @staticmethod
+    def _backward(ctx, gz2, gpooled):
         x, y1, z1, y2, z2, c1, c2, w1, w2 = ctx.saved_tensors
         cd = x.dtype
         gz = ops.to_nhwc(gz2, cd) if gz2 is not None else None
@@ -701,6 +742,11 @@ class UpCatConvTFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gcat):
+        with ops.reductions_at_return():          # the weight gradient is complete before autograd sees it
+            return UpCatConvTFn._backward(ctx, gcat)
+
+    @staticmethod
+    def _backward(ctx, gcat):
         x1, wT = ctx.saved_tensors
         C2, Cup, off, padded = ctx.geom
         B, C1, h, w = x1.shape
@@ -733,7 +779,7 @@ class UpCatConvTFn(torch.autograd.Function):
             pT = getattr(ctx, "param_obj", wT)
             kept = _grad_kept_as_is(pT, dW)
             side = kept and ops.wgrad_on_side_stream()
-            defer = (kept or _sink_owns(pT, dW)) and not side
+            defer = _defer_mode(pT, dW, kept, side)
             run = lambda: ops.gconv_wgrad(d, x1, gup, dW, 0, s_ci, s_co, sq=s_q, defer=defer)  # noqa: E731
             if side:
                 ops.on_side_stream(run, x1, g)
@@ -795,6 +841,7 @@ class SpatialGateFn(torch.autograd.Function):
         stats, gate = ops.sa_forward(x, wc, out)
         if cfg.save:
             ctx.save_for_backward(x, wc, stats, gate)
+            ctx.param_obj = w
         return out
 
     @staticmethod
@@ -802,10 +849,13 @@ class SpatialGateFn(torch.autograd.Function):
         x, wc, stats, gate = ctx.saved_tensors
         g = ops.to_nhwc(gout, x.dtype)
         dx = ops.empty_nhwc(*x.shape, x.dtype, x.device)
-        dw = torch.empty(98, dtype=torch.float32, device=x.device)
+        # the kernel writes dw as 98 contiguous values: into the gradient sink when that is laid out so
+        dw = grad_dst(ctx.param_obj)
+        if dw is None or not dw.is_contiguous():
+            dw = torch.empty((1, 2, 7, 7), dtype=torch.float32, device=x.device)
         ops.sa_backward(g, x, wc, stats, gate, dx, dw)
         need = ctx.needs_input_grad
-        return (dx if need[0] else None), (dw.view(1, 2, 7, 7) if need[1] else None), None
+        return (dx if need[0] else None), (dw if need[1] else None), None
 
 
 # ------------------------------------------------------------------------------------------------

@@ -13,6 +13,8 @@ from __future__ import annotations
 
 import torch
 
+from .functional import graph_replayed
+
 
 class GraphedStep:
     def __init__(self, step_fn, example_inputs, warmup=3):
@@ -40,6 +42,7 @@ class GraphedStep:
 
     def replay(self):
         self.graph.replay()
+        graph_replayed()                # the weights and running statistics moved: drop the cached operands
         return self.static_loss
 
     def __call__(self, *inputs):

@@ -479,44 +479,96 @@ def gconv_dgrad_bnbwd(d, g, wp, gx, yprev, coefs_prev):
 
 
 # ------------------------------------------------------------------------------------------------
-# deferred split reductions of the weight gradients: one multi-tensor launch per backward pass
+# deferred split reductions of the weight gradients: one multi-tensor launch for several layers
 # ------------------------------------------------------------------------------------------------
 # A wgrad kernel writes `splits` partial results; reducing them layer by layer costs 22 small launches per step.
-# When nothing reads the gradient before the backward pass ends (functional._grad_kept_as_is, or a data-parallel
-# sink that owns p.grad), the reduction is queued and all queued layers are reduced by ONE launch from an autograd
-# engine callback at the end of the pass -- for a segmented backward (ddp.segmented_backward) that is the end of
-# each torch.autograd.grad call, i.e. before the segment's bucket is all-reduced.
-# NOTE the queue keeps the partials alive but only the ADDRESS of the gradient: AccumulateGrad adopts a gradient
-# tensor without copying only while nobody else references it (use_count check) -- a reference held here would make
-# it clone the not-yet-reduced buffer.  The gradient itself is kept alive by p.grad (or is a bucket view).
-_REDUCE_JOBS = []          # (partials, dst address, st, sc, sq, sn, splits, ntaps, Cin, N, Cq)
-_REDUCE_PENDING = [None]
+# Two ways to batch them, both chosen per layer by functional (gconv_wgrad's `defer`):
+# * "call": the reductions queued while one Function's backward runs (functional.DoubleConvFn: both of its convs;
+#   UpCatConvTFn: its ConvTranspose) are made by ONE launch when that backward returns (`reductions_at_return`).  Autograd only sees the gradients after
+#   that, so everything that reads them during the pass -- AccumulateGrad and hooks on its node (where stock
+#   DistributedDataParallel and FSDP attach), the engine summing the two contributions of a parameter used twice --
+#   reads finished values.
+# * "pass": when a data-parallel sink owns the gradient (functional._sink_owns: the reducer drives the pass through
+#   torch.autograd.grad and is its only reader), the reduction is queued and all queued layers are reduced by ONE
+#   launch from an autograd-engine callback at the end of the pass -- for a segmented backward
+#   (ddp.segmented_backward) that is the end of each torch.autograd.grad call, i.e. before the segment's bucket is
+#   all-reduced.
+# NOTE a job keeps the partials alive but only the ADDRESS of the gradient: AccumulateGrad adopts a gradient tensor
+# without copying only while nobody else references it (use_count check) -- a reference held here would make it clone
+# the not-yet-reduced buffer.  A pass that raises never runs its callback, so its jobs must never reach a later
+# flush: a job arriving for another graph task, or a forward entry outside any backward pass
+# (`drop_aborted_work_if_idle`), finds them and drops them.
+_REDUCE_JOBS = []          # (partials, dst address, st, sc, sq, sn, splits, ntaps, Cin, N, Cq): "pass" jobs
+_REDUCE_PENDING = [None]   # graph task whose callback will flush _REDUCE_JOBS
+_CALL_JOBS = [None]        # the "call" jobs of the Function backward running now (None: outside reductions_at_return)
 DEFER_REDUCE = _os.environ.get("UNETB200_DEFER_REDUCE", "1") != "0"
+
+
+def graph_task():
+    """Id of the autograd graph task running on this thread (< 0 outside a backward pass; None on old PyTorch)."""
+    return torch._C._current_graph_task_id() if hasattr(torch._C, "_current_graph_task_id") else None
+
+
+def _reduce_multi(jobs):
+    if not jobs:
+        return
+    arr = (_lib.ReduceJob * len(jobs))()
+    nbytes = 0.0
+    for j, (partials, dst, st, sc, sq, sn, splits, ntaps, Cin, N, Cq) in enumerate(jobs):
+        arr[j].partials, arr[j].dst = partials.data_ptr(), dst
+        arr[j].st, arr[j].sc, arr[j].sq, arr[j].sn = st, sc, sq, sn
+        arr[j].splits, arr[j].ntaps, arr[j].Cin, arr[j].N, arr[j].Cq, arr[j].accumulate = splits, ntaps, Cin, N, Cq, 0
+        nbytes += 4.0 * ntaps * Cin * N * (splits + 1)
+    n = len(jobs)
+    _run("wgrad_reduce", lib().unetb200_wgrad_reduce_multi, arr, n, _stream(), nbytes=nbytes, kernels=(n + 31) // 32)
 
 
 def flush_wgrad_reduce():
     """Reduce every queued weight gradient on the current stream (no-op when nothing is queued)."""
     _REDUCE_PENDING[0] = None
-    if not _REDUCE_JOBS:
-        return
-    jobs = (_lib.ReduceJob * len(_REDUCE_JOBS))()
-    nbytes = 0.0
-    for j, (partials, dst, st, sc, sq, sn, splits, ntaps, Cin, N, Cq) in enumerate(_REDUCE_JOBS):
-        jobs[j].partials, jobs[j].dst = partials.data_ptr(), dst
-        jobs[j].st, jobs[j].sc, jobs[j].sq, jobs[j].sn = st, sc, sq, sn
-        jobs[j].splits, jobs[j].ntaps, jobs[j].Cin, jobs[j].N, jobs[j].Cq, jobs[j].accumulate = splits, ntaps, Cin, N, Cq, 0
-        nbytes += 4.0 * ntaps * Cin * N * (splits + 1)
-    n = len(_REDUCE_JOBS)
     try:
-        _run("wgrad_reduce", lib().unetb200_wgrad_reduce_multi, jobs, n, _stream(), nbytes=nbytes,
-             kernels=(n + 31) // 32)
+        _reduce_multi(_REDUCE_JOBS)
     finally:
         _REDUCE_JOBS.clear()
 
 
+@contextlib.contextmanager
+def reductions_at_return():
+    """The "call" reductions queued inside the block are made by one launch when it ends without an exception."""
+    prev, _CALL_JOBS[0] = _CALL_JOBS[0], []
+    try:
+        yield
+        jobs = _CALL_JOBS[0]
+    finally:
+        _CALL_JOBS[0] = prev
+    _reduce_multi(jobs)
+
+
+def drop_aborted_work():
+    """Forget the weight-gradient work of a backward pass that raised before its end-of-pass callbacks ran: order the
+    current stream after the side stream (its kernels may still write into tensors of the failed pass), then drop the
+    queued reductions -- their destinations may have been freed and handed out again -- and the side-stream operands."""
+    side_stream_sync()
+    _SIDE_KEEP.clear()
+    _SIDE_PENDING[0] = False
+    _REDUCE_JOBS.clear()
+    _REDUCE_PENDING[0] = None
+
+
+def drop_aborted_work_if_idle():
+    """At the entry of a forward pass: outside any backward pass nothing may still be queued or held for one -- what
+    is, belongs to a pass that raised.  Inside a backward pass (re-computation under use_checkpointing) no-op."""
+    if _REDUCE_JOBS or _SIDE_KEEP or _SIDE_PENDING[0]:
+        task = graph_task()
+        if task is not None and task < 0:
+            drop_aborted_work()
+
+
 def _queue_reduce(job):
+    task = graph_task()
+    if _REDUCE_JOBS and _REDUCE_PENDING[0] != task:
+        drop_aborted_work()                          # queued by a pass whose flush callback never ran
     _REDUCE_JOBS.append(job)
-    task = torch._C._current_graph_task_id() if hasattr(torch._C, "_current_graph_task_id") else None
     if task is None or task < 0:
         flush_wgrad_reduce()                         # not inside a backward pass: nothing to wait for
         return
@@ -536,8 +588,12 @@ def _wgrad_once(d, x, gy, dst, st, sc, sn, sq, accumulate, flops, tag, defer=Fal
     _run(f"conv_wgrad_{_ALGO_NAME.get(used.value, '?')}" + tag, lib().unetb200_gconv_wgrad, C.byref(d2), _p(x), _p(gy),
          _p(partials), splits.value, _stream(), flops=flops,
          nbytes=float(es) * d.B * (d.Hin * d.Win * d.Cin + d.Hout * d.Wout * (d.N // d.nquad)) + 4.0 * K * d.N)
-    if defer and not accumulate and DEFER_REDUCE:
-        _queue_reduce((partials, dst.data_ptr(), st, sc, sq, sn, splits.value, d.ntaps, d.Cin, d.N, d.N // d.nquad))
+    if defer and not accumulate and DEFER_REDUCE and (defer == "pass" or _CALL_JOBS[0] is not None):
+        job = (partials, dst.data_ptr(), st, sc, sq, sn, splits.value, d.ntaps, d.Cin, d.N, d.N // d.nquad)
+        if defer == "pass":
+            _queue_reduce(job)
+        else:
+            _CALL_JOBS[0].append(job)
         return used.value
     _run("wgrad_reduce", lib().unetb200_wgrad_reduce, _p(partials), splits.value, d.ntaps, d.Cin, d.N,
          d.N // d.nquad, _p(dst), st, sc, sq, sn, 1 if accumulate else 0, _stream(),
@@ -547,8 +603,9 @@ def _wgrad_once(d, x, gy, dst, st, sc, sn, sq, accumulate, flops, tag, defer=Fal
 
 def gconv_wgrad(d, x, gy, dst, st, sc, sn, sq=0, x_split=None, gy_split=None, defer=False):
     """dst (parameter layout, fp32) = weight gradient; dst[t*st + c*sc + q*sq + co*sn], n = q*Cq + co.
-    defer=True: nothing reads dst before the end of the backward pass -- its split reduction may join the
-    one multi-tensor launch at the end of the pass (flush_wgrad_reduce)."""
+    defer="call": the split reduction joins the one launch made when the enclosing reductions_at_return block ends
+    (made at once outside such a block); defer="pass": nothing but the data-parallel reducer reads dst before the end
+    of the backward pass -- the reduction joins the one launch at the end of the pass (flush_wgrad_reduce)."""
     if not x3_active(d):
         return _wgrad_once(d, x, gy, dst, st, sc, sn, sq, False, gconv_flops(d), _shape_tag(d), defer=defer)
     # 3xTF32: dW = hi(x)^T hi(g) + lo(x)^T hi(g) + hi(x)^T lo(g), the last two accumulated by the split reduction
