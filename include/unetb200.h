@@ -374,6 +374,24 @@ int unetb200_ce_dice_fwd(const void* logits, int dtype, const int64_t* target, i
 int unetb200_ce_dice_bwd(const void* logits, int dtype, const int64_t* target, int64_t npix, int C,
                          const float* coefs, const float* gscale, void* glogits, void* stream);
 
+/* Fused criterion of the binary branch, train.py:118-134 (n_classes == 1), without its boundary term:
+ * BCEWithLogitsLoss(x, t) + dice_loss(sigmoid(x), t) (dice_score.py:5-25, reduce_batch_first=True on the
+ * 3-D input: one global ratio, sets == 0 -> inter).  BCE uses the logit itself (stable form
+ * max(x,0) - x t + log1p(exp(-|x|))), the dice term the sigmoid rounded to `dtype` (autocast: bf16 logits
+ * give bf16 probabilities).  logits [npix] of `dtype` (UNETB200_F32 / UNETB200_BF16) in the same element
+ * order as target [npix] of `tgt_dtype` (UNETB200_F32, UNETB200_I64 or UNETB200_U8), whose VALUE is used
+ * (soft targets and un-remapped class index 2 included).  Deterministic: per-block partials in a fixed order.
+ *   work  : unetb200_bce_dice_work_bytes(npix) bytes; every slot is written by the call, no zeroing needed
+ *   out   : float[4] = {bce + dice_loss, bce, dice_loss, dice_coeff}
+ *   coefs : float[4] saved for backward                                                        */
+int64_t unetb200_bce_dice_work_bytes(int64_t npix);
+int unetb200_bce_dice_fwd(const void* logits, int dtype, const void* target, int tgt_dtype, int64_t npix,
+                          float epsilon, void* work, float* out, float* coefs, void* stream);
+/* glogits [npix] of `dtype` = gscale[0] * d(bce + dice_loss)/dlogits (train.py:118-134); fp32 arithmetic,
+ * rounded once at the store */
+int unetb200_bce_dice_bwd(const void* logits, int dtype, const void* target, int tgt_dtype, int64_t npix,
+                          const float* coefs, const float* gscale, void* glogits, void* stream);
+
 /* dice_coeff (dice_score.py:5-25) on fp32 contiguous input/target viewed as [G][L]: per group
  * inter = 2*sum(x*t), sets = sum x + sum t, sets==0 -> inter, dice = (inter+eps)/(sets+eps);
  * out[0] = mean over groups.  acc: double[3*G] workspace.  saved: float[2*G] for backward. */

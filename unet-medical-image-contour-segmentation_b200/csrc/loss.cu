@@ -1,6 +1,8 @@
-// Loss kernels: fused softmax + cross-entropy + dice (train.py:137-142, dice_score.py:5-36),
-// generic dice_coeff, and the integer-count boundary loss (boundary_loss.py:5-118).
-// All memory-bound single-pass reductions: warp shuffles -> shared memory -> fp64 / int64 atomics.
+// Loss kernels: fused softmax + cross-entropy + dice (train.py:137-142, dice_score.py:5-36), fused
+// BCE-with-logits + sigmoid dice (train.py:118-134), generic dice_coeff, and the integer-count boundary loss
+// (boundary_loss.py:5-118).
+// All memory-bound single-pass reductions: warp shuffles -> shared memory -> fp64 / int64 atomics, or (BCE + dice)
+// per-block fp64 partials summed in a fixed order.
 #include "common.cuh"
 
 namespace ub {
@@ -114,6 +116,128 @@ __global__ void ce_dice_bwd_kernel(const T* __restrict__ logits, const int64_t* 
         Elem<T>::st(glogits + p * C + c, gs * g);
       }
   }
+}
+
+// ------------------------------------------------------------------------------------------
+// fused BCE-with-logits / sigmoid / dice of the binary branch (train.py:118-134)
+// ------------------------------------------------------------------------------------------
+// 8 consecutive target values widened to fp32 (16-byte loads; 8 bytes for uint8)
+__device__ __forceinline__ void load8t(const float* p, float v[8]) { load8(p, v); }
+__device__ __forceinline__ void load8t(const long long* p, float v[8]) {
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    longlong2 r = reinterpret_cast<const longlong2*>(p)[i];
+    v[2 * i] = (float)r.x;
+    v[2 * i + 1] = (float)r.y;
+  }
+}
+__device__ __forceinline__ void load8t(const uint8_t* p, float v[8]) {
+  uint2 r = *reinterpret_cast<const uint2*>(p);
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    v[i] = (float)((r.x >> (8 * i)) & 0xffu);
+    v[4 + i] = (float)((r.y >> (8 * i)) & 0xffu);
+  }
+}
+
+struct BceDiceSums {
+  float bce = 0.f, st = 0.f, s = 0.f, t = 0.f;
+  // BCE on the unrounded logit (binary_cross_entropy_with_logits is on autocast's fp32 list), dice on the
+  // sigmoid rounded to the logits' storage type (F.sigmoid of bf16 logits returns bf16)
+  template <typename T>
+  __device__ __forceinline__ void add(float x, float tv) {
+    bce += fmaxf(x, 0.f) - x * tv + log1pf(expf(-fabsf(x)));
+    const float sr = Elem<T>::round(1.f / (1.f + expf(-x)));
+    st += sr * tv;
+    s += sr;
+    t += tv;
+  }
+};
+
+// vec: the vector path over npix / 8 groups of 8 pixels (every pointer aligned for it); the pixels after the last
+// full group -- all of them when !vec -- are a grid-stride scalar loop.  Each block writes its four sums to
+// partials[k * gridDim.x + blockIdx.x]: no atomics, so the finalize's fixed-order sum is reproducible.
+template <typename T, typename TT>
+__global__ void __launch_bounds__(256) bce_dice_fwd_kernel(const T* __restrict__ logits, const TT* __restrict__ target,
+                                                           int64_t npix, bool vec, double* __restrict__ partials) {
+  __shared__ double sm[32];
+  BceDiceSums acc;
+  const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x, nthr = (int64_t)gridDim.x * blockDim.x;
+  const int64_t nvec = vec ? npix >> 3 : 0;
+  for (int64_t v = tid; v < nvec; v += nthr) {
+    float x[8], t[8];
+    load8(logits + 8 * v, x);
+    load8t(target + 8 * v, t);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) acc.add<T>(x[i], t[i]);
+  }
+  for (int64_t p = 8 * nvec + tid; p < npix; p += nthr) acc.add<T>(Elem<T>::ld(logits + p), (float)target[p]);
+  const double r0 = block_sum((double)acc.bce, sm), r1 = block_sum((double)acc.st, sm),
+               r2 = block_sum((double)acc.s, sm), r3 = block_sum((double)acc.t, sm);
+  if (threadIdx.x == 0) {
+    partials[0 * gridDim.x + blockIdx.x] = r0;
+    partials[1 * gridDim.x + blockIdx.x] = r1;
+    partials[2 * gridDim.x + blockIdx.x] = r2;
+    partials[3 * gridDim.x + blockIdx.x] = r3;
+  }
+}
+
+// one block: the nblk partials of each sum in a fixed order, then dice_coeff(reduce_batch_first=True) on the
+// 3-D input (dice_score.py:12-18: one global ratio, sets == 0 -> inter)
+__global__ void bce_dice_finalize_kernel(const double* __restrict__ partials, int nblk, int64_t npix, float eps,
+                                         float* __restrict__ out, float* __restrict__ coefs) {
+  __shared__ double sm[32];
+  double v[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int b = threadIdx.x; b < nblk; b += blockDim.x)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) v[k] += partials[k * nblk + b];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) v[k] = block_sum(v[k], sm);
+  if (threadIdx.x) return;
+  const float bce = (float)(v[0] / (double)npix);
+  const float inter = 2.f * (float)v[1];
+  float sets = (float)v[2] + (float)v[3];
+  const bool empty = (sets == 0.f);
+  if (empty) sets = inter;
+  const float dice = (inter + eps) / (sets + eps);
+  const float dl = 1.f - dice;
+  out[0] = bce + dl;
+  out[1] = bce;
+  out[2] = dl;
+  out[3] = dice;
+  coefs[0] = 1.f / (float)npix;
+  // d(1 - dice)/ds = -(a t - b); an empty set makes the ratio (inter+eps)/(inter+eps), a constant
+  coefs[1] = empty ? 0.f : 2.f / (sets + eps);
+  coefs[2] = empty ? 0.f : (inter + eps) / ((sets + eps) * (sets + eps));
+  coefs[3] = 0.f;
+}
+
+// d(bce + 1 - dice)/dx = (sigma(x) - t)/npix - (a t - b) s (1 - s),  s = sigma(x) rounded to T
+template <typename T>
+__device__ __forceinline__ float bce_dice_grad(float x, float tv, float invn, float a, float b, float gs) {
+  const float sig = 1.f / (1.f + expf(-x));
+  const float sr = Elem<T>::round(sig);
+  return gs * ((sig - tv) * invn - (a * tv - b) * sr * (1.f - sr));
+}
+
+template <typename T, typename TT>
+__global__ void __launch_bounds__(256) bce_dice_bwd_kernel(const T* __restrict__ logits, const TT* __restrict__ target,
+                                                           int64_t npix, bool vec, const float* __restrict__ coefs,
+                                                           const float* __restrict__ gscale, T* __restrict__ glogits) {
+  const float invn = coefs[0], a = coefs[1], b = coefs[2];
+  const float gs = gscale ? gscale[0] : 1.f;
+  const int64_t tid = blockIdx.x * (int64_t)blockDim.x + threadIdx.x, nthr = (int64_t)gridDim.x * blockDim.x;
+  const int64_t nvec = vec ? npix >> 3 : 0;
+  for (int64_t v = tid; v < nvec; v += nthr) {
+    float x[8], t[8];
+    load8(logits + 8 * v, x);
+    load8t(target + 8 * v, t);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) x[i] = bce_dice_grad<T>(x[i], t[i], invn, a, b, gs);
+    store8(glogits + 8 * v, x);
+  }
+  for (int64_t p = 8 * nvec + tid; p < npix; p += nthr)
+    Elem<T>::st(glogits + p, bce_dice_grad<T>(Elem<T>::ld(logits + p), (float)target[p], invn, a, b, gs));
 }
 
 // ------------------------------------------------------------------------------------------
@@ -350,6 +474,71 @@ int unetb200_ce_dice_bwd(const void* logits, int dtype, const int64_t* target, i
   UB_LAUNCH_CHECK("ce_dice_bwd");
   return 0;
 }
+
+static inline int bce_dice_grid(int64_t npix) { return loss_grid((npix + 7) / 8, 256); }
+
+static inline bool bce_dice_vec(const void* logits, const void* target, int tgt_dtype, const void* glogits) {
+  const uintptr_t talign = tgt_dtype == UNETB200_U8 ? 8 : 16;
+  return aligned16(logits) && (reinterpret_cast<uintptr_t>(target) & (talign - 1)) == 0 &&
+         (glogits == nullptr || aligned16(glogits));
+}
+
+// GO(T, TT) for the (logits, target) storage types given by `dtype`, `tgt_dtype`
+#define BCE_DICE_DISPATCH()                                                      \
+  do {                                                                           \
+    if (dtype == UNETB200_BF16) {                                                \
+      if (tgt_dtype == UNETB200_F32) GO(bf16, float);                            \
+      else if (tgt_dtype == UNETB200_I64) GO(bf16, long long);                   \
+      else GO(bf16, uint8_t);                                                    \
+    } else {                                                                     \
+      if (tgt_dtype == UNETB200_F32) GO(float, float);                           \
+      else if (tgt_dtype == UNETB200_I64) GO(float, long long);                  \
+      else GO(float, uint8_t);                                                   \
+    }                                                                            \
+  } while (0)
+
+int64_t unetb200_bce_dice_work_bytes(int64_t npix) {
+  if (npix <= 0) return 0;
+  return 4 * (int64_t)bce_dice_grid(npix) * (int64_t)sizeof(double);
+}
+
+int unetb200_bce_dice_fwd(const void* logits, int dtype, const void* target, int tgt_dtype, int64_t npix, float epsilon,
+                          void* work, float* out, float* coefs, void* stream) {
+  UB_CHECK_ARG(dtype == UNETB200_F32 || dtype == UNETB200_BF16, "bce_dice_fwd: dtype");
+  UB_CHECK_ARG(tgt_dtype == UNETB200_F32 || tgt_dtype == UNETB200_I64 || tgt_dtype == UNETB200_U8,
+               "bce_dice_fwd: target dtype");
+  UB_CHECK_ARG(npix > 0, "bce_dice_fwd: npix=%lld", (long long)npix);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int g = bce_dice_grid(npix);
+  const bool vec = bce_dice_vec(logits, target, tgt_dtype, nullptr);
+  double* partials = (double*)work;
+#define GO(T, TT) \
+  bce_dice_fwd_kernel<T, TT><<<g, 256, 0, s>>>((const T*)logits, (const TT*)target, npix, vec, partials)
+  BCE_DICE_DISPATCH();
+#undef GO
+  bce_dice_finalize_kernel<<<1, 256, 0, s>>>(partials, g, npix, epsilon, out, coefs);
+  UB_LAUNCH_CHECK("bce_dice_fwd");
+  return 0;
+}
+
+int unetb200_bce_dice_bwd(const void* logits, int dtype, const void* target, int tgt_dtype, int64_t npix,
+                          const float* coefs, const float* gscale, void* glogits, void* stream) {
+  UB_CHECK_ARG(dtype == UNETB200_F32 || dtype == UNETB200_BF16, "bce_dice_bwd: dtype");
+  UB_CHECK_ARG(tgt_dtype == UNETB200_F32 || tgt_dtype == UNETB200_I64 || tgt_dtype == UNETB200_U8,
+               "bce_dice_bwd: target dtype");
+  UB_CHECK_ARG(npix > 0, "bce_dice_bwd: npix=%lld", (long long)npix);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int g = bce_dice_grid(npix);
+  const bool vec = bce_dice_vec(logits, target, tgt_dtype, glogits);
+#define GO(T, TT)                                                                                               \
+  bce_dice_bwd_kernel<T, TT><<<g, 256, 0, s>>>((const T*)logits, (const TT*)target, npix, vec, coefs, gscale, \
+                                               (T*)glogits)
+  BCE_DICE_DISPATCH();
+#undef GO
+  UB_LAUNCH_CHECK("bce_dice_bwd");
+  return 0;
+}
+#undef BCE_DICE_DISPATCH
 
 int unetb200_dice_fwd(const float* x, const float* t, int64_t G, int64_t L, float epsilon, double* acc, float* out,
                       float* saved, void* stream) {

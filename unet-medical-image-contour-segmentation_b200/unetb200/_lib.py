@@ -110,6 +110,9 @@ PROTOTYPES = {
                                              c_i64, C.c_int, C.c_int, c_p]),
     "unetb200_ce_dice_fwd": (C.c_int, [c_p, C.c_int, c_p, c_i64, C.c_int, C.c_float, c_p, c_p, c_p, c_p]),
     "unetb200_ce_dice_bwd": (C.c_int, [c_p, C.c_int, c_p, c_i64, C.c_int, c_p, c_p, c_p, c_p]),
+    "unetb200_bce_dice_work_bytes": (c_i64, [c_i64]),
+    "unetb200_bce_dice_fwd": (C.c_int, [c_p, C.c_int, c_p, C.c_int, c_i64, C.c_float, c_p, c_p, c_p, c_p]),
+    "unetb200_bce_dice_bwd": (C.c_int, [c_p, C.c_int, c_p, C.c_int, c_i64, c_p, c_p, c_p, c_p]),
     "unetb200_dice_fwd": (C.c_int, [c_p, c_p, c_i64, c_i64, C.c_float, c_p, c_p, c_p, c_p]),
     "unetb200_dice_bwd": (C.c_int, [c_p, c_p, c_i64, c_i64, C.c_float, c_p, c_p, c_p, c_p]),
     "unetb200_boundary_loss": (C.c_int, [c_p, C.c_int, c_i64, c_i64, c_i64, c_p, C.c_int, c_i64, c_i64, c_i64,

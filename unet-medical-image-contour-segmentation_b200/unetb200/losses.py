@@ -4,6 +4,9 @@
   boundary_loss                                   -- reference utils/boundary_loss.py:5-118
   ce_dice_loss                                    -- the fused form of train.py:137-142
                                                      (CrossEntropyLoss + multiclass dice on softmax/one-hot)
+  bce_dice_loss                                   -- the fused form of train.py:118-134 without its boundary term
+                                                     (BCEWithLogitsLoss + dice on sigmoid, n_classes == 1)
+  training_criterion                              -- either branch plus its boundary term
 """
 from __future__ import annotations
 
@@ -12,7 +15,7 @@ import ctypes as C
 import torch
 
 from . import _lib, ops
-from ._lib import BF16, F32, I64
+from ._lib import BF16, F32, I64, U8
 
 
 # ------------------------------------------------------------------------------------------------
@@ -178,10 +181,93 @@ def ce_dice_loss(logits, target, epsilon=1e-6, return_parts=False):
     return (total, parts) if return_parts else total
 
 
-def training_criterion(logits, masks, boundary_coeff=0.2, edge_width=51, edge_weight=7):
-    """The multi-class loss train.py optimises: CE + dice (train.py:137-142) plus the boundary term in
-    its train.py:143-147 form (coefficient boundary_weight*norm_factor = 0.2)."""
-    loss = ce_dice_loss(logits, masks)
+# ------------------------------------------------------------------------------------------------
+# fused BCE + sigmoid dice criterion (the binary branch)
+# ------------------------------------------------------------------------------------------------
+_TGT_DT = {torch.float32: F32, torch.int64: I64, torch.uint8: U8}
+
+
+class BceDiceFn(torch.autograd.Function):
+    """logits and target in the same (pixel) element order; see :func:`bce_dice_loss`."""
+
+    @staticmethod
+    def forward(ctx, logits, target, eps):
+        dev = logits.device
+        npix = logits.numel()
+        L = ops.lib()
+        work = torch.empty(L.unetb200_bce_dice_work_bytes(npix), dtype=torch.uint8, device=dev)
+        out = torch.empty(4, dtype=torch.float32, device=dev)
+        coefs = torch.empty(4, dtype=torch.float32, device=dev)
+        ops._run("bce_dice_fwd", L.unetb200_bce_dice_fwd, ops._p(logits), ops.dt(logits), ops._p(target),
+                 _TGT_DT[target.dtype], npix, eps, ops._p(work), ops._p(out), ops._p(coefs), ops._stream(), kernels=2,
+                 nbytes=float(npix) * (logits.element_size() + target.element_size()))
+        ctx.save_for_backward(logits, target, coefs)
+        ctx.mark_non_differentiable(out)
+        return out[0].clone().reshape(()), out
+
+    @staticmethod
+    def backward(ctx, g, _gparts):
+        logits, target, coefs = ctx.saved_tensors
+        npix = logits.numel()
+        gs = g.detach().float().reshape(1).contiguous()
+        gl = torch.empty_like(logits)              # a dense layout keeps its strides (same element order)
+        ops._run("bce_dice_bwd", ops.lib().unetb200_bce_dice_bwd, ops._p(logits), ops.dt(logits), ops._p(target),
+                 _TGT_DT[target.dtype], npix, ops._p(coefs), ops._p(gs), ops._p(gl), ops._stream(),
+                 nbytes=float(npix) * (2 * logits.element_size() + target.element_size()))
+        return gl, None, None
+
+
+def bce_dice_loss(logits, target, epsilon=1e-6, return_parts=False):
+    """BCEWithLogitsLoss(logits, target) + dice_loss(sigmoid(logits), target) in one pass over the logits: the
+    binary branch of train.py:118-134 without its boundary term.  logits: [B,1,H,W] or [B,H,W], fp32 / bf16 (the
+    dice term uses the sigmoid rounded to that type, as under autocast); target: [B,H,W] fp32 / int64 / uint8,
+    used by value (soft targets allowed).  return_parts: also a device float[4] {total, bce, dice_loss, dice}."""
+    ops.require_cuda(logits, "bce_dice_loss")
+    if logits.dim() == 4 and logits.size(1) == 1:
+        B, _, H, W = logits.shape
+    elif logits.dim() == 3:
+        B, H, W = logits.shape
+    else:
+        raise ValueError(f"bce_dice_loss: logits must be [B,1,H,W] or [B,H,W], got {tuple(logits.shape)}")
+    if tuple(target.shape) != (B, H, W):
+        raise ValueError(f"bce_dice_loss: target {tuple(target.shape)} does not match logits {(B, H, W)}")
+    if logits.numel() == 0:
+        raise ValueError("bce_dice_loss: empty input")
+    lg = logits
+    if lg.dtype not in (torch.float32, torch.bfloat16):
+        lg = lg.float()
+    # one channel: NCHW and channels_last hold the pixels in the same order; anything else is made contiguous
+    if not (lg.squeeze(1) if lg.dim() == 4 else lg).is_contiguous():
+        lg = lg.contiguous()
+    tgt = target
+    if tgt.dtype not in _TGT_DT:
+        tgt = tgt.float()
+    if not tgt.is_contiguous():
+        tgt = tgt.contiguous()
+    total, parts = BceDiceFn.apply(lg, tgt, float(epsilon))
+    return (total, parts) if return_parts else total
+
+
+# boundary-term constants of the two branches of train.py: (coefficient, edge_width, edge_weight)
+_BOUNDARY_BINARY = (0.25, 51, 15)          # train.py:118-134
+_BOUNDARY_MULTICLASS = (0.2, 51, 7)        # train.py:143-147 (boundary_weight * norm_factor = 0.2)
+
+
+def training_criterion(logits, masks, boundary_coeff=None, edge_width=None, edge_weight=None):
+    """The loss train.py optimises, branch chosen by the channel count of ``logits``:
+
+    * one channel (n_classes == 1, train.py:118-134): BCEWithLogits + dice(sigmoid) (:func:`bce_dice_loss`)
+      + 0.25 * boundary_loss(edge_width=51, edge_weight=15);
+    * more (train.py:137-147): CE + multiclass dice (:func:`ce_dice_loss`) + 0.2 * boundary_loss(51, 7).
+
+    ``None`` means that branch's train.py constant; explicit values win and ``boundary_coeff=0`` drops the term.
+    Binary masks are used by value: train.py's ``true_masks //= 2`` remap is the caller's."""
+    binary = logits.dim() == 4 and logits.size(1) == 1
+    d_coeff, d_width, d_weight = _BOUNDARY_BINARY if binary else _BOUNDARY_MULTICLASS
+    boundary_coeff = d_coeff if boundary_coeff is None else boundary_coeff
+    edge_width = d_width if edge_width is None else edge_width
+    edge_weight = d_weight if edge_weight is None else edge_weight
+    loss = bce_dice_loss(logits, masks) if binary else ce_dice_loss(logits, masks)
     if boundary_coeff:
         # train.py passes true_masks.float(); the int64 class indices compare identically to 255
         loss = loss + boundary_coeff * boundary_loss(logits, masks, edge_width=edge_width, edge_weight=edge_weight)
