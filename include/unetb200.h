@@ -428,6 +428,23 @@ int unetb200_rmsprop_step(float* const* w, float* const* g, float* const* sq, fl
                           const int64_t* numel, int ntensors, const double* sumsq, float max_norm, float lr,
                           float alpha, float eps, float weight_decay, float momentum, int write_clipped_grad,
                           void* stream);
+/* GradScaler and LR schedules inside a captured step, train.py:154-159 (scale(loss).backward(), unscale_,
+ * clip_grad_norm_, step, update).  Every value that changes between replays is read from DEVICE memory.
+ * One read pass: *sumsq = sum_i sum((g_i * inv_scale)^2) (the order of unetb200_grad_sqnorm), and
+ * *found_inf = 1.0f if any element of any g_i is non-finite (isfinite per element; accumulated into, never
+ * cleared, as torch's found_inf).  inv_scale NULL means 1; sumsq NULL skips the norm (check only); found_inf NULL
+ * skips the check. */
+int unetb200_grad_sqnorm_amp(float* const* grads, const int64_t* numel, int ntensors, const float* inv_scale,
+                             double* sumsq, float* found_inf, void* stream);
+/* unetb200_rmsprop_step with *lr read on the device, g multiplied by *inv_scale (NULL: 1) before the clip
+ * coefficient, whose norm is that of the unscaled gradients.  found_inf != NULL and *found_inf != 0: nothing is
+ * stored (w, sq, mom, g and step unchanged, as when GradScaler skips optimizer.step()).  Otherwise each step[i]
+ * (fp32 0-dim) is incremented, and write_clipped_grad stores the unscaled, clipped gradient. */
+int unetb200_rmsprop_step_amp(float* const* w, float* const* g, float* const* sq, float* const* mom,
+                              float* const* step, const int64_t* numel, int ntensors, const double* sumsq,
+                              float max_norm, const float* lr, const float* inv_scale, const float* found_inf,
+                              float alpha, float eps, float weight_decay, float momentum, int write_clipped_grad,
+                              void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Callers either side of the step (SURVEY.md section 8(f) N1, N3): evaluate / predict tail and the

@@ -121,6 +121,9 @@ PROTOTYPES = {
     "unetb200_grad_sqnorm": (C.c_int, [c_p, c_p, C.c_int, c_p, c_p]),
     "unetb200_rmsprop_step": (C.c_int, [c_p, c_p, c_p, c_p, c_p, C.c_int, c_p, C.c_float, C.c_float, C.c_float, C.c_float,
                                         C.c_float, C.c_float, C.c_int, c_p]),
+    "unetb200_grad_sqnorm_amp": (C.c_int, [c_p, c_p, C.c_int, c_p, c_p, c_p, c_p]),
+    "unetb200_rmsprop_step_amp": (C.c_int, [c_p, c_p, c_p, c_p, c_p, c_p, C.c_int, c_p, C.c_float, c_p, c_p, c_p,
+                                            C.c_float, C.c_float, C.c_float, C.c_float, C.c_int, c_p]),
     "unetb200_eval_counts": (C.c_int, [c_p, C.c_int, c_i64, c_i64, c_i64, c_i64, c_p, C.c_int, C.c_int, C.c_int,
                                        C.c_int, C.c_int, C.c_int, C.c_int, c_p, C.c_int, c_p, C.c_float, c_p, c_p]),
     "unetb200_resize_argmax": (C.c_int, [c_p, C.c_int, c_i64, c_i64, c_i64, c_i64] + [C.c_int] * 6 + [c_p, C.c_int, c_p]),
