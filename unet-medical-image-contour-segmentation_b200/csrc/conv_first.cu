@@ -563,13 +563,11 @@ static int first_blocks(long long M, int lanes) {
 
 long long first_fprop_tiles(const unetb200_gconv_t* d) {
   if (!first_common(d)) return 0;
-  const long long a = first_blocks((long long)d->B * d->Hm * d->Wm, 256 / (d->N / 8)), b = first_tc_stats_rows(d);
-  return a > b ? a : b;
+  return first_blocks((long long)d->B * d->Hm * d->Wm, 256 / (d->N / 8));
 }
 
 int first_fprop(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* wp, void* y, double* stats,
                 float* stats_ws, cudaStream_t s) {
-  if (first_tc_supported(d, y) && aligned16(wp)) return first_tc_fprop(d, x, wp, y, stats, stats_ws, nullptr, s);
   const int blocks = first_blocks(g.M, 256 / (d->N / 8));
   if (first_tiled_ok(d)) {
     const int tiles_w = (d->Wm + kFT_W - 1) / kFT_W, tiles_h = (d->Hm + kFT_H - 1) / kFT_H;

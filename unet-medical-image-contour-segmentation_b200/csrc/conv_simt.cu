@@ -1,43 +1,13 @@
 // CUDA-core (fp32 FMA) implicit-GEMM engine for the generalised convolution of unetb200.h.
 // It handles every shape (C_in = 1 or 3 first layer, widths that do not fill a UMMA tile, unaligned
-// channel slices) and is the arithmetic of the fp32 "exactness" mode.  Large bf16 layers are
-// dispatched to the tcgen05 engine in conv_tc.cu instead.
-#include <cstdlib>
-
+// channel slices) and is the arithmetic of the fp32 "exactness" mode; gconv.cu routes a descriptor here
+// when no specialised engine covers it.  Also the split-K reductions and the weight packing.
 #include "gconv.cuh"
 
 namespace ub {
 
 constexpr int FBM = 128, FBN = 64, FBK = 16;   // fprop tile
 constexpr int WBK = 64, WBN = 64, WBM = 16;    // wgrad tile (K rows x N cols, M step)
-
-int gconv_validate(const unetb200_gconv_t* d, GconvDev* o) {
-  UB_CHECK_ARG(d != nullptr, "gconv: null descriptor");
-  UB_CHECK_ARG(d->dtype == UNETB200_F32 || d->dtype == UNETB200_BF16, "gconv: dtype %d", d->dtype);
-  UB_CHECK_ARG(d->B > 0 && d->Hm > 0 && d->Wm > 0 && d->Cin > 0, "gconv: bad M grid / Cin");
-  UB_CHECK_ARG(d->ntaps >= 1 && d->ntaps <= 9, "gconv: ntaps %d", d->ntaps);
-  UB_CHECK_ARG(d->in_scale == 1 || d->in_scale == 2, "gconv: in_scale %d", d->in_scale);
-  UB_CHECK_ARG(d->out_scale == 1 || d->out_scale == 2, "gconv: out_scale %d", d->out_scale);
-  UB_CHECK_ARG(d->nquad == 1 || d->nquad == 4, "gconv: nquad %d", d->nquad);
-  UB_CHECK_ARG(d->N > 0 && d->N % d->nquad == 0, "gconv: N %d not divisible by nquad %d", d->N, d->nquad);
-  UB_CHECK_ARG(d->nquad == 1 || d->out_scale == 2, "gconv: nquad 4 needs out_scale 2");
-  UB_CHECK_ARG(d->Hin > 0 && d->Win > 0 && d->Hout > 0 && d->Wout > 0, "gconv: bad grids");
-  UB_CHECK_ARG(d->ld_in >= d->Cin && d->ld_out >= d->N / d->nquad, "gconv: pixel stride smaller than channels");
-  UB_CHECK_ARG(d->out_off_y >= 0 && d->out_off_x >= 0 &&
-                   (d->Hm - 1) * d->out_scale + (d->nquad == 4 ? 1 : 0) + d->out_off_y < d->Hout &&
-                   (d->Wm - 1) * d->out_scale + (d->nquad == 4 ? 1 : 0) + d->out_off_x < d->Wout,
-               "gconv: output does not fit the destination grid");
-  o->B = d->B; o->Hm = d->Hm; o->Wm = d->Wm; o->Cin = d->Cin; o->ntaps = d->ntaps;
-  for (int t = 0; t < 9; ++t) { o->tap_dy[t] = d->tap_dy[t]; o->tap_dx[t] = d->tap_dx[t]; }
-  o->in_scale = d->in_scale; o->in_off_y = d->in_off_y; o->in_off_x = d->in_off_x;
-  o->Hin = d->Hin; o->Win = d->Win; o->ld_in = d->ld_in;
-  o->N = d->N; o->nquad = d->nquad; o->Cq = d->N / d->nquad; o->out_scale = d->out_scale;
-  o->out_off_y = d->out_off_y; o->out_off_x = d->out_off_x; o->Hout = d->Hout; o->Wout = d->Wout;
-  o->ld_out = d->ld_out;
-  o->M = (long long)d->B * d->Hm * d->Wm;
-  o->K = d->ntaps * d->Cin;
-  return 0;
-}
 
 __device__ __forceinline__ void decode_m(const GconvDev& d, long long m, int& b, int& i, int& j) {
   j = (int)(m % d.Wm);
@@ -665,7 +635,9 @@ static int simt_fbn(int N) { return N <= 16 ? 16 : (N <= 32 ? 32 : 64); }
 static int simt_fbm(int N) { return 8 * 256 / (simt_fbn(N) / 4); }
 static int simt_wbk(int N) { return 4 * 256 / (simt_fbn(N) / 4); }
 
-static int simt_wgrad_splits(const GconvDev& g) {
+long long simt_fprop_tiles(const GconvDev& g) { return (g.M + FBM - 1) / FBM; }
+
+int simt_wgrad_splits(const GconvDev& g) {
   const int wbn = simt_fbn(g.N), wbk = simt_wbk(g.N);
   long long tiles = (long long)((g.K + wbk - 1) / wbk) * ((g.N + wbn - 1) / wbn);
   long long want = ((long long)sm_count() * 6 + tiles - 1) / tiles;
@@ -676,75 +648,10 @@ static int simt_wgrad_splits(const GconvDev& g) {
   return (int)want;
 }
 
-}  // namespace ub
-
-using namespace ub;
 typedef __nv_bfloat16 bf16;
 
-extern "C" {
-
-int64_t unetb200_gconv_stats_workspace(const unetb200_gconv_t* d) {
-  GconvDev g;
-  if (gconv_validate(d, &g)) return -1;
-  long long simt_tiles = (g.M + FBM - 1) / FBM;
-  long long tiles = simt_tiles;
-  long long ft = first_fprop_tiles(d);
-  if (ft > tiles) tiles = ft;
-  long long n = tiles * 2 * g.N;
-  long long n2 = tc2_stats_workspace(d);
-  if (n2 > n) n = n2;
-  long long n3 = tc3_stats_workspace(d);
-  if (n3 > n) n = n3;
-  const long long n4 = narrow_tc_stats_rows(d) * 2 * g.N;
-  if (n4 > n) n = n4;
-  const long long n5 = halo_stats_rows(d) * 2 * g.N;
-  if (n5 > n) n = n5;
-  const long long n6 = first_narrow_rows(d) * 2 * g.N;
-  if (n6 > n) n = n6;
-  const long long n7 = fprop_narrow_f32_rows(d) * 2 * g.N;
-  return n > n7 ? n : n7;
-}
-
-int unetb200_gconv_fprop(const unetb200_gconv_t* d, const void* x, const void* wp, const float* bias, void* y,
-                         double* stats, float* stats_ws, int* algo_used, void* stream) {
-  GconvDev g;
-  int rc = gconv_validate(d, &g);
-  if (rc) return rc;
-  UB_CHECK_ARG(x && wp && y, "gconv_fprop: null pointer");
-  UB_CHECK_ARG(!stats || (stats_ws && d->nquad == 1), "gconv_fprop: stats need a workspace and nquad == 1");
-  if (!stats) stats_ws = nullptr;
-  cudaStream_t s = (cudaStream_t)stream;
-  int algo = d->algo;
-  if (algo != UNETB200_ALGO_SIMT && !stats && halo_t_fprop_supported(d, x, wp, y)) {  // narrow ConvTranspose2d
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    return halo_t_fprop(d, x, wp, bias, y, s);
-  }
-  if (algo != UNETB200_ALGO_SIMT && !stats && !bias && halo_t_dgrad_supported(d, x, wp, y)) {      // ... and its dgrad
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    return halo_t_dgrad(d, x, wp, y, s);
-  }
-  if (!bias && first_narrow_supported(d, y)) {          // C_in = 1 -> 8 / 16 / 32 channels
-    if (algo_used) *algo_used = UNETB200_ALGO_SIMT;
-    return first_narrow_fprop(d, x, wp, y, stats, stats_ws, nullptr, s);
-  }
-  if (algo != UNETB200_ALGO_SIMT && !bias && halo_fprop_supported(d, x, wp, y)) {     // 16 / 32 / 64 channels: TMA halo box
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    return halo_fprop(d, x, wp, y, stats, stats_ws, nullptr, s);
-  }
-  if (algo != UNETB200_ALGO_SIMT && !bias && narrow_tc_supported(d, x, wp, y)) {      // narrow channel counts: thread-built im2col
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    return narrow_tc_fprop(d, x, wp, y, stats, stats_ws, nullptr, s);
-  }
-  if (algo == UNETB200_ALGO_AUTO || algo == UNETB200_ALGO_PREFER_TC) algo = tc_fprop_supported(d, x, wp, y) ? UNETB200_ALGO_TC : UNETB200_ALGO_SIMT;
-  if (algo_used) *algo_used = algo;
-  if (algo == UNETB200_ALGO_TC) {
-    UB_CHECK_ARG(tc_fprop_supported(d, x, wp, y), "gconv_fprop: tcgen05 path requested but shape/alignment unsupported");
-    if (tc3_fprop_supported(d, x, wp, bias, y)) return tc3_fprop(d, g, x, wp, y, stats, stats_ws, s);
-    return tc2_fprop(d, g, x, wp, bias, y, stats, stats_ws, s);
-  }
-  UB_CHECK_ARG(algo == UNETB200_ALGO_SIMT, "gconv_fprop: unknown algo %d", algo);
-  if (!bias && first_fprop_supported(d, y)) return first_fprop(d, g, x, wp, y, stats, stats_ws, s);
-  if (!bias && fprop_narrow_f32_supported(d, x, wp, y)) return fprop_narrow_f32(d, x, wp, y, stats, stats_ws, s);
+int simt_fprop(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* wp, const float* bias, void* y,
+               double* stats, float* stats_ws, cudaStream_t s) {
   const int fbn = simt_fbn(g.N), fbm = simt_fbm(g.N);
   dim3 grid((unsigned)((g.M + fbm - 1) / fbm), (unsigned)((g.N + fbn - 1) / fbn));
   const bool vec = simt_vec_ok(d, x, wp, y) && (g.K % 4 == 0);
@@ -762,207 +669,8 @@ int unetb200_gconv_fprop(const unetb200_gconv_t* d, const void* x, const void* w
   return 0;
 }
 
-// conv3x3 -> BatchNorm(eval) -> ReLU with the normalisation folded into the tcgen05 epilogue (inference only)
-int unetb200_gconv_fprop_affine_relu_supported(const unetb200_gconv_t* d, const void* x, const void* wp, const void* z) {
-  GconvDev g;
-  if (gconv_validate(d, &g)) return 0;
-  static const bool off = getenv("UNETB200_NO_BN_FOLD") != nullptr;
-  static const bool wide = getenv("UNETB200_TC3_MAXBN") && atoi(getenv("UNETB200_TC3_MAXBN")) >= 256;
-  if (off || d->algo == UNETB200_ALGO_SIMT) return 0;
-  if (first_tc_supported(d, z) && aligned16(wp)) return 1;            // first layer: thread-built im2col kernel
-  if (first_narrow_supported(d, z)) return 1;                         // C_in = 1 -> 8 / 16 / 32 channels
-  if (halo_fprop_supported(d, x, wp, z)) return 1;                    // 16 / 32 / 64 channels: TMA halo box
-  if (narrow_tc_supported(d, x, wp, z)) return 1;                     // narrow channel counts: the same, generalised
-  if (d->N % 128 != 0 && d->N % 64 != 0) return 0;
-  if (d->dtype == UNETB200_BF16 && d->N % 256 == 0 && wide) return 0;
-  return tc_fprop_supported(d, x, wp, z) && tc3_fprop_supported(d, x, wp, nullptr, z);
-}
-
-int unetb200_gconv_fprop_affine_relu(const unetb200_gconv_t* d, const void* x, const void* wp, const float* scale_shift,
-                                     void* z, void* stream) {
-  GconvDev g;
-  int rc = gconv_validate(d, &g);
-  if (rc) return rc;
-  UB_CHECK_ARG(x && wp && z && scale_shift, "gconv_fprop_affine_relu: null pointer");
-  UB_CHECK_ARG(unetb200_gconv_fprop_affine_relu_supported(d, x, wp, z),
-               "gconv_fprop_affine_relu: shape not covered by the fused kernel (query _supported first and run "
-               "gconv_fprop + bn_relu_apply instead)");
-  if (first_tc_supported(d, z) && aligned16(wp))
-    return first_tc_fprop(d, x, wp, z, nullptr, nullptr, scale_shift, (cudaStream_t)stream);
-  if (first_narrow_supported(d, z))
-    return first_narrow_fprop(d, x, wp, z, nullptr, nullptr, scale_shift, (cudaStream_t)stream);
-  if (halo_fprop_supported(d, x, wp, z))
-    return halo_fprop(d, x, wp, z, nullptr, nullptr, scale_shift, (cudaStream_t)stream);
-  if (narrow_tc_supported(d, x, wp, z))
-    return narrow_tc_fprop(d, x, wp, z, nullptr, nullptr, scale_shift, (cudaStream_t)stream);
-  return tc3_fprop(d, g, x, wp, z, nullptr, nullptr, (cudaStream_t)stream, scale_shift);
-}
-
-// the same with MaxPool2d(2) of the activation as a second output (Down: unet_parts.py:26-37 under .eval()): the CTA-pair
-// kernel only -- a warp's 4 x 8 pixel patch of the epilogue holds whole 2 x 2 windows
-int unetb200_gconv_fprop_affine_relu_pool_supported(const unetb200_gconv_t* d, const void* x, const void* wp, const void* z,
-                                                    const void* pooled, int64_t ld_pooled) {
-  GconvDev g;
-  if (gconv_validate(d, &g)) return 0;
-  static const bool off = getenv("UNETB200_NO_POOL_FOLD") != nullptr;
-  if (off || d->dtype != UNETB200_BF16 || !pooled || (ld_pooled & 1) || (reinterpret_cast<uintptr_t>(pooled) & 3)) return 0;
-  if (!unetb200_gconv_fprop_affine_relu_supported(d, x, wp, z)) return 0;
-  if ((first_tc_supported(d, z) && aligned16(wp)) || first_narrow_supported(d, z)) return 0;   // first-layer kernels: no
-  if (!halo_fprop_supported(d, x, wp, z) && narrow_tc_supported(d, x, wp, z)) return 0;        // thread-built im2col: no
-  return d->Hm >= 2 && d->Wm >= 2;                 // the TMA-staged narrow kernel and the CTA-pair kernel: yes
-}
-
-int unetb200_gconv_fprop_affine_relu_pool(const unetb200_gconv_t* d, const void* x, const void* wp, const float* scale_shift,
-                                          void* z, void* pooled, int64_t ld_pooled, void* stream) {
-  GconvDev g;
-  int rc = gconv_validate(d, &g);
-  if (rc) return rc;
-  UB_CHECK_ARG(x && wp && z && scale_shift && pooled, "gconv_fprop_affine_relu_pool: null pointer");
-  UB_CHECK_ARG(unetb200_gconv_fprop_affine_relu_pool_supported(d, x, wp, z, pooled, ld_pooled),
-               "gconv_fprop_affine_relu_pool: shape not covered (query _supported first and run gconv_fprop_affine_relu + "
-               "maxpool2_fwd instead)");
-  if (halo_fprop_supported(d, x, wp, z))
-    return halo_fprop(d, x, wp, z, nullptr, nullptr, scale_shift, (cudaStream_t)stream, nullptr, 0, nullptr, pooled,
-                      (long long)ld_pooled);
-  return tc3_fprop(d, g, x, wp, z, nullptr, nullptr, (cudaStream_t)stream, scale_shift, nullptr, 0, nullptr, nullptr, pooled,
-                   (long long)ld_pooled);
-}
-
-// dgrad of a 3x3 convolution + the reduction pass of the BatchNorm/ReLU backward of the layer that produced its input
-int unetb200_gconv_dgrad_bnbwd_supported(const unetb200_gconv_t* d, const void* g, const void* wp, const void* gx) {
-  GconvDev gd;
-  if (gconv_validate(d, &gd)) return 0;
-  static const bool off = getenv("UNETB200_NO_BNBWD_FUSE") != nullptr;
-  if (off || d->algo == UNETB200_ALGO_SIMT) return 0;
-  if (halo_bnbwd_supported(d, g, wp, gx)) return 1;                   // narrow layers: the TMA-staged kernel's epilogue
-  return tc_fprop_supported(d, g, wp, gx) && tc3_fprop_supported(d, g, wp, nullptr, gx) && tc3_bnbwd_supported(d);
-}
-
-int unetb200_gconv_dgrad_bnbwd(const unetb200_gconv_t* d, const void* g, const void* wp, void* gx, const void* yprev,
-                               int64_t ld_yprev, const float* coefs, double* sums, float* ws, void* stream) {
-  GconvDev gd;
-  int rc = gconv_validate(d, &gd);
-  if (rc) return rc;
-  UB_CHECK_ARG(g && wp && gx && yprev && coefs && sums && ws, "gconv_dgrad_bnbwd: null pointer");
-  UB_CHECK_ARG(ld_yprev >= d->N, "gconv_dgrad_bnbwd: ld_yprev < N");
-  UB_CHECK_ARG(unetb200_gconv_dgrad_bnbwd_supported(d, g, wp, gx),
-               "gconv_dgrad_bnbwd: shape not covered by the fused kernel (query _supported first and run gconv_fprop + "
-               "bn_relu_bwd_reduce instead)");
-  if (halo_bnbwd_supported(d, g, wp, gx))
-    return halo_fprop(d, g, wp, gx, sums, ws, nullptr, (cudaStream_t)stream, yprev, (long long)ld_yprev, coefs);
-  return tc3_fprop(d, gd, g, wp, gx, sums, ws, (cudaStream_t)stream, nullptr, yprev, (long long)ld_yprev, coefs);
-}
-
-// last conv of the network in inference: conv3x3 -> BatchNorm(eval) -> ReLU -> OutConv 1x1 + bias in one kernel
-int unetb200_gconv_fprop_affine_relu_outconv_supported(const unetb200_gconv_t* d, const void* x, const void* wp,
-                                                       int ncls) {
-  GconvDev g;
-  if (gconv_validate(d, &g)) return 0;
-  static const bool off = getenv("UNETB200_NO_BN_FOLD") != nullptr || getenv("UNETB200_NO_OUTCONV_FOLD") != nullptr;
-  if (off || d->algo == UNETB200_ALGO_SIMT || !aligned16(x) || !aligned16(wp)) return 0;
-  return tc3_affine_outconv_supported(d, ncls);
-}
-
-int unetb200_gconv_fprop_affine_relu_outconv(const unetb200_gconv_t* d, const void* x, const void* wp,
-                                             const float* scale_shift, const float* oc_w, const float* oc_b,
-                                             void* logits, int ncls, void* stream) {
-  GconvDev g;
-  int rc = gconv_validate(d, &g);
-  if (rc) return rc;
-  UB_CHECK_ARG(x && wp && scale_shift && oc_w && logits, "gconv_fprop_affine_relu_outconv: null pointer");
-  UB_CHECK_ARG(unetb200_gconv_fprop_affine_relu_outconv_supported(d, x, wp, ncls),
-               "gconv_fprop_affine_relu_outconv: shape not covered (query _supported first)");
-  Tc3OutConv oc = {oc_w, oc_b, logits, ncls};
-  return tc3_fprop(d, g, x, wp, logits, nullptr, nullptr, (cudaStream_t)stream, scale_shift, nullptr, 0, nullptr, &oc);
-}
-
-int unetb200_gconv_wgrad_plan(const unetb200_gconv_t* d, int* splits, int* algo_used) {
-  GconvDev g;
-  int rc = gconv_validate(d, &g);
-  if (rc) return rc;
-  int algo = d->algo;
-  if (first_narrow_supported(d, nullptr)) {               // C_in = 1 -> 8 / 16 / 32 channels
-    if (algo_used) *algo_used = UNETB200_ALGO_SIMT;
-    if (splits) *splits = first_narrow_wgrad_splits(d);
-    return 0;
-  }
-  if (algo != UNETB200_ALGO_SIMT && halo_wgrad_supported(d, nullptr, nullptr)) {        // 16 / 32 / 64 channels: TMA boxes
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    if (splits) *splits = halo_wgrad_splits(d);
-    return 0;
-  }
-  if (algo != UNETB200_ALGO_SIMT && halo_t_wgrad_supported(d, nullptr, nullptr)) {      // narrow ConvTranspose2d
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    if (splits) *splits = halo_t_wgrad_splits(d);
-    return 0;
-  }
-  if (algo != UNETB200_ALGO_SIMT && narrow_wgrad_supported(d, nullptr, nullptr)) {      // narrow channel counts
-    if (algo_used) *algo_used = UNETB200_ALGO_TC;
-    if (splits) *splits = narrow_wgrad_splits(d);
-    return 0;
-  }
-  if (algo == UNETB200_ALGO_AUTO || algo == UNETB200_ALGO_PREFER_TC) algo = tc_wgrad_supported(d, nullptr, nullptr) ? UNETB200_ALGO_TC : UNETB200_ALGO_SIMT;
-  if (algo == UNETB200_ALGO_TC)
-    UB_CHECK_ARG(tc_wgrad_supported(d, nullptr, nullptr), "gconv_wgrad: tcgen05 path requested but shape unsupported");
-  if (algo_used) *algo_used = algo;
-  if (splits) {
-    if (algo == UNETB200_ALGO_TC)
-      *splits = tc4_wgrad_preferred(d) ? tc4_wgrad_splits(d)
-                : tc3_wgrad_supported(d, nullptr, nullptr) ? tc3_wgrad_splits(d) : tc2_wgrad_splits(d);
-    else if (first_wgrad_supported(d, nullptr)) *splits = first_wgrad_splits(d);
-    else if (wgrad_narrow_f32_supported(d, nullptr, nullptr)) *splits = wgrad_narrow_f32_splits(d);
-    else *splits = simt_wgrad_splits(g);
-  }
-  return 0;
-}
-
-int unetb200_gconv_wgrad(const unetb200_gconv_t* d, const void* x, const void* gy, float* partials, int splits,
-                         void* stream) {
-  GconvDev g;
-  int rc = gconv_validate(d, &g);
-  if (rc) return rc;
-  UB_CHECK_ARG(x && gy && partials && splits >= 1, "gconv_wgrad: null pointer / bad splits");
-  cudaStream_t s = (cudaStream_t)stream;
-  int algo = d->algo;
-  if (first_narrow_supported(d, nullptr)) {
-    UB_CHECK_ARG(first_narrow_supported(d, gy), "gconv_wgrad: the first-layer kernel needs a 16-byte aligned gradient");
-    return first_narrow_wgrad(d, x, gy, partials, splits, s);
-  }
-  if (algo != UNETB200_ALGO_SIMT && halo_wgrad_supported(d, nullptr, nullptr)) {
-    UB_CHECK_ARG(halo_wgrad_supported(d, x, gy), "gconv_wgrad: the TMA-staged narrow kernel needs 16-byte aligned operands");
-    return halo_wgrad(d, x, gy, partials, splits, s);
-  }
-  if (algo != UNETB200_ALGO_SIMT && halo_t_wgrad_supported(d, nullptr, nullptr)) {
-    UB_CHECK_ARG(halo_t_wgrad_supported(d, x, gy), "gconv_wgrad: the TMA-staged narrow kernel needs 16-byte aligned operands");
-    return halo_t_wgrad(d, x, gy, partials, splits, s);
-  }
-  if (algo != UNETB200_ALGO_SIMT && narrow_wgrad_supported(d, nullptr, nullptr)) {
-    UB_CHECK_ARG(narrow_wgrad_supported(d, x, gy), "gconv_wgrad: the narrow tcgen05 kernel needs 16-byte aligned operands");
-    return narrow_wgrad(d, x, gy, partials, splits, s);
-  }
-  if (algo == UNETB200_ALGO_AUTO || algo == UNETB200_ALGO_PREFER_TC) algo = tc_wgrad_supported(d, nullptr, nullptr) ? UNETB200_ALGO_TC : UNETB200_ALGO_SIMT;
-  if (algo == UNETB200_ALGO_TC) {
-    UB_CHECK_ARG(tc_wgrad_supported(d, x, gy), "gconv_wgrad: tcgen05 path requested but shape/alignment unsupported");
-    if (tc4_wgrad_preferred(d)) {
-      UB_CHECK_ARG(tc4_wgrad_supported(d, x, gy), "gconv_wgrad: tcgen05 path needs 16-byte aligned operands");
-      return tc4_wgrad(d, g, x, gy, partials, splits, s);
-    }
-    if (tc3_wgrad_supported(d, nullptr, nullptr)) {
-      UB_CHECK_ARG(tc3_wgrad_supported(d, x, gy), "gconv_wgrad: tcgen05 path needs 16-byte aligned operands");
-      return tc3_wgrad(d, g, x, gy, partials, splits, s);
-    }
-    UB_CHECK_ARG(tc2_wgrad_supported(d, x, gy), "gconv_wgrad: tcgen05 path needs 16-byte aligned operands");
-    return tc2_wgrad(d, g, x, gy, partials, splits, s);
-  }
-  if (first_wgrad_supported(d, nullptr)) {
-    UB_CHECK_ARG(first_wgrad_supported(d, gy) && splits == first_wgrad_splits(d),
-                 "gconv_wgrad: first-layer kernel needs 16-byte aligned dY and the planned split count");
-    return first_wgrad(d, g, x, gy, partials, splits, s);
-  }
-  if (wgrad_narrow_f32_supported(d, nullptr, nullptr)) {
-    UB_CHECK_ARG(wgrad_narrow_f32_supported(d, x, gy), "gconv_wgrad: the narrow fp32 kernel needs 16-byte aligned operands");
-    return wgrad_narrow_f32(d, x, gy, partials, splits, s);
-  }
+int simt_wgrad(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* gy, float* partials, int splits,
+               cudaStream_t s) {
   long long mper = (g.M + splits - 1) / splits;
   mper = (mper + WBM - 1) / WBM * WBM;
   const int wbn = simt_fbn(g.N), wbk = simt_wbk(g.N);
@@ -983,6 +691,12 @@ int unetb200_gconv_wgrad(const unetb200_gconv_t* d, const void* x, const void* g
   UB_LAUNCH_CHECK("gconv_wgrad_simt");
   return 0;
 }
+
+}  // namespace ub
+
+using namespace ub;
+
+extern "C" {
 
 int unetb200_wgrad_reduce(const float* partials, int splits, int ntaps, int Cin, int N, int Cq, float* dst,
                           int64_t st, int64_t sc, int64_t sq, int64_t sn, int accumulate, void* stream) {

@@ -160,20 +160,13 @@ struct Tc4WPlan {
   int tap[3][3];
 };
 
-static int tc4_mode() {
-  // UNETB200_TC4W=0: off; =all: also the layers the CTA-pair kernel (tc3_wgrad) covers (A/B runs)
-  static const int mode = [] {
-    const char* e = getenv("UNETB200_TC4W");
-    if (!e) return 1;
-    if (!strcmp(e, "0")) return 0;
-    if (!strcmp(e, "all")) return 2;
-    return 1;
-  }();
-  return mode;
-}
-
 static bool tc4_wgrad_plan(const unetb200_gconv_t* d, Tc4WPlan* w) {
-  if (tc4_mode() == 0) return false;
+  // UNETB200_TC4W=0: off, for A/B runs (=all is read by the route in gconv.cu)
+  static const bool off = [] {
+    const char* e = getenv("UNETB200_TC4W");
+    return e && !strcmp(e, "0");
+  }();
+  if (off) return false;
   if (d->dtype != UNETB200_BF16) return false;
   if (d->nquad != 1 || d->in_scale != 1 || d->out_scale != 1 || d->ntaps != 9) return false;
   if (d->in_off_y || d->in_off_x) return false;
@@ -200,13 +193,6 @@ int tc4_wgrad_supported(const unetb200_gconv_t* d, const void* x, const void* gy
   if (!tc4_wgrad_plan(d, &w)) return 0;
   if ((x && !aligned16(x)) || (gy && !aligned16(gy))) return 0;
   return 1;
-}
-
-// 1 = this kernel is the better choice for the shape (the CTA-pair kernel needs C_in >= 256 and N % 128 == 0)
-int tc4_wgrad_preferred(const unetb200_gconv_t* d) {
-  if (!tc4_wgrad_supported(d, nullptr, nullptr)) return 0;
-  if (tc4_mode() == 2) return 1;
-  return tc3_wgrad_supported(d, nullptr, nullptr) ? 0 : 1;
 }
 
 int tc4_wgrad_splits(const unetb200_gconv_t* d) {

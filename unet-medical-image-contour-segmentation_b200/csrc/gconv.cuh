@@ -1,4 +1,5 @@
-// Device-side view of unetb200_gconv_t and the dispatch hooks between the SIMT and tcgen05 engines.
+// Device-side view of unetb200_gconv_t and the engines of the generalised convolution: each engine's shape check,
+// split count and launcher.  gconv.cu routes a descriptor to one of them.
 #pragma once
 #include "common.cuh"
 
@@ -14,8 +15,6 @@ struct GconvDev {
   long long M;   // B*Hm*Wm
   int K;         // ntaps*Cin
 };
-
-int gconv_validate(const unetb200_gconv_t* d, GconvDev* out);
 
 // Split count for a split-K grid of `tiles` work items per split on `slots` one-per-SM execution slots (SMs, or SM
 // pairs for cluster kernels): these kernels hold a whole SM each, so the grid runs in waves and a grid of 2.03
@@ -40,10 +39,17 @@ inline int pick_splits(long long tiles, int slots, long long smax) {
   return (int)pick;
 }
 
-// tcgen05 engines, common gate (tc_host.cu): 1 when the shape/dtype/alignment fits one of the kernel generations.
-int tc_fprop_supported(const unetb200_gconv_t* d, const void* x, const void* wp, const void* y);
-int tc_wgrad_supported(const unetb200_gconv_t* d, const void* x, const void* gy);
+// CUDA-core implicit GEMM for any shape, the arithmetic of the exact-fp32 mode (conv_simt.cu)
+long long simt_fprop_tiles(const GconvDev& g);
+int simt_fprop(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* wp, const float* bias, void* y,
+               double* stats, float* stats_ws, cudaStream_t s);
+int simt_wgrad_splits(const GconvDev& g);
+int simt_wgrad(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* gy, float* partials, int splits,
+               cudaStream_t s);
 int launch_stats_reduce(const float* ws, long long ntiles, int C2, double* stats, cudaStream_t s);
+
+// tcgen05 engines, the layout conditions every kernel generation shares (tc_host.cu)
+bool tc_common_ok(const unetb200_gconv_t* d);
 
 // persistent tcgen05 engine, second generation (conv_tc2.cu)
 int tc2_fprop_supported(const unetb200_gconv_t* d, const void* x, const void* wp, const void* y);
@@ -79,7 +85,6 @@ int tc3_wgrad(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const
 
 // N-stacked wgrad for the narrow 3x3 layers, fourth generation (conv_tc4.cu)
 int tc4_wgrad_supported(const unetb200_gconv_t* d, const void* x, const void* gy);
-int tc4_wgrad_preferred(const unetb200_gconv_t* d);
 int tc4_wgrad_splits(const unetb200_gconv_t* d);
 int tc4_wgrad(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* gy, float* partials, int splits,
               cudaStream_t stream);

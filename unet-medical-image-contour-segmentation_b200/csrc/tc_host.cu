@@ -111,7 +111,7 @@ int encode_weights(CUtensorMap* m, int dtype, const void* base, int K, int N, in
   return 0;
 }
 
-static bool tc_common_ok(const unetb200_gconv_t* d) {
+bool tc_common_ok(const unetb200_gconv_t* d) {
   const int esz = d->dtype == UNETB200_BF16 ? 2 : 4;
   const int epr = 128 / esz;
   const int Cq = d->N / d->nquad;
@@ -126,19 +126,4 @@ static bool tc_common_ok(const unetb200_gconv_t* d) {
   return true;
 }
 
-int tc_fprop_supported(const unetb200_gconv_t* d, const void* x, const void* wp, const void* y) {
-  if (d->dtype != UNETB200_BF16 && d->dtype != UNETB200_F32) return 0;
-  if (d->dtype == UNETB200_F32 && d->algo != UNETB200_ALGO_TC && d->algo != UNETB200_ALGO_PREFER_TC) return 0;   // fp32 defaults to exact FMA
-  if (!tc_common_ok(d)) return 0;
-  if (!aligned16(x) || !aligned16(wp) || !aligned16(y)) return 0;
-  return tc3_fprop_supported(d, x, wp, nullptr, y) || tc2_fprop_supported(d, x, wp, y);
-}
-
-int tc_wgrad_supported(const unetb200_gconv_t* d, const void* x, const void* gy) {
-  if (d->dtype != UNETB200_BF16 && d->dtype != UNETB200_F32) return 0;
-  if (d->dtype == UNETB200_F32 && d->algo != UNETB200_ALGO_TC && d->algo != UNETB200_ALGO_PREFER_TC) return 0;
-  if (!tc_common_ok(d) || d->in_scale != 1) return 0;
-  if ((x && !aligned16(x)) || (gy && !aligned16(gy))) return 0;
-  return tc4_wgrad_supported(d, x, gy) || tc3_wgrad_supported(d, x, gy) || tc2_wgrad_supported(d, x, gy);
-}
 }  // namespace ub
