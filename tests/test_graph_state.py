@@ -2,10 +2,11 @@
 
 The library caches packed weight operands (functional._PRE) and eval-mode BatchNorm coefficients
 (functional._EVAL_COEFS), lets kernels write gradients straight into registered sinks, and batches the split
-reductions of weight gradients (ops._REDUCE_JOBS).  These tests drive a model through several modes in a row --
-CUDA-graph replays then evaluation, replays then an eager step, SegmentedStep on every model variant, a backward
-pass that raises and its retry, gradient consumers inside backward -- and compare each result with a fresh model or
-with a plain PyTorch-CPU fp32 restatement of the same operation.  The last test checks the reduction queue on the CPU.
+reductions of weight gradients in the record of the running backward pass (unetb200.backward_pass).  These tests
+drive a model through several modes in a row -- CUDA-graph replays then evaluation, replays then an eager step,
+SegmentedStep on every model variant, a backward pass that raises and its retry, gradient consumers inside backward
+-- and compare each result with a fresh model or with a plain PyTorch-CPU fp32 restatement of the same operation.  The
+last tests check the per-pass record (reduction queue, gradient hand-offs, end-of-pass callback) on the CPU.
 """
 import os
 import socket
@@ -48,15 +49,12 @@ def precision(request, monkeypatch):
 
 @pytest.fixture
 def clean_queues():
-    """Host-side reset of the reduction queue and side-stream bookkeeping after a test, so that a failure in one test
-    can never leave work behind that a later backward pass would launch."""
+    """Host-side reset of the backward-pass record (reduction queue, side-stream bookkeeping, hand-offs) after a
+    test, so that a failure in one test can never leave work behind that a later backward pass would launch."""
     yield
-    from unetb200 import ops
+    from unetb200 import backward_pass
     torch.cuda.synchronize()
-    ops._REDUCE_JOBS.clear()
-    ops._REDUCE_PENDING[0] = None
-    ops._SIDE_KEEP.clear()
-    ops._SIDE_PENDING[0] = False
+    backward_pass._PASS[0] = None
 
 
 def _ctx(mode):
@@ -282,9 +280,9 @@ class _Boom(RuntimeError):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("wgrad_side", [False, True])
-def test_failed_backward_then_retry(wgrad_side, monkeypatch, clean_queues):
+def test_failed_backward_drops_its_record_then_retry(wgrad_side, monkeypatch, clean_queues):
     from oracle import unet_oracle as O
-    from unetb200 import ops
+    from unetb200 import backward_pass, ops
     monkeypatch.setenv("UNET_B200_PRECISION", "fp32")
     monkeypatch.setattr(ops, "_WGRAD_SIDE", wgrad_side)
     st = O.build_state(1, 2, False, seed=0)
@@ -305,8 +303,9 @@ def test_failed_backward_then_retry(wgrad_side, monkeypatch, clean_queues):
         loss.backward()          # inc's backward runs last: the other stages' weight gradients are done by now
     del m.inc.run, loss
     _loss(m, x, t, "bf16")       # a forward only: its graph is dropped at once
-    assert not ops._REDUCE_JOBS, "reductions of the failed pass are still queued"
-    assert not ops._SIDE_KEEP, "operands of the failed pass are still held for the side stream"
+    rec = backward_pass._PASS[0]
+    assert rec is None or not rec.jobs, "reductions of the failed pass are still queued"
+    assert rec is None, "operands or hand-offs of the failed pass are still held"
 
     m.use_checkpointing()
     for p in m.parameters():
@@ -460,22 +459,25 @@ def test_stock_ddp_world1(gloo_world1, monkeypatch):
 
 
 # ------------------------------------------------------------------------------------------------
-# f. the reduction queue on the CPU: nothing of an aborted pass reaches the next pass's flush
+# f. the per-pass record on the CPU: nothing of an aborted pass reaches the next pass
 # ------------------------------------------------------------------------------------------------
-def test_reduce_queue_drops_jobs_of_a_failed_pass(monkeypatch):
-    from unetb200 import ops
+def _record_flushes(monkeypatch):
+    """unetb200.backward_pass with an empty record, deferred reductions on, and every multi-tensor reduction recorded
+    (as the list of its destination addresses) instead of launched."""
+    from unetb200 import backward_pass, ops
     flushed = []
+    monkeypatch.setattr(backward_pass, "_PASS", [None])
+    monkeypatch.setattr(ops, "DEFER_REDUCE", True)
+    monkeypatch.setattr(backward_pass, "_reduce_multi", lambda jobs: flushed.append([j[1] for j in jobs]))
+    return backward_pass, flushed
 
-    def record():
-        flushed.append([j[1] for j in ops._REDUCE_JOBS])
-        ops._REDUCE_JOBS.clear()
-        ops._REDUCE_PENDING[0] = None
-    monkeypatch.setattr(ops, "_REDUCE_JOBS", [])
-    monkeypatch.setattr(ops, "_REDUCE_PENDING", [None])
-    monkeypatch.setattr(ops, "flush_wgrad_reduce", record)
 
-    def job(dst):
-        return (torch.zeros(4), dst, 1, 1, 0, 1, 2, 1, 1, 1, 1)
+def _job(dst):
+    return (torch.zeros(4), dst, 1, 1, 0, 1, 2, 1, 1, 1, 1)
+
+
+def test_pass_record_drops_jobs_of_a_failed_pass(monkeypatch):
+    backward_pass, flushed = _record_flushes(monkeypatch)
 
     class Queue(torch.autograd.Function):
         @staticmethod
@@ -485,7 +487,7 @@ def test_reduce_queue_drops_jobs_of_a_failed_pass(monkeypatch):
 
         @staticmethod
         def backward(ctx, g):
-            ops._queue_reduce(job(ctx.dst))
+            backward_pass.defer_reduce(_job(ctx.dst), "pass")
             if ctx.fail:
                 raise _Boom("backward failed")
             return g * 2, None, None
@@ -497,5 +499,88 @@ def test_reduce_queue_drops_jobs_of_a_failed_pass(monkeypatch):
     Queue.apply(x, 0x2000, False).sum().backward()
     assert flushed == [[0x2000]], f"the flush saw {flushed}"
     # outside any backward pass a job is reduced at once
-    ops._queue_reduce(job(0x3000))
+    backward_pass.defer_reduce(_job(0x3000), "pass")
     assert flushed[-1] == [0x3000]
+
+
+class _InBackward(torch.autograd.Function):
+    """Identity whose backward calls `fn()`: the library's bookkeeping as a Function's backward does it."""
+
+    @staticmethod
+    def forward(ctx, x, fn):
+        ctx.fn = fn
+        return x.clone()
+
+    @staticmethod
+    def backward(ctx, g):
+        ctx.fn()
+        return g, None
+
+
+def _backward_running(fn):
+    _InBackward.apply(torch.ones(3, requires_grad=True), fn).sum().backward()
+
+
+def test_hand_off_of_a_failed_pass_is_never_taken(monkeypatch):
+    backward_pass, _ = _record_flushes(monkeypatch)
+    g = torch.zeros(2, 3)
+
+    def leave_and_fail():
+        backward_pass.leave("bn_sums", g, "sums of the failed pass")
+        raise _Boom("backward failed")
+    taken = []
+    with pytest.raises(_Boom):
+        _backward_running(leave_and_fail)
+    _backward_running(lambda: taken.append(backward_pass.take("bn_sums", g)))
+    with pytest.raises(_Boom):
+        _backward_running(leave_and_fail)
+    backward_pass.begin_forward()
+    assert backward_pass._PASS[0] is None, "a forward entry outside backward keeps the failed pass's record"
+    _backward_running(lambda: taken.append(backward_pass.take("bn_sums", g)))
+    assert taken == [None, None]
+
+
+def test_one_end_of_pass_callback_per_pass(monkeypatch):
+    """Queued reductions and hand-offs share the pass's record and its one engine callback."""
+    backward_pass, flushed = _record_flushes(monkeypatch)
+
+    class CountingEngine:
+        def __init__(self, engine):
+            self.engine, self.callbacks = engine, 0
+
+        def queue_callback(self, cb):
+            self.callbacks += 1
+            return self.engine.queue_callback(cb)
+
+        def __getattr__(self, name):
+            return getattr(self.engine, name)
+    engine = CountingEngine(torch.autograd.Variable._execution_engine)
+    monkeypatch.setattr(torch.autograd.Variable, "_execution_engine", engine)
+    g = torch.zeros(2, 3)
+
+    def work():
+        backward_pass.defer_reduce(_job(0x1000), "pass")
+        backward_pass.leave("bn_sums", g, "sums")
+        backward_pass.defer_reduce(_job(0x2000), "pass")
+        backward_pass.leave("colsum", g, "column sums", token=object())
+    _backward_running(work)
+    assert engine.callbacks == 1
+    assert flushed == [[0x1000, 0x2000]]
+    assert backward_pass._PASS[0] is None, "the record outlived its pass"
+
+
+def test_hand_off_matches_address_shape_and_token(monkeypatch):
+    backward_pass, _ = _record_flushes(monkeypatch)
+    g = torch.zeros(2, 3)
+    token = object()
+    got = {}
+
+    def work():
+        backward_pass.leave("bn_sums", g, "sums")
+        got["other shape"] = backward_pass.take("bn_sums", g.view(3, 2))
+        backward_pass.leave("colsum", g, "column sums", token=token)
+        got["other token"] = backward_pass.take("colsum", g, token=object())
+        backward_pass.leave("colsum", g, "column sums", token=token)
+        got["match"] = backward_pass.take("colsum", g, token=token)
+    _backward_running(work)
+    assert got == {"other shape": None, "other token": None, "match": "column sums"}

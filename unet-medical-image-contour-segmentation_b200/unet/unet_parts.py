@@ -10,8 +10,8 @@ hand-written sm_100a kernels through the C ABI; there is no cuDNN/ATen and no CP
 import torch
 import torch.nn as nn
 
+from unetb200 import backward_pass, ops
 from unetb200 import functional as UF
-from unetb200 import ops
 from unetb200.functional import _Cfg
 
 
@@ -27,7 +27,7 @@ def _to_internal(x, dtype):
 def _prep(x, what):
     """Caller tensor (fp32 NCHW-logical, usually channels_last) -> NHWC of the compute dtype."""
     ops.require_cuda(x, what)
-    UF.begin_forward()
+    backward_pass.begin_forward()
     if x.dim() != 4:
         raise ValueError(f"{what}: expected a [B, C, H, W] tensor, got {tuple(x.shape)}")
     return _to_internal(x, UF.compute_dtype(x))

@@ -3,6 +3,7 @@
 ``_lib``        ctypes binding of libunetb200.so (C ABI: include/unetb200.h)
 ``ops``         tensor-level wrappers (pointer / shape / stream marshalling only)
 ``functional``  torch.autograd.Function per UNet part
+``backward_pass`` what a backward pass owns outside autograd (deferred reductions, side stream, hand-offs)
 ``losses``      dice / boundary / fused CE+dice
 ``ddp``         data-parallel gradient all-reduce (NCCL) overlapped with backward
 ``graph``       whole-step CUDA graph
@@ -12,4 +13,4 @@
 """
 from . import _lib  # noqa: F401
 
-__all__ = ["_lib", "ops", "functional", "losses", "ddp", "graph", "optim", "eval_tail", "data"]
+__all__ = ["_lib", "ops", "functional", "backward_pass", "losses", "ddp", "graph", "optim", "eval_tail", "data"]

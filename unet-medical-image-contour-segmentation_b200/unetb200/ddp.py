@@ -26,14 +26,7 @@ from __future__ import annotations
 import torch
 import torch.distributed as dist
 
-
-def _side_stream_sync():
-    try:
-        from . import ops
-    except Exception:  # noqa: BLE001  (CPU-only use of this module in the gloo tests)
-        return
-    if torch.cuda.is_available():
-        ops.side_stream_sync()
+from . import backward_pass
 
 
 def _functional():
@@ -284,7 +277,7 @@ class GradAllReducer:
     # optimizer graph
     def pack_all(self):
         """Bring every gradient into its bucket (no communication)."""
-        _side_stream_sync()
+        backward_pass.side_stream_sync()
         for b in self.buckets:
             self._fill(b)
 
@@ -331,7 +324,7 @@ class GradAllReducer:
             self._launch(b)
 
     def _launch(self, b):
-        _side_stream_sync()          # weight gradients may be produced on the library's side stream
+        backward_pass.side_stream_sync()    # weight gradients may be produced on the library's side stream
         self._fill(b)
         b["work"] = self._allreduce(b)
         self.launched += 1

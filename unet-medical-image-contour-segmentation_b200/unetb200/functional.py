@@ -16,7 +16,7 @@ import os
 
 import torch
 
-from . import _lib, ops
+from . import _lib, backward_pass, ops
 from ._lib import ALGO_AUTO, ALGO_PREFER_TC, ALGO_SIMT
 
 
@@ -240,21 +240,21 @@ def grad_dst(param, like=None):
 # ------------------------------------------------------------------------------------------------
 # forward: a conv-BN-ReLU stage registers, for its activation z = relu(bn(y)), the pair (y, coefs) that its backward
 # reduction needs; the consumer of z (OutConv, ...) looks it up and saves it.  backward: the consumer's kernel writes
-# the gradient g of z and, in the same pass, sum(g*mask) / sum(g*mask*xhat); it leaves them here keyed by g's
-# storage, and the stage's own backward takes them instead of running unetb200_bn_relu_bwd_reduce.
+# the gradient g of z and, in the same pass, sum(g*mask) / sum(g*mask*xhat); it leaves them for g
+# (backward_pass.leave "bn_sums"), and the stage's own backward takes them instead of running
+# unetb200_bn_relu_bwd_reduce.
 _BNBWD_MIN_N = int(os.environ.get("UNETB200_BNBWD_MIN_N", "0"))        # A/B switches: fuse only for these widths
 _BNBWD_MAX_N = int(os.environ.get("UNETB200_BNBWD_MAX_N", "1000000"))
 _BN_OF_ACT = {}    # data_ptr(z) -> (weakref(y), weakref(coefs), shape)
-_GRAD_SUMS = {}    # data_ptr(g) -> (sums, shape)
 
 
 # Column sums of a gradient made by the dgrad that writes it: the ConvTranspose2d bias gradient (unet_parts.py:73) is
 # the per-channel sum of the `up` half of the concat gradient, which the decoder's first conv's dgrad produces -- its
-# epilogue already knows how to sum the tile it stores (the forward BatchNorm statistics path).
-# Both hand-offs carry a per-call token, so an entry that was never consumed can never be mistaken for another call's
-# (addresses repeat once the allocator recycles a block).
+# epilogue already knows how to sum the tile it stores (the forward BatchNorm statistics path); the sums are left for
+# the concat gradient (backward_pass.leave "colsum").
+# Both the request and the hand-off carry a per-call token, so an entry that was never consumed can never be mistaken
+# for another call's (addresses repeat once the allocator recycles a block).
 _WANT_COLSUM = {}    # data_ptr(concat buffer) -> (shape, token): registered by UpCatConvTFn.forward, read by DoubleConvFn.forward
-_GRAD_COLSUM = {}    # data_ptr(concat gradient) -> (fp64 stats[2*C], shape, token)
 COLSUM_FUSE = os.environ.get("UNETB200_COLSUM_FUSE", "1") != "0"
 
 
@@ -274,31 +274,6 @@ def bn_of(z):
     if y is None or coefs is None or y.shape != z.shape or y.dtype != z.dtype:
         return None
     return y, coefs
-
-
-def begin_forward():
-    """Entry of a drop-in forward pass.  Outside any backward pass, whatever a backward pass left queued or handed
-    off belongs to a pass that raised (train.py's OOM retry takes this route): drop it before it can reach the next
-    pass.  Inside one (re-computation under use_checkpointing) nothing changes."""
-    if _GRAD_SUMS or _GRAD_COLSUM:
-        task = ops.graph_task()
-        if task is not None and task < 0:
-            _GRAD_SUMS.clear()
-            _GRAD_COLSUM.clear()
-    ops.drop_aborted_work_if_idle()
-
-
-def leave_grad_sums(g, sums):
-    if len(_GRAD_SUMS) > 64:
-        _GRAD_SUMS.clear()
-    _GRAD_SUMS[g.data_ptr()] = (sums, tuple(g.shape))
-
-
-def take_grad_sums(g):
-    ent = _GRAD_SUMS.pop(g.data_ptr(), None)
-    if ent is None or ent[1] != tuple(g.shape):
-        return None
-    return ent[0]
 
 
 def _f32c(t):
@@ -488,17 +463,26 @@ def _sink_owns(param, dW):
             and not torch.is_grad_enabled())
 
 
-def _defer_mode(param, dW, kept, side):
-    """gconv_wgrad's `defer` for the weight gradient dW of `param`: "pass" when a data-parallel sink owns it (its split
-    reduction joins the one launch at the end of the backward pass); "call" when autograd keeps dW as it is (one
-    launch for the layers of the running Function's backward, before autograd sees dW); else, and on the side stream,
-    the reduction follows its wgrad.  Deferred reductions all run on the multi-tensor kernel, whose per-layer
-    summation order does not depend on how the layers are grouped."""
-    if side:
-        return False
-    if _sink_owns(param, dW):
-        return "pass"
-    return "call" if kept else False
+def _weight_grad(param, like, shape, launch, *keep):
+    """dW = weight gradient of `param` (shape `shape`), made by launch(dW, defer) after the layer's data gradient.
+
+    dW is the parameter's gradient sink, else a tensor in the parameter's own layout (`like`'s: OIHW or channels_last,
+    so AccumulateGrad keeps it without a copy), else -- taps not linear in memory -- a contiguous one.  When
+    AccumulateGrad will simply keep dW the launch may go to the side stream (it overlaps the memory-bound BatchNorm
+    backward of the previous layer); else gconv_wgrad's `defer` is "pass" when a data-parallel sink owns dW, "call" when
+    autograd keeps dW as it is, False when it would accumulate or re-layout dW at once.  Deferred reductions all run on
+    the multi-tensor kernel, whose per-layer summation order does not depend on how the layers are grouped."""
+    dW = grad_dst(param)
+    if dW is None:
+        dW = torch.empty_like(like, dtype=torch.float32)
+    if dW.shape != shape or dW.stride(2) != shape[3] * dW.stride(3):
+        dW = torch.empty(shape, dtype=torch.float32, device=like.device)
+    kept = _grad_kept_as_is(param, dW)
+    if kept and backward_pass.wgrad_on_side_stream():
+        backward_pass.on_side_stream(lambda: launch(dW, False), *keep)
+    else:
+        launch(dW, "pass" if _sink_owns(param, dW) else "call" if kept else False)
+    return dW
 
 
 def _vec_dst(param, Cc):
@@ -522,16 +506,6 @@ def conv_bn_relu_bwd(gz, x, y, w, coefs, batch_stats, need_gx, param=None, bn_pa
     cd = x.dtype
     gy, dgamma, dbeta = ops.bn_relu_bwd(gz, y, coefs, batch_stats, _vec_dst(bn_params[0], Cout),
                                         _vec_dst(bn_params[1], Cout), sums=sums, peer=peer)
-    # the gradient takes the parameter's own memory layout (OIHW or channels_last): AccumulateGrad then keeps it
-    # without a copy, and for channels_last the split reduction writes it coalesced; with a registered sink
-    # (data-parallel bucket view) it is written there
-    dW = grad_dst(param)
-    if dW is None:
-        dW = torch.empty_like(w, dtype=torch.float32)
-    so, si, skh, skw = dW.stride()
-    if skh != 3 * skw or dW.shape != (Cout, Cin, 3, 3):
-        dW = torch.empty((Cout, Cin, 3, 3), dtype=torch.float32, device=x.device)
-        so, si, skh, skw = dW.stride()
     gx = None
     dw_desc = _gconv3x3(x, Cout, gy, cd)
     gs = ops.x3_split(gy) if (ops.x3_active(dw_desc) and Cout >= 16) else None   # 3xTF32: one split serves both GEMMs
@@ -547,21 +521,11 @@ def conv_bn_relu_bwd(gz, x, y, w, coefs, batch_stats, need_gx, param=None, bn_pa
             # x is an Up stage's concat buffer: leave the per-channel sums of its gradient for the ConvTranspose bias
             cs = torch.zeros(2 * Cin, dtype=torch.float64, device=x.device)
             ops.gconv_fprop(dd, gy, wd, None, gx, cs, kind="dgrad")
-            if len(_GRAD_COLSUM) > 16:
-                _GRAD_COLSUM.clear()
-            _GRAD_COLSUM[gx.data_ptr()] = (cs, tuple(gx.shape), colsum)
+            backward_pass.leave("colsum", gx, cs, token=colsum)
         else:
             ops.gconv_fprop(dd, gy, wd, None, gx, None, kind="dgrad", x_split=gs)
-    # after the dgrad, on the side stream: overlaps the (memory-bound) BatchNorm backward of the previous layer
-    # (only when AccumulateGrad will simply keep dW: an existing .grad would be accumulated into on the main stream)
-    kept = _grad_kept_as_is(param, dW)
-    side = kept and ops.wgrad_on_side_stream()
-    defer = _defer_mode(param, dW, kept, side)
-    run = lambda: ops.gconv_wgrad(dw_desc, x, gy, dW, skw, si, so, gy_split=gs, defer=defer)  # noqa: E731
-    if side:
-        ops.on_side_stream(run, x, gy)      # AccumulateGrad keeps dW as it is (same layout, no other owner)
-    else:
-        run()                               # (else it would accumulate / re-layout dW on the main stream right away)
+    dW = _weight_grad(param, w, (Cout, Cin, 3, 3), lambda dW, defer: ops.gconv_wgrad(
+        dw_desc, x, gy, dW, dW.stride(3), dW.stride(1), dW.stride(0), gy_split=gs, defer=defer), x, gy)
     return gx, dW, dgamma, dbeta, sums_below
 
 
@@ -628,7 +592,7 @@ class DoubleConvFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gz2, gpooled=None):
-        with ops.reductions_at_return():          # both weight gradients complete before autograd sees them
+        with backward_pass.reductions_at_return():    # both weight gradients complete before autograd sees them
             return DoubleConvFn._backward(ctx, gz2, gpooled)
 
     @staticmethod
@@ -638,7 +602,7 @@ class DoubleConvFn(torch.autograd.Function):
         gz = ops.to_nhwc(gz2, cd) if gz2 is not None else None
         # reduction of bn2's backward already made by the kernel that wrote gz (OutConv backward)?  Only valid while
         # gz is exactly that tensor: not after the pool gradient has been accumulated into it below.
-        sums2 = take_grad_sums(gz) if gz is not None else None
+        sums2 = backward_pass.take("bn_sums", gz) if gz is not None else None
         if ctx.has_pool and gpooled is not None:
             sums2 = None
             gp = ops.to_nhwc(gpooled, cd)
@@ -742,7 +706,7 @@ class UpCatConvTFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gcat):
-        with ops.reductions_at_return():          # the weight gradient is complete before autograd sees it
+        with backward_pass.reductions_at_return():    # the weight gradient is complete before autograd sees it
             return UpCatConvTFn._backward(ctx, gcat)
 
     @staticmethod
@@ -758,39 +722,22 @@ class UpCatConvTFn(torch.autograd.Function):
         gup = ops.channel_slice(g, C2, Cup)
         ld = ops.nhwc_ld(g)
         dW = dB = gx1 = None
-        if need[2]:
-            d = ops.make_gconv(ops._DT[cd], conv_algo(cd), B, h, w, C1, ops.TAPS1, 1, (0, 0), h, w, ops.nhwc_ld(x1),
-                               4 * Cup, 4, 2, off, H, W, ld)
-            # gradient in the parameter's own layout (see conv_bn_relu_bwd); quadrant q = kh*2 + kw must stay linear
-            pT = getattr(ctx, "param_obj", wT)
-            dW = grad_dst(pT)
-            if dW is None:
-                dW = torch.empty_like(wT, dtype=torch.float32)
-            if dW.shape != (C1, Cup, 2, 2) or dW.stride(2) != 2 * dW.stride(3):
-                dW = torch.empty((C1, Cup, 2, 2), dtype=torch.float32, device=g.device)
-            s_ci, s_co, _, s_q = dW.stride()
         if need[0]:
             gx1 = ops.empty_nhwc(B, C1, h, w, cd, g.device)
             dd = ops.make_gconv(ops._DT[cd], conv_algo(cd), B, h, w, Cup, ops.TAPS_Q, 2, off, H, W, ld,
                                 C1, 1, 1, (0, 0), h, w, ops.nhwc_ld(gx1))
             ops.gconv_fprop(dd, gup, packT_dgrad(wT, cd), None, gx1, None, kind="convT_dgrad")
         if need[2]:
-            # after the dgrad, on the side stream (see conv_bn_relu_bwd)
-            pT = getattr(ctx, "param_obj", wT)
-            kept = _grad_kept_as_is(pT, dW)
-            side = kept and ops.wgrad_on_side_stream()
-            defer = _defer_mode(pT, dW, kept, side)
-            run = lambda: ops.gconv_wgrad(d, x1, gup, dW, 0, s_ci, s_co, sq=s_q, defer=defer)  # noqa: E731
-            if side:
-                ops.on_side_stream(run, x1, g)
-            else:
-                run()
-        cs = _GRAD_COLSUM.pop(g.data_ptr(), None)
+            d = ops.make_gconv(ops._DT[cd], conv_algo(cd), B, h, w, C1, ops.TAPS1, 1, (0, 0), h, w, ops.nhwc_ld(x1),
+                               4 * Cup, 4, 2, off, H, W, ld)
+            # dW[ci][co][kh][kw]: quadrant q = kh*2 + kw
+            dW = _weight_grad(getattr(ctx, "param_obj", wT), wT, (C1, Cup, 2, 2), lambda dW, defer: ops.gconv_wgrad(
+                d, x1, gup, dW, 0, dW.stride(0), dW.stride(1), sq=dW.stride(3), defer=defer), x1, g)
+        cs = backward_pass.take("colsum", g, token=getattr(ctx, "colsum_token", None))
         if need[3]:
             dst = _vec_dst(getattr(ctx, "bias_obj", None), Cup)
-            if (cs is not None and cs[1] == tuple(g.shape) and cs[2] is getattr(ctx, "colsum_token", None)
-                    and not padded and g is gcat):
-                dB = ops.f64_to_f32(cs[0][C2:C2 + Cup], dst)      # summed by the dgrad epilogue that wrote g
+            if cs is not None and not padded and g is gcat:
+                dB = ops.f64_to_f32(cs[C2:C2 + Cup], dst)      # summed by the dgrad epilogue that wrote g
             else:
                 region = gup if not padded else ops.to_nhwc(
                     gup[:, :, off[0]:off[0] + 2 * h, off[1]:off[1] + 2 * w].contiguous(memory_format=torch.channels_last), cd)
@@ -903,5 +850,5 @@ class OutConvFn(torch.autograd.Function):
             db = torch.empty(K, dtype=torch.float32, device=x.device)
         sums = ops.outconv_bwd(x, w2, g, gx, dw, db, below=below)
         if sums is not None:
-            leave_grad_sums(gx, sums)      # x = relu(bn(yb)): the stage below takes them in its backward
+            backward_pass.leave("bn_sums", gx, sums)      # x = relu(bn(yb)): the stage below takes them
         return gx, dw if need[1] else None, db if (need[2] and ctx.has_bias) else None, None

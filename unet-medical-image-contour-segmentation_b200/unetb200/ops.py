@@ -17,7 +17,7 @@ import os
 
 import torch
 
-from . import _lib
+from . import _lib, backward_pass
 from ._lib import ALGO_AUTO, ALGO_SIMT, ALGO_TC, BF16, F32, I64, GConv  # noqa: F401
 
 _DT = {torch.float32: F32, torch.bfloat16: BF16}
@@ -78,95 +78,6 @@ def _run(name, fn, *args, kernels=1, flops=0.0, nbytes=0.0):
         rc = fn(*args)
     LAUNCHES += kernels
     _lib.check(rc, name)
-
-
-# ------------------------------------------------------------------------------------------------
-# side stream for weight gradients
-# ------------------------------------------------------------------------------------------------
-# A weight gradient is needed only by the optimizer, while the BatchNorm backward of the previous layer (HBM bound,
-# few registers, no shared memory) needs the data gradient and is what autograd runs next.  Issuing the wgrad GEMM
-# on a second stream -- ordered after the dgrad of the same layer -- lets the memory-bound kernels of the next
-# layer run on the SM resources the tensor kernel leaves idle.  The streams are joined by an autograd-engine
-# callback at the end of the backward pass (so callers such as the reference train.py need no change), and the
-# operands are kept alive until then.  UNETB200_WGRAD_STREAM=1 turns this on (see _WGRAD_SIDE below);
-# UNETB200_SIDE_STREAM=0 disables the side stream altogether (also the operand pre-packing).
-import os as _os
-
-_SIDE = {}            # device index -> torch.cuda.Stream
-_SIDE_KEEP = []       # tensors the side stream still reads
-_SIDE_PENDING = [False]
-_SIDE_ON = _os.environ.get("UNETB200_SIDE_STREAM", "1") != "0"          # master switch (prepack + wgrad)
-# weight gradients on the side stream: OFF by default -- it paid (+4 %) while the wgrad grids had a nearly empty
-# third wave for the BatchNorm kernels to fill; with wave-exact split counts the serial order is 1-2 % faster
-_WGRAD_SIDE = _os.environ.get("UNETB200_WGRAD_STREAM", "0") != "0"
-
-
-def _wait_side(s):
-    """current stream waits for side stream `s` -- unless a CUDA-graph capture is in progress that `s` is not part
-    of (a captured stream may not wait on work outside its capture; there is then nothing pending on `s` either)."""
-    cur = torch.cuda.current_stream(s.device)
-    if torch.cuda.is_current_stream_capturing():
-        with torch.cuda.stream(s):
-            if not torch.cuda.is_current_stream_capturing():
-                return
-    cur.wait_stream(s)
-
-
-def _side_join():
-    _SIDE_PENDING[0] = False
-    for s in _SIDE.values():
-        _wait_side(s)
-    _SIDE_KEEP.clear()
-
-
-def side_stream_sync():
-    """Order the current stream after the side stream (for code that reads weight gradients DURING backward)."""
-    for s in _SIDE.values():
-        _wait_side(s)
-
-
-def side_enabled():
-    return _SIDE_ON and _PROFILE is None
-
-
-def wgrad_on_side_stream():
-    """True when on_side_stream(..., join=True) would really move the work to the side stream."""
-    return _SIDE_ON and _PROFILE is None and _WGRAD_SIDE
-
-
-def on_side_stream(fn, *keep, join=True):
-    """Run fn() on the side stream, ordered after everything enqueued so far on the current stream.  join=True
-    queues the end-of-backward join (weight gradients); join=False leaves ordering to events recorded by fn
-    (see functional.prepack)."""
-    if not _SIDE_ON or _PROFILE is not None or (join and not _WGRAD_SIDE):
-        return fn()
-    dev = torch.cuda.current_device()
-    side = _SIDE.get(dev)
-    if side is None:
-        side = _SIDE[dev] = torch.cuda.Stream(device=dev)
-    ev = torch.cuda.Event()
-    ev.record(torch.cuda.current_stream())
-    _SIDE_KEEP.extend(keep)
-    with torch.cuda.stream(side):
-        side.wait_event(ev)
-        out = fn()
-    if join:
-        # one join per backward pass, keyed by the autograd graph-task id (robust against a backward pass that
-        # raised before its callback ran); outside a backward pass: join right away
-        task = torch._C._current_graph_task_id() if hasattr(torch._C, "_current_graph_task_id") else None
-        if task is None or task < 0:
-            try:
-                if task is None and not _SIDE_PENDING[0]:
-                    _SIDE_PENDING[0] = True
-                    torch.autograd.Variable._execution_engine.queue_callback(_side_join)
-                elif task is not None:
-                    _side_join()
-            except RuntimeError:
-                _side_join()
-        elif _SIDE_PENDING[0] != ("task", task):
-            _SIDE_PENDING[0] = ("task", task)
-            torch.autograd.Variable._execution_engine.queue_callback(_side_join)
-    return out
 
 
 def _p(t):
@@ -478,103 +389,13 @@ def gconv_dgrad_bnbwd(d, g, wp, gx, yprev, coefs_prev):
     return sums
 
 
-# ------------------------------------------------------------------------------------------------
-# deferred split reductions of the weight gradients: one multi-tensor launch for several layers
-# ------------------------------------------------------------------------------------------------
-# A wgrad kernel writes `splits` partial results; reducing them layer by layer costs 22 small launches per step.
-# Two ways to batch them, both chosen per layer by functional (gconv_wgrad's `defer`):
-# * "call": the reductions queued while one Function's backward runs (functional.DoubleConvFn: both of its convs;
-#   UpCatConvTFn: its ConvTranspose) are made by ONE launch when that backward returns (`reductions_at_return`).  Autograd only sees the gradients after
-#   that, so everything that reads them during the pass -- AccumulateGrad and hooks on its node (where stock
-#   DistributedDataParallel and FSDP attach), the engine summing the two contributions of a parameter used twice --
-#   reads finished values.
-# * "pass": when a data-parallel sink owns the gradient (functional._sink_owns: the reducer drives the pass through
-#   torch.autograd.grad and is its only reader), the reduction is queued and all queued layers are reduced by ONE
-#   launch from an autograd-engine callback at the end of the pass -- for a segmented backward
-#   (ddp.segmented_backward) that is the end of each torch.autograd.grad call, i.e. before the segment's bucket is
-#   all-reduced.
-# NOTE a job keeps the partials alive but only the ADDRESS of the gradient: AccumulateGrad adopts a gradient tensor
-# without copying only while nobody else references it (use_count check) -- a reference held here would make it clone
-# the not-yet-reduced buffer.  A pass that raises never runs its callback, so its jobs must never reach a later
-# flush: a job arriving for another graph task, or a forward entry outside any backward pass
-# (`drop_aborted_work_if_idle`), finds them and drops them.
-_REDUCE_JOBS = []          # (partials, dst address, st, sc, sq, sn, splits, ntaps, Cin, N, Cq): "pass" jobs
-_REDUCE_PENDING = [None]   # graph task whose callback will flush _REDUCE_JOBS
-_CALL_JOBS = [None]        # the "call" jobs of the Function backward running now (None: outside reductions_at_return)
-DEFER_REDUCE = _os.environ.get("UNETB200_DEFER_REDUCE", "1") != "0"
-
-
-def graph_task():
-    """Id of the autograd graph task running on this thread (< 0 outside a backward pass; None on old PyTorch)."""
-    return torch._C._current_graph_task_id() if hasattr(torch._C, "_current_graph_task_id") else None
-
-
-def _reduce_multi(jobs):
-    if not jobs:
-        return
-    arr = (_lib.ReduceJob * len(jobs))()
-    nbytes = 0.0
-    for j, (partials, dst, st, sc, sq, sn, splits, ntaps, Cin, N, Cq) in enumerate(jobs):
-        arr[j].partials, arr[j].dst = partials.data_ptr(), dst
-        arr[j].st, arr[j].sc, arr[j].sq, arr[j].sn = st, sc, sq, sn
-        arr[j].splits, arr[j].ntaps, arr[j].Cin, arr[j].N, arr[j].Cq, arr[j].accumulate = splits, ntaps, Cin, N, Cq, 0
-        nbytes += 4.0 * ntaps * Cin * N * (splits + 1)
-    n = len(jobs)
-    _run("wgrad_reduce", lib().unetb200_wgrad_reduce_multi, arr, n, _stream(), nbytes=nbytes, kernels=(n + 31) // 32)
-
-
-def flush_wgrad_reduce():
-    """Reduce every queued weight gradient on the current stream (no-op when nothing is queued)."""
-    _REDUCE_PENDING[0] = None
-    try:
-        _reduce_multi(_REDUCE_JOBS)
-    finally:
-        _REDUCE_JOBS.clear()
-
-
-@contextlib.contextmanager
-def reductions_at_return():
-    """The "call" reductions queued inside the block are made by one launch when it ends without an exception."""
-    prev, _CALL_JOBS[0] = _CALL_JOBS[0], []
-    try:
-        yield
-        jobs = _CALL_JOBS[0]
-    finally:
-        _CALL_JOBS[0] = prev
-    _reduce_multi(jobs)
-
-
-def drop_aborted_work():
-    """Forget the weight-gradient work of a backward pass that raised before its end-of-pass callbacks ran: order the
-    current stream after the side stream (its kernels may still write into tensors of the failed pass), then drop the
-    queued reductions -- their destinations may have been freed and handed out again -- and the side-stream operands."""
-    side_stream_sync()
-    _SIDE_KEEP.clear()
-    _SIDE_PENDING[0] = False
-    _REDUCE_JOBS.clear()
-    _REDUCE_PENDING[0] = None
-
-
-def drop_aborted_work_if_idle():
-    """At the entry of a forward pass: outside any backward pass nothing may still be queued or held for one -- what
-    is, belongs to a pass that raised.  Inside a backward pass (re-computation under use_checkpointing) no-op."""
-    if _REDUCE_JOBS or _SIDE_KEEP or _SIDE_PENDING[0]:
-        task = graph_task()
-        if task is not None and task < 0:
-            drop_aborted_work()
-
-
-def _queue_reduce(job):
-    task = graph_task()
-    if _REDUCE_JOBS and _REDUCE_PENDING[0] != task:
-        drop_aborted_work()                          # queued by a pass whose flush callback never ran
-    _REDUCE_JOBS.append(job)
-    if task is None or task < 0:
-        flush_wgrad_reduce()                         # not inside a backward pass: nothing to wait for
-        return
-    if _REDUCE_PENDING[0] != task:
-        _REDUCE_PENDING[0] = task
-        torch.autograd.Variable._execution_engine.queue_callback(flush_wgrad_reduce)
+# Switches of the backward pass's bookkeeping (unetb200.backward_pass reads them at each use, so a script or test may
+# flip them here): batched split reductions; the side stream at all; weight gradients on it -- OFF by default: it paid
+# (+4 %) while the wgrad grids had a nearly empty third wave for the BatchNorm kernels to fill; with wave-exact split
+# counts the serial order is 1-2 % faster.
+DEFER_REDUCE = os.environ.get("UNETB200_DEFER_REDUCE", "1") != "0"
+_SIDE_ON = os.environ.get("UNETB200_SIDE_STREAM", "1") != "0"
+_WGRAD_SIDE = os.environ.get("UNETB200_WGRAD_STREAM", "0") != "0"
 
 
 def _wgrad_once(d, x, gy, dst, st, sc, sn, sq, accumulate, flops, tag, defer=False):
@@ -588,12 +409,8 @@ def _wgrad_once(d, x, gy, dst, st, sc, sn, sq, accumulate, flops, tag, defer=Fal
     _run(f"conv_wgrad_{_ALGO_NAME.get(used.value, '?')}" + tag, lib().unetb200_gconv_wgrad, C.byref(d2), _p(x), _p(gy),
          _p(partials), splits.value, _stream(), flops=flops,
          nbytes=float(es) * d.B * (d.Hin * d.Win * d.Cin + d.Hout * d.Wout * (d.N // d.nquad)) + 4.0 * K * d.N)
-    if defer and not accumulate and DEFER_REDUCE and (defer == "pass" or _CALL_JOBS[0] is not None):
-        job = (partials, dst.data_ptr(), st, sc, sq, sn, splits.value, d.ntaps, d.Cin, d.N, d.N // d.nquad)
-        if defer == "pass":
-            _queue_reduce(job)
-        else:
-            _CALL_JOBS[0].append(job)
+    if defer and not accumulate and backward_pass.defer_reduce(
+            (partials, dst.data_ptr(), st, sc, sq, sn, splits.value, d.ntaps, d.Cin, d.N, d.N // d.nquad), defer):
         return used.value
     _run("wgrad_reduce", lib().unetb200_wgrad_reduce, _p(partials), splits.value, d.ntaps, d.Cin, d.N,
          d.N // d.nquad, _p(dst), st, sc, sq, sn, 1 if accumulate else 0, _stream(),
@@ -603,9 +420,10 @@ def _wgrad_once(d, x, gy, dst, st, sc, sn, sq, accumulate, flops, tag, defer=Fal
 
 def gconv_wgrad(d, x, gy, dst, st, sc, sn, sq=0, x_split=None, gy_split=None, defer=False):
     """dst (parameter layout, fp32) = weight gradient; dst[t*st + c*sc + q*sq + co*sn], n = q*Cq + co.
-    defer="call": the split reduction joins the one launch made when the enclosing reductions_at_return block ends
-    (made at once outside such a block); defer="pass": nothing but the data-parallel reducer reads dst before the end
-    of the backward pass -- the reduction joins the one launch at the end of the pass (flush_wgrad_reduce)."""
+    defer="call": the split reduction joins the one launch made when the enclosing backward_pass.reductions_at_return
+    block ends (made at once outside such a block); defer="pass": nothing but the data-parallel reducer reads dst
+    before the end of the backward pass -- the reduction joins the one launch at the end of the pass
+    (backward_pass.defer_reduce)."""
     if not x3_active(d):
         return _wgrad_once(d, x, gy, dst, st, sc, sn, sq, False, gconv_flops(d), _shape_tag(d), defer=defer)
     # 3xTF32: dW = hi(x)^T hi(g) + lo(x)^T hi(g) + hi(x)^T lo(g), the last two accumulated by the split reduction
@@ -696,7 +514,7 @@ def maxpool2_bwd(x, gp, gx, accumulate):
 # Measured at C2 (4 encoder stages, B = 16): fused 1.18 ms against 0.54 ms + 0.38 ms for the separate reduction
 # passes -- ~110 registers per thread (four coefficient vectors + two sum vectors on top of the pool's own state)
 # leave two blocks per SM and the stream runs at 0.55 of the copy peak -- so the fused form is opt-in; it stays tested.
-POOL_BNBWD_FUSE = _os.environ.get("UNETB200_POOL_BNBWD_FUSE", "0") != "0" and _os.environ.get("UNETB200_NO_BNBWD_FUSE") is None
+POOL_BNBWD_FUSE = os.environ.get("UNETB200_POOL_BNBWD_FUSE", "0") != "0" and os.environ.get("UNETB200_NO_BNBWD_FUSE") is None
 
 
 def maxpool2_bwd_bnreduce(x, gp, gx, y, coefs):
@@ -786,7 +604,7 @@ def outconv_fwd(x, w, bias, logits):
 # OutConv backward fused with the BatchNorm-backward reduction of the stage below: measured at B = 16, 512x512, 64
 # channels, 2 classes: 0.786 ms against 0.380 ms + 0.23 ms for the separate reduction pass (the 48 extra registers
 # halve the occupancy of this latency-bound stream), so the fused form is opt-in; it stays tested.
-OUTCONV_FUSE = _os.environ.get("UNETB200_OUTCONV_FUSE", "0") != "0"
+OUTCONV_FUSE = os.environ.get("UNETB200_OUTCONV_FUSE", "0") != "0"
 
 
 def outconv_bwd(x, w, glogits, gx, dw, dbias, below=None):

@@ -19,7 +19,7 @@ import ctypes as C
 
 import torch
 
-from . import ops
+from . import backward_pass, ops
 
 
 def _dense(t):
@@ -138,7 +138,7 @@ class FusedRMSprop(torch.optim.Optimizer):
             norm = self._step_amp(groups, all_grads, clip_max_norm, write_clipped_grad, grad_scale, found_inf)
             return norm if clip_max_norm is not None else loss
         torch._foreach_add_(steps, 1)                  # one launch for all step counters
-        ops.side_stream_sync()
+        backward_pass.side_stream_sync()
         norm = None
         sumsq = None
         if clip_max_norm is not None:
@@ -163,7 +163,7 @@ class FusedRMSprop(torch.optim.Optimizer):
     def _step_amp(self, groups, all_grads, clip_max_norm, write_clipped_grad, grad_scale, found_inf):
         """The device-side step: lr, 1/grad_scale and found_inf are read by the kernels, step counters move only
         when the step is taken."""
-        ops.side_stream_sync()
+        backward_pass.side_stream_sync()
         dev = all_grads[0].device
         inv_scale = None
         if grad_scale is not None:
