@@ -320,7 +320,6 @@ static int sa_blocks(int64_t work_items, int per_block) {
 }  // namespace ub
 
 using namespace ub;
-typedef __nv_bfloat16 bf16;
 
 extern "C" {
 
@@ -337,17 +336,16 @@ int unetb200_sa_forward(const void* x, int64_t ld_x, const float* w, float* stat
   const int gth = (H + kSgTH - 1) / kSgTH, gtw = (W + kSgTW - 1) / kSgTW;
   const int64_t gblocks = (int64_t)B * gth * gtw;
   UB_CHECK_ARG(gblocks < (1LL << 31), "sa_forward: too many tiles");
-#define UB_SA_T(T)                                                                                                    \
-  do {                                                                                                                \
-    if (vec) sa_stats_kernel<T><<<sa_blocks(npix, 256 / LPP), 256, 0, s>>>((const T*)x, ld_x, stats, npix, C, LPP);   \
-    else sa_stats_scalar_kernel<T><<<sa_blocks(npix, 256), 256, 0, s>>>((const T*)x, ld_x, stats, npix, C);           \
-    sa_gate_tiled_kernel<T><<<(unsigned)gblocks, 256, 0, s>>>(stats, w, gate, B, H, W, gth, gtw);                      \
-    if (vec) sa_apply_kernel<T, 8><<<sa_blocks(npix * (C / 8), 256), 256, 0, s>>>((const T*)x, ld_x, gate, (T*)out, ld_out, npix, C / 8); \
-    else sa_apply_kernel<T, 1><<<sa_blocks(npix * C, 256), 256, 0, s>>>((const T*)x, ld_x, gate, (T*)out, ld_out, npix, C); \
-  } while (0)
-  if (dtype == UNETB200_BF16) UB_SA_T(bf16);
-  else UB_SA_T(float);
-#undef UB_SA_T
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    if (vec) sa_stats_kernel<T><<<sa_blocks(npix, 256 / LPP), 256, 0, s>>>((const T*)x, ld_x, stats, npix, C, LPP);
+    else sa_stats_scalar_kernel<T><<<sa_blocks(npix, 256), 256, 0, s>>>((const T*)x, ld_x, stats, npix, C);
+    sa_gate_tiled_kernel<T><<<(unsigned)gblocks, 256, 0, s>>>(stats, w, gate, B, H, W, gth, gtw);
+    with_vec<8>(vec, [&](auto V) {
+      sa_apply_kernel<T, V><<<sa_blocks(npix * (C / V), 256), 256, 0, s>>>((const T*)x, ld_x, gate, (T*)out, ld_out,
+                                                                           npix, C / V);
+    });
+  });
   UB_LAUNCH_CHECK("sa_forward");
   return 0;
 }
@@ -379,17 +377,16 @@ int unetb200_sa_backward(const void* g, int64_t ld_g, const void* x, int64_t ld_
   const int tiles_h = (H + kSaTH - 1) / kSaTH, tiles_w = (W + kSaTW - 1) / kSaTW;
   const int64_t blocks = (int64_t)B * tiles_h * tiles_w;
   UB_CHECK_ARG(blocks < (1LL << 31), "sa_backward: too many tiles");
-#define UB_SA_B(T)                                                                                                    \
-  do {                                                                                                                \
-    sa_bwd_dgate_kernel<T><<<sa_blocks(npix, 256 / LPP), 256, 0, s>>>((const T*)g, ld_g, (const T*)x, ld_x, gate, da, npix, C, LPP); \
-    sa_bwd_dw_kernel<<<(unsigned)blocks, 128, 0, s>>>(da, stats, partial, B, H, W, tiles_h, tiles_w);                 \
-    sa_bwd_dw_reduce_kernel<<<(kSaTaps + 7) / 8, 256, 0, s>>>(partial, (int)blocks, dw);                              \
-    sa_bwd_dstats_kernel<T><<<(unsigned)gblocks, 256, 0, s>>>(da, w, dstats, B, H, W, gth, gtw);                      \
-    sa_bwd_dx_kernel<T><<<sa_blocks(npix, 256 / LPP), 256, 0, s>>>((const T*)g, ld_g, (const T*)x, ld_x, gate, dstats, (T*)dx, ld_dx, B, H, W, C, LPP); \
-  } while (0)
-  if (dtype == UNETB200_BF16) UB_SA_B(bf16);
-  else UB_SA_B(float);
-#undef UB_SA_B
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    sa_bwd_dgate_kernel<T><<<sa_blocks(npix, 256 / LPP), 256, 0, s>>>((const T*)g, ld_g, (const T*)x, ld_x, gate, da,
+                                                                      npix, C, LPP);
+    sa_bwd_dw_kernel<<<(unsigned)blocks, 128, 0, s>>>(da, stats, partial, B, H, W, tiles_h, tiles_w);
+    sa_bwd_dw_reduce_kernel<<<(kSaTaps + 7) / 8, 256, 0, s>>>(partial, (int)blocks, dw);
+    sa_bwd_dstats_kernel<T><<<(unsigned)gblocks, 256, 0, s>>>(da, w, dstats, B, H, W, gth, gtw);
+    sa_bwd_dx_kernel<T><<<sa_blocks(npix, 256 / LPP), 256, 0, s>>>((const T*)g, ld_g, (const T*)x, ld_x, gate, dstats,
+                                                                   (T*)dx, ld_dx, B, H, W, C, LPP);
+  });
   UB_LAUNCH_CHECK("sa_backward");
   return 0;
 }

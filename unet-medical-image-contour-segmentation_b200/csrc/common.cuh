@@ -6,10 +6,13 @@
 #include <stdio.h>
 
 #include <string>
+#include <type_traits>
 
 #include "../../include/unetb200.h"
 
 namespace ub {
+
+typedef __nv_bfloat16 bf16;
 
 void set_error(const char* fmt, ...);
 int cuda_fail(cudaError_t e, const char* what);
@@ -21,6 +24,66 @@ int cuda_fail(cudaError_t e, const char* what);
       return UNETB200_E_INVALID;               \
     }                                          \
   } while (0)
+
+#define UB_DTYPE_OK(dt) UB_CHECK_ARG((dt) == UNETB200_F32 || (dt) == UNETB200_BF16, "unsupported dtype %d", (int)(dt))
+
+// ---- host-side dispatch: the runtime values an ABI call receives -> template arguments ------------------------
+// Each helper calls `f` once with a tag that carries the choice in its type: a value of the chosen storage type
+// (`using T = decltype(t);`) or a std::integral_constant (usable as a template argument as it is).  The last
+// candidate of a list catches every value no earlier one matches, so a launcher validates its arguments first.
+
+template <typename T>
+struct dtype_code;
+template <>
+struct dtype_code<float> : std::integral_constant<int, UNETB200_F32> {};
+template <>
+struct dtype_code<bf16> : std::integral_constant<int, UNETB200_BF16> {};
+template <>
+struct dtype_code<long long> : std::integral_constant<int, UNETB200_I64> {};
+template <>
+struct dtype_code<uint8_t> : std::integral_constant<int, UNETB200_U8> {};
+
+// the first of T, Rest... whose dtype code is `code`, else the last
+template <typename T, typename... Rest, typename F>
+inline void with_type(int code, F&& f) {
+  if constexpr (sizeof...(Rest) == 0)
+    f(T{});
+  else if (code == dtype_code<T>::value)
+    f(T{});
+  else
+    with_type<Rest...>(code, f);
+}
+
+// element (activation) storage type: bf16 for UNETB200_BF16, float otherwise
+template <typename F>
+inline void with_elem(int dtype, F&& f) {
+  with_type<bf16, float>(dtype, f);
+}
+
+// the first of I, Rest... equal to `v`, else the last
+template <int I, int... Rest, typename F>
+inline void with_int(int v, F&& f) {
+  if constexpr (sizeof...(Rest) == 0)
+    f(std::integral_constant<int, I>{});
+  else if (v == I)
+    f(std::integral_constant<int, I>{});
+  else
+    with_int<Rest...>(v, f);
+}
+
+// vector width: V elements per access when `vec`, else 1
+template <int V, typename F>
+inline void with_vec(bool vec, F&& f) {
+  with_int<V, 1>(vec ? V : 1, f);
+}
+
+template <typename F>
+inline void with_bool(bool b, F&& f) {
+  if (b)
+    f(std::true_type{});
+  else
+    f(std::false_type{});
+}
 
 #define UB_LAUNCH_CHECK(what)                              \
   do {                                                     \

@@ -572,50 +572,36 @@ int first_fprop(const unetb200_gconv_t* d, const GconvDev& g, const void* x, con
   if (first_tiled_ok(d)) {
     const int tiles_w = (d->Wm + kFT_W - 1) / kFT_W, tiles_h = (d->Hm + kFT_H - 1) / kFT_H;
     const int ntiles = d->B * tiles_w * tiles_h;
-    if (d->dtype == UNETB200_BF16)
-      first_conv_fprop_tiled_kernel<__nv_bfloat16><<<blocks, 256, 0, s>>>(g, (const __nv_bfloat16*)x, (const __nv_bfloat16*)wp,
-                                                                          (__nv_bfloat16*)y, stats ? stats_ws : nullptr,
-                                                                          tiles_w, tiles_h, ntiles);
-    else
-      first_conv_fprop_tiled_kernel<float><<<blocks, 256, 0, s>>>(g, (const float*)x, (const float*)wp, (float*)y,
-                                                                  stats ? stats_ws : nullptr, tiles_w, tiles_h, ntiles);
+    with_elem(d->dtype, [&](auto t) {
+      using T = decltype(t);
+      first_conv_fprop_tiled_kernel<T><<<blocks, 256, 0, s>>>(g, (const T*)x, (const T*)wp, (T*)y,
+                                                              stats ? stats_ws : nullptr, tiles_w, tiles_h, ntiles);
+    });
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "first_conv_fprop_tiled");
     if (stats) return launch_stats_reduce(stats_ws, blocks, 2 * d->N, stats, s);
     return 0;
   }
   if (first_px4_ok(d)) {
-#define GO4(T, CIN) \
-  first_conv_fprop_px4_kernel<T, CIN><<<blocks, 256, 0, s>>>(g, (const T*)x, (const T*)wp, (T*)y, stats ? stats_ws : nullptr)
-    if (d->dtype == UNETB200_BF16) {
-      if (d->Cin == 2) GO4(__nv_bfloat16, 2); else if (d->Cin == 3) GO4(__nv_bfloat16, 3); else GO4(__nv_bfloat16, 4);
-    } else {
-      if (d->Cin == 2) GO4(float, 2); else if (d->Cin == 3) GO4(float, 3); else GO4(float, 4);
-    }
-#undef GO4
+    with_elem(d->dtype, [&](auto t) {
+      with_int<2, 3, 4>(d->Cin, [&](auto CIN) {
+        using T = decltype(t);
+        first_conv_fprop_px4_kernel<T, CIN><<<blocks, 256, 0, s>>>(g, (const T*)x, (const T*)wp, (T*)y,
+                                                                   stats ? stats_ws : nullptr);
+      });
+    });
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "first_conv_fprop_px4");
     if (stats) return launch_stats_reduce(stats_ws, blocks, 2 * d->N, stats, s);
     return 0;
   }
-#define GO(T, CIN) \
-  first_conv_fprop_kernel<T, CIN><<<blocks, 256, 0, s>>>(g, (const T*)x, (const T*)wp, (T*)y, stats ? stats_ws : nullptr)
-  if (d->dtype == UNETB200_BF16) {
-    switch (d->Cin) {
-      case 1: GO(__nv_bfloat16, 1); break;
-      case 2: GO(__nv_bfloat16, 2); break;
-      case 3: GO(__nv_bfloat16, 3); break;
-      default: GO(__nv_bfloat16, 4); break;
-    }
-  } else {
-    switch (d->Cin) {
-      case 1: GO(float, 1); break;
-      case 2: GO(float, 2); break;
-      case 3: GO(float, 3); break;
-      default: GO(float, 4); break;
-    }
-  }
-#undef GO
+  with_elem(d->dtype, [&](auto t) {
+    with_int<1, 2, 3, 4>(d->Cin, [&](auto CIN) {
+      using T = decltype(t);
+      first_conv_fprop_kernel<T, CIN><<<blocks, 256, 0, s>>>(g, (const T*)x, (const T*)wp, (T*)y,
+                                                             stats ? stats_ws : nullptr);
+    });
+  });
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "first_conv_fprop");
   if (stats) return launch_stats_reduce(stats_ws, blocks, 2 * d->N, stats, s);
@@ -638,21 +624,19 @@ int first_wgrad(const unetb200_gconv_t* d, const GconvDev& g, const void* x, con
   if (first_tiled_ok(d)) {
     const int tiles_w = (d->Wm + kFT_W - 1) / kFT_W, tiles_h = (d->Hm + kFT_H - 1) / kFT_H;
     const int ntiles = d->B * tiles_w * tiles_h;
-    if (d->dtype == UNETB200_BF16)
-      first_conv_wgrad_tiled_kernel<__nv_bfloat16><<<splits, 256, 0, s>>>(g, (const __nv_bfloat16*)x, (const __nv_bfloat16*)gy,
-                                                                          partials, tiles_w, tiles_h, ntiles);
-    else
-      first_conv_wgrad_tiled_kernel<float><<<splits, 256, 0, s>>>(g, (const float*)x, (const float*)gy, partials, tiles_w,
-                                                                  tiles_h, ntiles);
+    with_elem(d->dtype, [&](auto t) {
+      using T = decltype(t);
+      first_conv_wgrad_tiled_kernel<T><<<splits, 256, 0, s>>>(g, (const T*)x, (const T*)gy, partials, tiles_w, tiles_h,
+                                                              ntiles);
+    });
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return cuda_fail(e, "first_conv_wgrad_tiled");
     return 0;
   }
-  if (d->dtype == UNETB200_BF16)
-    first_conv_wgrad_kernel<__nv_bfloat16><<<splits, 256, 0, s>>>(g, (const __nv_bfloat16*)x,
-                                                                  (const __nv_bfloat16*)gy, partials);
-  else
-    first_conv_wgrad_kernel<float><<<splits, 256, 0, s>>>(g, (const float*)x, (const float*)gy, partials);
+  with_elem(d->dtype, [&](auto t) {
+    using T = decltype(t);
+    first_conv_wgrad_kernel<T><<<splits, 256, 0, s>>>(g, (const T*)x, (const T*)gy, partials);
+  });
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return cuda_fail(e, "first_conv_wgrad");
   return 0;

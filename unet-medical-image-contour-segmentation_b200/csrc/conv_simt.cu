@@ -648,22 +648,19 @@ int simt_wgrad_splits(const GconvDev& g) {
   return (int)want;
 }
 
-typedef __nv_bfloat16 bf16;
-
 int simt_fprop(const unetb200_gconv_t* d, const GconvDev& g, const void* x, const void* wp, const float* bias, void* y,
                double* stats, float* stats_ws, cudaStream_t s) {
   const int fbn = simt_fbn(g.N), fbm = simt_fbm(g.N);
   dim3 grid((unsigned)((g.M + fbm - 1) / fbm), (unsigned)((g.N + fbn - 1) / fbn));
   const bool vec = simt_vec_ok(d, x, wp, y) && (g.K % 4 == 0);
-#define UB_SIMT_F(T, V, BN) gconv_fprop_simt_kernel<T, V, BN><<<grid, 256, 0, s>>>(g, (const T*)x, (const T*)wp, bias, (T*)y, stats_ws)
-#define UB_SIMT_FN(T, V) do { if (fbn == 16) UB_SIMT_F(T, V, 16); else if (fbn == 32) UB_SIMT_F(T, V, 32); else UB_SIMT_F(T, V, 64); } while (0)
-  if (d->dtype == UNETB200_BF16) {
-    if (vec) UB_SIMT_FN(bf16, true); else UB_SIMT_FN(bf16, false);
-  } else {
-    if (vec) UB_SIMT_FN(float, true); else UB_SIMT_FN(float, false);
-  }
-#undef UB_SIMT_FN
-#undef UB_SIMT_F
+  with_elem(d->dtype, [&](auto t) {
+    with_bool(vec, [&](auto V) {
+      with_int<16, 32, 64>(fbn, [&](auto BN) {
+        using T = decltype(t);
+        gconv_fprop_simt_kernel<T, V, BN><<<grid, 256, 0, s>>>(g, (const T*)x, (const T*)wp, bias, (T*)y, stats_ws);
+      });
+    });
+  });
   UB_LAUNCH_CHECK("gconv_fprop_simt");
   if (stats) return launch_stats_reduce(stats_ws, (g.M + fbm - 1) / fbm, 2 * g.N, stats, s);
   return 0;
@@ -679,15 +676,14 @@ int simt_wgrad(const unetb200_gconv_t* d, const GconvDev& g, const void* x, cons
   const bool vec = d->Cin % 4 == 0 && g.Cq % 4 == 0 && d->ld_in % 4 == 0 && d->ld_out % 4 == 0 &&
                    (reinterpret_cast<uintptr_t>(x) % (4 * esz)) == 0 &&
                    (reinterpret_cast<uintptr_t>(gy) % (4 * esz)) == 0;
-#define UB_SIMT_W(T, V, BN) gconv_wgrad_simt_kernel<T, V, BN><<<grid, 256, 0, s>>>(g, (const T*)x, (const T*)gy, partials, mper)
-#define UB_SIMT_WN(T, V) do { if (wbn == 16) UB_SIMT_W(T, V, 16); else if (wbn == 32) UB_SIMT_W(T, V, 32); else UB_SIMT_W(T, V, 64); } while (0)
-  if (d->dtype == UNETB200_BF16) {
-    if (vec) UB_SIMT_WN(bf16, true); else UB_SIMT_WN(bf16, false);
-  } else {
-    if (vec) UB_SIMT_WN(float, true); else UB_SIMT_WN(float, false);
-  }
-#undef UB_SIMT_WN
-#undef UB_SIMT_W
+  with_elem(d->dtype, [&](auto t) {
+    with_bool(vec, [&](auto V) {
+      with_int<16, 32, 64>(wbn, [&](auto BN) {
+        using T = decltype(t);
+        gconv_wgrad_simt_kernel<T, V, BN><<<grid, 256, 0, s>>>(g, (const T*)x, (const T*)gy, partials, mper);
+      });
+    });
+  });
   UB_LAUNCH_CHECK("gconv_wgrad_simt");
   return 0;
 }
@@ -765,17 +761,17 @@ int unetb200_pack_weights(const float* src, void* dst, int dst_dtype, int64_t n0
   if (s0 == 1 && s2 != 1 && n0 >= 32 && n2 >= 32 && n1 <= 65535) {
     // source contiguous along the OUTER destination index (e.g. the dgrad operand of a channels_last weight)
     dim3 grid((unsigned)((n0 + 31) / 32), (unsigned)((n2 + 31) / 32), (unsigned)n1);
-    if (dst_dtype == UNETB200_BF16)
-      pack_weights_t_kernel<bf16><<<grid, 256, 0, s>>>(src, (bf16*)dst, (int)n0, (int)n1, (int)n2, s1, s2, off);
-    else
-      pack_weights_t_kernel<float><<<grid, 256, 0, s>>>(src, (float*)dst, (int)n0, (int)n1, (int)n2, s1, s2, off);
+    with_elem(dst_dtype, [&](auto t) {
+      using D = decltype(t);
+      pack_weights_t_kernel<D><<<grid, 256, 0, s>>>(src, (D*)dst, (int)n0, (int)n1, (int)n2, s1, s2, off);
+    });
     UB_LAUNCH_CHECK("pack_weights_t");
     return 0;
   }
-  if (dst_dtype == UNETB200_BF16)
-    pack_weights_kernel<bf16><<<(unsigned)blocks, 256, 0, s>>>(src, (bf16*)dst, n0, n1, n2, s0, s1, s2, off);
-  else
-    pack_weights_kernel<float><<<(unsigned)blocks, 256, 0, s>>>(src, (float*)dst, n0, n1, n2, s0, s1, s2, off);
+  with_elem(dst_dtype, [&](auto t) {
+    using D = decltype(t);
+    pack_weights_kernel<D><<<(unsigned)blocks, 256, 0, s>>>(src, (D*)dst, n0, n1, n2, s0, s1, s2, off);
+  });
   UB_LAUNCH_CHECK("pack_weights");
   return 0;
 }
@@ -803,8 +799,7 @@ int unetb200_pack_weights_multi(const unetb200_pack_job_t* jobs, int njobs, int 
       UB_CHECK_ARG(blocks < (1LL << 31), "pack_weights_multi: too many tiles");
     }
     T.njobs = count;
-    if (dst_dtype == UNETB200_BF16) pack_multi_kernel<bf16><<<(unsigned)blocks, 256, 0, s>>>(T);
-    else pack_multi_kernel<float><<<(unsigned)blocks, 256, 0, s>>>(T);
+    with_elem(dst_dtype, [&](auto t) { pack_multi_kernel<decltype(t)><<<(unsigned)blocks, 256, 0, s>>>(T); });
   }
   UB_LAUNCH_CHECK("pack_weights_multi");
   return 0;

@@ -799,9 +799,6 @@ __global__ void double_to_float_kernel(const double* __restrict__ a, float* __re
 }  // namespace ub
 
 using namespace ub;
-typedef __nv_bfloat16 bf16;
-
-#define UB_DTYPE_OK(dt) UB_CHECK_ARG((dt) == UNETB200_F32 || (dt) == UNETB200_BF16, "unsupported dtype %d", (int)(dt))
 
 // ---- 3xTF32 operand split (fp32 exactness mode on the tensor cores) ------------------------------------------
 // x = hi + lo exactly, hi = x rounded to TF32's 10-bit mantissa (round half away from zero on the magnitude bits),
@@ -887,25 +884,21 @@ int unetb200_bn_relu_apply(const void* y, int64_t ld_y, const float* scale, cons
   UB_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0 && ld_y >= C && ld_z >= C, "bn_relu_apply: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t npix = (int64_t)B * H * W;
-#define GO(T, V)                                                                                              \
-  do {                                                                                                        \
-    int CV = C / V;                                                                                           \
-    if (pooled) {                                                                                             \
-      CsGeom g_ = cs_geom(CV, (int64_t)B * ((H + 1) / 2) * ((W + 1) / 2), 2);                                 \
-      bn_relu_apply_pool_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(                                     \
-          (const T*)y, ld_y, scale, shift, (T*)z, ld_z, (T*)pooled, ld_p, B, H, W, CV, g_.CVB);               \
-    } else {                                                                                                  \
-      CsGeom g_ = cs_geom(CV, npix, 8);                                                                       \
-      bn_relu_apply_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>((const T*)y, ld_y, scale, shift, (T*)z,   \
-                                                                   ld_z, npix, CV, g_.CVB);                   \
-    }                                                                                                         \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_y, ld_z, pooled ? ld_p : 0}, {y, z, pooled})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_y, ld_z, pooled ? ld_p : 0}, {y, z, pooled})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_y, ld_z, pooled ? ld_p : 0}, {y, z, pooled}), [&](auto V) {
+      int CV = C / V;
+      if (pooled) {
+        CsGeom g_ = cs_geom(CV, (int64_t)B * ((H + 1) / 2) * ((W + 1) / 2), 2);
+        bn_relu_apply_pool_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(
+            (const T*)y, ld_y, scale, shift, (T*)z, ld_z, (T*)pooled, ld_p, B, H, W, CV, g_.CVB);
+      } else {
+        CsGeom g_ = cs_geom(CV, npix, 8);
+        bn_relu_apply_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>((const T*)y, ld_y, scale, shift, (T*)z,
+                                                                     ld_z, npix, CV, g_.CVB);
+      }
+    });
+  });
   UB_LAUNCH_CHECK("bn_relu_apply");
   return 0;
 }
@@ -915,19 +908,14 @@ int unetb200_maxpool2_fwd(const void* x, int64_t ld_x, void* p, int64_t ld_p, in
   UB_DTYPE_OK(dtype);
   UB_CHECK_ARG(B > 0 && H >= 2 && W >= 2 && C > 0, "maxpool2_fwd: bad shape %d %d %d %d", B, H, W, C);
   cudaStream_t s = (cudaStream_t)stream;
-#define GO(T, V)                                                                                         \
-  do {                                                                                                   \
-    int CV = C / V;                                                                                      \
-    int64_t work = (int64_t)B * (H / 2) * (W / 2) * CV;                                                  \
-    maxpool2_fwd_kernel<T, V><<<grid_for(work, 256, 16), 256, 0, s>>>((const T*)x, ld_x, (T*)p, ld_p, B, \
-                                                                      H, W, CV);                         \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_x, ld_p}, {x, p})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_x, ld_p}, {x, p})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_x, ld_p}, {x, p}), [&](auto V) {
+      int CV = C / V;
+      int64_t work = (int64_t)B * (H / 2) * (W / 2) * CV;
+      maxpool2_fwd_kernel<T, V><<<grid_for(work, 256, 16), 256, 0, s>>>((const T*)x, ld_x, (T*)p, ld_p, B, H, W, CV);
+    });
+  });
   UB_LAUNCH_CHECK("maxpool2_fwd");
   return 0;
 }
@@ -937,23 +925,17 @@ int unetb200_maxpool2_bwd(const void* x, int64_t ld_x, const void* gp, int64_t l
   UB_DTYPE_OK(dtype);
   UB_CHECK_ARG(B > 0 && H >= 2 && W >= 2 && C > 0, "maxpool2_bwd: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
-#define GO(T, V)                                                                                              \
-  do {                                                                                                        \
-    int CV = C / V;                                                                                           \
-    int64_t work = (int64_t)B * ((H + 1) / 2) * ((W + 1) / 2) * CV;                                           \
-    if (accumulate)                                                                                           \
-      maxpool2_bwd_kernel<T, V, true><<<grid_for(work, 256, 16), 256, 0, s>>>(                                \
-          (const T*)x, ld_x, (const T*)gp, ld_gp, (T*)gx, ld_gx, B, H, W, CV);                                \
-    else                                                                                                      \
-      maxpool2_bwd_kernel<T, V, false><<<grid_for(work, 256, 16), 256, 0, s>>>(                               \
-          (const T*)x, ld_x, (const T*)gp, ld_gp, (T*)gx, ld_gx, B, H, W, CV);                                \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_x, ld_gp, ld_gx}, {x, gp, gx})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_x, ld_gp, ld_gx}, {x, gp, gx})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_x, ld_gp, ld_gx}, {x, gp, gx}), [&](auto V) {
+      int CV = C / V;
+      int64_t work = (int64_t)B * ((H + 1) / 2) * ((W + 1) / 2) * CV;
+      with_bool(accumulate, [&](auto ACC) {
+        maxpool2_bwd_kernel<T, V, ACC><<<grid_for(work, 256, 16), 256, 0, s>>>(
+            (const T*)x, ld_x, (const T*)gp, ld_gp, (T*)gx, ld_gx, B, H, W, CV);
+      });
+    });
+  });
   UB_LAUNCH_CHECK("maxpool2_bwd");
   return 0;
 }
@@ -966,20 +948,16 @@ int unetb200_maxpool2_bwd_bnreduce(const void* x, int64_t ld_x, const void* gp, 
                "maxpool2_bwd_bnreduce: bad args");
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t nwin = (int64_t)B * ((H + 1) / 2) * ((W + 1) / 2);
-#define GO(T, V)                                                                                              \
-  do {                                                                                                        \
-    const int CV = (C + V - 1) / V;                                                                           \
-    CsGeom g_ = cs_geom(CV, nwin, 2, V == 8 ? 64 : 256);                                                      \
-    maxpool2_bwd_bnreduce_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(                                    \
-        (const T*)x, ld_x, (const T*)gp, ld_gp, (T*)gx, ld_gx, (const T*)y, ld_y, scale, shift, mean, invstd, \
-        sums, B, H, W, C, CV, g_.CVB);                                                                        \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_x, ld_gp, ld_gx, ld_y}, {x, gp, gx, y})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_x, ld_gp, ld_gx, ld_y}, {x, gp, gx, y})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_x, ld_gp, ld_gx, ld_y}, {x, gp, gx, y}), [&](auto V) {
+      const int CV = (C + V - 1) / V;
+      CsGeom g_ = cs_geom(CV, nwin, 2, V == 8 ? 64 : 256);
+      maxpool2_bwd_bnreduce_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(
+          (const T*)x, ld_x, (const T*)gp, ld_gp, (T*)gx, ld_gx, (const T*)y, ld_y, scale, shift, mean, invstd,
+          sums, B, H, W, C, CV, g_.CVB);
+    });
+  });
   UB_LAUNCH_CHECK("maxpool2_bwd_bnreduce");
   return 0;
 }
@@ -991,19 +969,15 @@ int unetb200_bn_relu_bwd_reduce(const void* gz, int64_t ld_gz, const void* y, in
   UB_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0, "bn_relu_bwd_reduce: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t npix = (int64_t)B * H * W;
-#define GO(T, V)                                                                                              \
-  do {                                                                                                        \
-    int CV = C / V;                                                                                           \
-    CsGeom g_ = cs_geom(CV, npix, 8, V == 8 ? 64 : 256);   /* CVB * V <= the kernel's shared reduction row */   \
-    bn_relu_bwd_reduce_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(                                       \
-        (const T*)gz, ld_gz, (const T*)y, ld_y, scale, shift, mean, invstd, sums, npix, C, CV, g_.CVB);       \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_gz, ld_y}, {gz, y})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_gz, ld_y}, {gz, y})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_gz, ld_y}, {gz, y}), [&](auto V) {
+      int CV = C / V;
+      CsGeom g_ = cs_geom(CV, npix, 8, V == 8 ? 64 : 256);   // CVB * V <= the kernel's shared reduction row
+      bn_relu_bwd_reduce_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(
+          (const T*)gz, ld_gz, (const T*)y, ld_y, scale, shift, mean, invstd, sums, npix, C, CV, g_.CVB);
+    });
+  });
   UB_LAUNCH_CHECK("bn_relu_bwd_reduce");
   return 0;
 }
@@ -1024,20 +998,16 @@ int unetb200_bn_relu_bwd_apply(const void* gz, int64_t ld_gz, const void* y, int
   UB_CHECK_ARG(B > 0 && H > 0 && W > 0 && C > 0, "bn_relu_bwd_apply: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   const int64_t npix = (int64_t)B * H * W;
-#define GO(T, V)                                                                                             \
-  do {                                                                                                       \
-    int CV = C / V;                                                                                          \
-    CsGeom g_ = cs_geom(CV, npix, 8);                                                                        \
-    bn_relu_bwd_apply_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(                                       \
-        (const T*)gz, ld_gz, (const T*)y, ld_y, scale, shift, mean, invstd, coef, (T*)gy, ld_gy, npix, C, CV,  \
-        g_.CVB);                                                                                             \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_gz, ld_y, ld_gy}, {gz, y, gy})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_gz, ld_y, ld_gy}, {gz, y, gy})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_gz, ld_y, ld_gy}, {gz, y, gy}), [&](auto V) {
+      int CV = C / V;
+      CsGeom g_ = cs_geom(CV, npix, 8);
+      bn_relu_bwd_apply_kernel<T, V><<<dim3(g_.gx, g_.gy), 256, 0, s>>>(
+          (const T*)gz, ld_gz, (const T*)y, ld_y, scale, shift, mean, invstd, coef, (T*)gy, ld_gy, npix, C, CV,
+          g_.CVB);
+    });
+  });
   UB_LAUNCH_CHECK("bn_relu_bwd_apply");
   return 0;
 }
@@ -1052,19 +1022,15 @@ int unetb200_upsample2x_fwd(const void* x, int64_t ld_x, void* y, int64_t ld_y, 
                "upsample2x_fwd: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   float sy = ac_scale(h, 2 * h), sx = ac_scale(w, 2 * w);
-#define GO(T, V)                                                                                           \
-  do {                                                                                                     \
-    int CV = C / V;                                                                                        \
-    int64_t work = (int64_t)B * 4 * h * w * CV;                                                            \
-    upsample2x_fwd_kernel<T, V><<<grid_for(work, 256, 16), 256, 0, s>>>(                                   \
-        (const T*)x, ld_x, (T*)y, ld_y, B, h, w, CV, Hout, Wout, off_y, off_x, sy, sx);                    \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_x, ld_y}, {x, y})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_x, ld_y}, {x, y})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_x, ld_y}, {x, y}), [&](auto V) {
+      int CV = C / V;
+      int64_t work = (int64_t)B * 4 * h * w * CV;
+      upsample2x_fwd_kernel<T, V><<<grid_for(work, 256, 16), 256, 0, s>>>(
+          (const T*)x, ld_x, (T*)y, ld_y, B, h, w, CV, Hout, Wout, off_y, off_x, sy, sx);
+    });
+  });
   UB_LAUNCH_CHECK("upsample2x_fwd");
   return 0;
 }
@@ -1077,19 +1043,15 @@ int unetb200_upsample2x_bwd(const void* gy, int64_t ld_gy, void* gx, int64_t ld_
                "upsample2x_bwd: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   float sy = ac_scale(h, 2 * h), sx = ac_scale(w, 2 * w);
-#define GO(T, V)                                                                                           \
-  do {                                                                                                     \
-    int CV = C / V;                                                                                        \
-    int64_t work = (int64_t)B * h * w * CV;                                                                \
-    upsample2x_bwd_kernel<T, V><<<grid_for(work, 128, 16), 128, 0, s>>>(                                   \
-        (const T*)gy, ld_gy, (T*)gx, ld_gx, B, h, w, CV, Hout, Wout, off_y, off_x, sy, sx);                \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (vec_ok<bf16>(C, {ld_gy, ld_gx}, {gy, gx})) GO(bf16, 8); else GO(bf16, 1);
-  } else {
-    if (vec_ok<float>(C, {ld_gy, ld_gx}, {gy, gx})) GO(float, 8); else GO(float, 1);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_gy, ld_gx}, {gy, gx}), [&](auto V) {
+      int CV = C / V;
+      int64_t work = (int64_t)B * h * w * CV;
+      upsample2x_bwd_kernel<T, V><<<grid_for(work, 128, 16), 128, 0, s>>>(
+          (const T*)gy, ld_gy, (T*)gx, ld_gx, B, h, w, CV, Hout, Wout, off_y, off_x, sy, sx);
+    });
+  });
   UB_LAUNCH_CHECK("upsample2x_bwd");
   return 0;
 }
@@ -1105,22 +1067,24 @@ int unetb200_gather_nhwc(const void* src, int src_dtype, int64_t sn, int64_t sc,
                      (reinterpret_cast<uintptr_t>(src) & 31) == 0 && (reinterpret_cast<uintptr_t>(dst) & 31) == 0;
   if (dense) {
     const int gf = grid_for(work / 8 + 1, 256, 16);
-#define GOF(S, D) convert_flat_kernel<S, D><<<gf, 256, 0, s>>>((const S*)src, (D*)dst, work)
-    if (src_dtype == UNETB200_F32 && dst_dtype == UNETB200_F32) GOF(float, float);
-    else if (src_dtype == UNETB200_F32) GOF(float, bf16);
-    else if (dst_dtype == UNETB200_F32) GOF(bf16, float);
-    else GOF(bf16, bf16);
-#undef GOF
+    with_elem(src_dtype, [&](auto src_t) {
+      with_elem(dst_dtype, [&](auto dst_t) {
+        using S = decltype(src_t);
+        using D = decltype(dst_t);
+        convert_flat_kernel<S, D><<<gf, 256, 0, s>>>((const S*)src, (D*)dst, work);
+      });
+    });
     UB_LAUNCH_CHECK("gather_nhwc (flat)");
     return 0;
   }
   int g = grid_for(work, 256, 16);
-#define GO(S, D) gather_nhwc_kernel<S, D><<<g, 256, 0, s>>>((const S*)src, sn, sc, sh, sw, (D*)dst, ld_dst, B, C, H, W)
-  if (src_dtype == UNETB200_F32 && dst_dtype == UNETB200_F32) GO(float, float);
-  else if (src_dtype == UNETB200_F32) GO(float, bf16);
-  else if (dst_dtype == UNETB200_F32) GO(bf16, float);
-  else GO(bf16, bf16);
-#undef GO
+  with_elem(src_dtype, [&](auto src_t) {
+    with_elem(dst_dtype, [&](auto dst_t) {
+      using S = decltype(src_t);
+      using D = decltype(dst_t);
+      gather_nhwc_kernel<S, D><<<g, 256, 0, s>>>((const S*)src, sn, sc, sh, sw, (D*)dst, ld_dst, B, C, H, W);
+    });
+  });
   UB_LAUNCH_CHECK("gather_nhwc");
   return 0;
 }
@@ -1131,21 +1095,16 @@ int unetb200_copy_channels(const void* src, int src_dtype, int64_t ld_src, void*
   UB_DTYPE_OK(dst_dtype);
   UB_CHECK_ARG(npix > 0 && C > 0 && ld_src >= C && ld_dst >= C, "copy_channels: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
-#define GO(S, D)                                                                                               \
-  do {                                                                                                         \
-    if (vec_ok<S>(C, {ld_src}, {src}) && vec_ok<D>(C, {ld_dst}, {dst}))                                        \
-      copy_channels_kernel<S, D, 8><<<grid_for(npix * (C / 8), 256, 16), 256, 0, s>>>((const S*)src, ld_src,   \
-                                                                                      (D*)dst, ld_dst, npix,   \
-                                                                                      C / 8);                  \
-    else                                                                                                       \
-      copy_channels_kernel<S, D, 1><<<grid_for(npix * C, 256, 16), 256, 0, s>>>((const S*)src, ld_src,         \
-                                                                                (D*)dst, ld_dst, npix, C);     \
-  } while (0)
-  if (src_dtype == UNETB200_F32 && dst_dtype == UNETB200_F32) GO(float, float);
-  else if (src_dtype == UNETB200_F32) GO(float, bf16);
-  else if (dst_dtype == UNETB200_F32) GO(bf16, float);
-  else GO(bf16, bf16);
-#undef GO
+  with_elem(src_dtype, [&](auto src_t) {
+    with_elem(dst_dtype, [&](auto dst_t) {
+      using S = decltype(src_t);
+      using D = decltype(dst_t);
+      with_vec<8>(vec_ok<S>(C, {ld_src}, {src}) && vec_ok<D>(C, {ld_dst}, {dst}), [&](auto V) {
+        copy_channels_kernel<S, D, V><<<grid_for(npix * (C / V), 256, 16), 256, 0, s>>>((const S*)src, ld_src,
+                                                                                        (D*)dst, ld_dst, npix, C / V);
+      });
+    });
+  });
   UB_LAUNCH_CHECK("copy_channels");
   return 0;
 }
@@ -1154,15 +1113,12 @@ int unetb200_zero_channels(void* dst, int dtype, int64_t ld_dst, int64_t npix, i
   UB_DTYPE_OK(dtype);
   UB_CHECK_ARG(npix > 0 && C > 0 && ld_dst >= C, "zero_channels: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
-#define GO(T)                                                                                              \
-  do {                                                                                                     \
-    if (vec_ok<T>(C, {ld_dst}, {dst}))                                                                     \
-      zero_channels_kernel<T, 8><<<grid_for(npix * (C / 8), 256, 16), 256, 0, s>>>((T*)dst, ld_dst, npix, C / 8); \
-    else                                                                                                   \
-      zero_channels_kernel<T, 1><<<grid_for(npix * C, 256, 16), 256, 0, s>>>((T*)dst, ld_dst, npix, C);    \
-  } while (0)
-  if (dtype == UNETB200_BF16) GO(bf16); else GO(float);
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_dst}, {dst}), [&](auto V) {
+      zero_channels_kernel<T, V><<<grid_for(npix * (C / V), 256, 16), 256, 0, s>>>((T*)dst, ld_dst, npix, C / V);
+    });
+  });
   UB_LAUNCH_CHECK("zero_channels");
   return 0;
 }
@@ -1172,17 +1128,13 @@ int unetb200_add_channels(void* a, int64_t ld_a, const void* b, int64_t ld_b, in
   UB_DTYPE_OK(dtype);
   UB_CHECK_ARG(npix > 0 && C > 0 && ld_a >= C && ld_b >= C, "add_channels: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
-#define GO(T)                                                                                               \
-  do {                                                                                                      \
-    if (vec_ok<T>(C, {ld_a, ld_b}, {a, b}))                                                                 \
-      add_channels_kernel<T, 8><<<grid_for(npix * (C / 8), 256, 16), 256, 0, s>>>((T*)a, ld_a, (const T*)b, \
-                                                                                  ld_b, npix, C / 8);       \
-    else                                                                                                    \
-      add_channels_kernel<T, 1><<<grid_for(npix * C, 256, 16), 256, 0, s>>>((T*)a, ld_a, (const T*)b, ld_b, \
-                                                                            npix, C);                       \
-  } while (0)
-  if (dtype == UNETB200_BF16) GO(bf16); else GO(float);
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    with_vec<8>(vec_ok<T>(C, {ld_a, ld_b}, {a, b}), [&](auto V) {
+      add_channels_kernel<T, V><<<grid_for(npix * (C / V), 256, 16), 256, 0, s>>>((T*)a, ld_a, (const T*)b, ld_b,
+                                                                                  npix, C / V);
+    });
+  });
   UB_LAUNCH_CHECK("add_channels");
   return 0;
 }
@@ -1201,26 +1153,19 @@ int unetb200_channel_sum(const void* g, int dtype, int64_t ld, int64_t npix, int
     const int64_t cap_v = (int64_t)sm_count() * 4;
     if (gx_v > cap_v) gx_v = cap_v;
     if (gx_v < 1) gx_v = 1;
-    if (dtype == UNETB200_BF16)
-      channel_sum_vec_kernel<bf16><<<(unsigned)gx_v, 256, 0, s>>>((const bf16*)g, ld, npix, C, acc);
-    else
-      channel_sum_vec_kernel<float><<<(unsigned)gx_v, 256, 0, s>>>((const float*)g, ld, npix, C, acc);
+    with_elem(dtype, [&](auto t) {
+      using T = decltype(t);
+      channel_sum_vec_kernel<T><<<(unsigned)gx_v, 256, 0, s>>>((const T*)g, ld, npix, C, acc);
+    });
     double_to_float_kernel<<<(C + 127) / 128, 128, 0, s>>>(acc, out, C);
     UB_LAUNCH_CHECK("channel_sum_vec");
     return 0;
   }
-  int CB = C < 256 ? C : 256;
-  int lanes = 256 / CB;
-  int gy_ = (C + CB - 1) / CB;
-  int64_t gx_ = (npix + (int64_t)lanes * 16 - 1) / ((int64_t)lanes * 16);
-  int64_t cap = (int64_t)sm_count() * 8 / gy_;
-  if (cap < 1) cap = 1;
-  if (gx_ > cap) gx_ = cap;
-  if (gx_ < 1) gx_ = 1;
-  if (dtype == UNETB200_BF16)
-    channel_sum_kernel<bf16><<<dim3((unsigned)gx_, gy_), 256, 0, s>>>((const bf16*)g, ld, npix, C, CB, acc);
-  else
-    channel_sum_kernel<float><<<dim3((unsigned)gx_, gy_), 256, 0, s>>>((const float*)g, ld, npix, C, CB, acc);
+  const CsGeom g_ = cs_geom(C, npix, 16);
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    channel_sum_kernel<T><<<dim3(g_.gx, g_.gy), 256, 0, s>>>((const T*)g, ld, npix, C, g_.CVB, acc);
+  });
   double_to_float_kernel<<<(C + 127) / 128, 128, 0, s>>>(acc, out, C);
   UB_LAUNCH_CHECK("channel_sum");
   return 0;
@@ -1236,10 +1181,9 @@ int unetb200_f64_to_f32(const double* src, float* dst, int n, void* stream) {
 int unetb200_split_tf32(const float* x, int64_t ld_x, float* out, int64_t npix, int C, int pattern, void* stream) {
   UB_CHECK_ARG(x && out && npix > 0 && C > 0 && ld_x >= C && (pattern == 0 || pattern == 1), "split_tf32: bad args");
   cudaStream_t s = (cudaStream_t)stream;
-  if (C % 4 == 0 && ld_x % 4 == 0 && aligned16(x) && aligned16(out))
-    split_tf32_kernel<4><<<grid_for(npix * (C / 4), 256, 16), 256, 0, s>>>(x, ld_x, out, npix, C / 4, pattern);
-  else
-    split_tf32_kernel<1><<<grid_for(npix * C, 256, 16), 256, 0, s>>>(x, ld_x, out, npix, C, pattern);
+  with_vec<4>(C % 4 == 0 && ld_x % 4 == 0 && aligned16(x) && aligned16(out), [&](auto V) {
+    split_tf32_kernel<V><<<grid_for(npix * (C / V), 256, 16), 256, 0, s>>>(x, ld_x, out, npix, C / V, pattern);
+  });
   UB_LAUNCH_CHECK("split_tf32");
   return 0;
 }

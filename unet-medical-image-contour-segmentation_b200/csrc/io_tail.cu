@@ -383,7 +383,6 @@ static void launch_rot_convert(const uint8_t* src, int H, int W, int C, const in
 }  // namespace ub
 
 using namespace ub;
-typedef __nv_bfloat16 bf16;
 
 static inline int tail_grid(int64_t work_per_image, int B, int threads) {
   int64_t b = (work_per_image + threads - 1) / threads;
@@ -404,28 +403,19 @@ static bool launch_eval_packed(const void* logits, int dtype, int64_t sb, int64_
   if (!aligned16(logits) || (target && !aligned16(target)) || (pred_out && !aligned16(pred_out))) return false;
   const int64_t groups = HW / 4;
   dim3 grid(tail_grid(groups, B, 256), B);
-#define GO4(T, TT, O, CC)                                                                                         \
-  eval_counts_packed_kernel<T, TT, O, CC><<<grid, 256, 0, s>>>((const T*)logits, (const TT*)target, groups, cls, \
-                                                               (O*)pred_out, cnt)
-#define GO3(T, TT, O)             \
-  do {                            \
-    if (C == 2) GO4(T, TT, O, 2); \
-    else if (C == 3) GO4(T, TT, O, 3); \
-    else GO4(T, TT, O, 4);        \
-  } while (0)
-#define GO2(T, TT)               \
-  do {                           \
-    if (u8) GO3(T, TT, uint8_t); \
-    else GO3(T, TT, long long);  \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (target && tgt_dtype == UNETB200_I64) GO2(bf16, long long); else GO2(bf16, float);
-  } else {
-    if (target && tgt_dtype == UNETB200_I64) GO2(float, long long); else GO2(float, float);
-  }
-#undef GO2
-#undef GO3
-#undef GO4
+  with_elem(dtype, [&](auto t) {
+    with_type<long long, float>(target ? tgt_dtype : UNETB200_F32, [&](auto tt) {
+      with_type<uint8_t, long long>(u8 ? UNETB200_U8 : UNETB200_I64, [&](auto o) {
+        with_int<2, 3, 4>(C, [&](auto CC) {
+          using T = decltype(t);
+          using TT = decltype(tt);
+          using O = decltype(o);
+          eval_counts_packed_kernel<T, TT, O, CC><<<grid, 256, 0, s>>>((const T*)logits, (const TT*)target, groups,
+                                                                       cls, (O*)pred_out, cnt);
+        });
+      });
+    });
+  });
   return true;
 }
 
@@ -457,21 +447,17 @@ int unetb200_eval_counts(const void* logits, int dtype, int64_t sb, int64_t sc, 
     UB_LAUNCH_CHECK("eval_counts");
     return 0;
   }
-#define GO3(T, TT, O)                                                                                      \
-  eval_counts_kernel<T, TT, O><<<grid, 256, 0, s>>>((const T*)logits, sb, sc, sh, sw, (const TT*)target, C, H, W, \
-                                                    cls, mode, (O*)pred_out, cnt)
-#define GO2(T, TT)            \
-  do {                        \
-    if (u8) GO3(T, TT, uint8_t); \
-    else GO3(T, TT, long long);  \
-  } while (0)
-  if (dtype == UNETB200_BF16) {
-    if (tgt_dtype == UNETB200_I64) GO2(bf16, long long); else GO2(bf16, float);
-  } else {
-    if (tgt_dtype == UNETB200_I64) GO2(float, long long); else GO2(float, float);
-  }
-#undef GO2
-#undef GO3
+  with_elem(dtype, [&](auto t) {
+    with_type<long long, float>(tgt_dtype, [&](auto tt) {
+      with_type<uint8_t, long long>(u8 ? UNETB200_U8 : UNETB200_I64, [&](auto o) {
+        using T = decltype(t);
+        using TT = decltype(tt);
+        using O = decltype(o);
+        eval_counts_kernel<T, TT, O><<<grid, 256, 0, s>>>((const T*)logits, sb, sc, sh, sw, (const TT*)target, C, H,
+                                                          W, cls, mode, (O*)pred_out, cnt);
+      });
+    });
+  });
   if (dice_out) eval_dice_finalize_kernel<<<1, 32, 0, s>>>(cnt, B, epsilon, dice_out);
   UB_LAUNCH_CHECK("eval_counts");
   return 0;
@@ -492,14 +478,14 @@ int unetb200_resize_argmax(const void* logits, int dtype, int64_t sb, int64_t sc
   }
   dim3 grid(tail_grid((int64_t)H * W, B, 256), B);
   const float sch = (float)h / (float)H, scw = (float)w / (float)W;
-#define GO(T, O) \
-  resize_argmax_kernel<T, O><<<grid, 256, 0, s>>>((const T*)logits, sb, sc, sh, sw, C, h, w, H, W, sch, scw, (O*)out)
-  if (dtype == UNETB200_BF16) {
-    if (out_dtype == UNETB200_U8) GO(bf16, uint8_t); else GO(bf16, long long);
-  } else {
-    if (out_dtype == UNETB200_U8) GO(float, uint8_t); else GO(float, long long);
-  }
-#undef GO
+  with_elem(dtype, [&](auto t) {
+    with_type<uint8_t, long long>(out_dtype, [&](auto o) {
+      using T = decltype(t);
+      using O = decltype(o);
+      resize_argmax_kernel<T, O><<<grid, 256, 0, s>>>((const T*)logits, sb, sc, sh, sw, C, h, w, H, W, sch, scw,
+                                                      (O*)out);
+    });
+  });
   UB_LAUNCH_CHECK("resize_argmax");
   return 0;
 }

@@ -430,7 +430,6 @@ __global__ void boundary_finalize_kernel(const unsigned long long* __restrict__ 
 }  // namespace ub
 
 using namespace ub;
-typedef __nv_bfloat16 bf16;
 
 static inline int loss_grid(int64_t work, int threads) {
   int64_t b = (work + threads - 1) / threads;
@@ -438,6 +437,14 @@ static inline int loss_grid(int64_t work, int threads) {
   if (b > cap) b = cap;
   if (b < 1) b = 1;
   return (int)b;
+}
+
+// calls f(logits element, target element) for the storage types given by `dtype`, `tgt_dtype`
+template <typename F>
+static void with_bce_dice_types(int dtype, int tgt_dtype, F&& f) {
+  with_elem(dtype, [&](auto t) {
+    with_type<float, long long, uint8_t>(tgt_dtype, [&](auto tt) { f(t, tt); });
+  });
 }
 
 extern "C" {
@@ -451,10 +458,10 @@ int unetb200_ce_dice_fwd(const void* logits, int dtype, const int64_t* target, i
   cudaError_t e = cudaMemsetAsync(acc, 0, 4 * sizeof(double), s);
   if (e != cudaSuccess) return cuda_fail(e, "ce_dice_fwd memset");
   int g = loss_grid(npix, 256);
-  if (dtype == UNETB200_BF16)
-    ce_dice_fwd_kernel<bf16><<<g, 256, 0, s>>>((const bf16*)logits, target, npix, C, acc);
-  else
-    ce_dice_fwd_kernel<float><<<g, 256, 0, s>>>((const float*)logits, target, npix, C, acc);
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    ce_dice_fwd_kernel<T><<<g, 256, 0, s>>>((const T*)logits, target, npix, C, acc);
+  });
   ce_dice_finalize_kernel<<<1, 32, 0, s>>>(acc, npix, epsilon, out, coefs);
   UB_LAUNCH_CHECK("ce_dice_fwd");
   return 0;
@@ -466,11 +473,10 @@ int unetb200_ce_dice_bwd(const void* logits, int dtype, const int64_t* target, i
   UB_CHECK_ARG(npix > 0 && C >= 1 && C <= kMaxClasses, "ce_dice_bwd: bad shape");
   cudaStream_t s = (cudaStream_t)stream;
   int g = loss_grid(npix, 256);
-  if (dtype == UNETB200_BF16)
-    ce_dice_bwd_kernel<bf16><<<g, 256, 0, s>>>((const bf16*)logits, target, npix, C, coefs, gscale, (bf16*)glogits);
-  else
-    ce_dice_bwd_kernel<float><<<g, 256, 0, s>>>((const float*)logits, target, npix, C, coefs, gscale,
-                                                (float*)glogits);
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    ce_dice_bwd_kernel<T><<<g, 256, 0, s>>>((const T*)logits, target, npix, C, coefs, gscale, (T*)glogits);
+  });
   UB_LAUNCH_CHECK("ce_dice_bwd");
   return 0;
 }
@@ -482,20 +488,6 @@ static inline bool bce_dice_vec(const void* logits, const void* target, int tgt_
   return aligned16(logits) && (reinterpret_cast<uintptr_t>(target) & (talign - 1)) == 0 &&
          (glogits == nullptr || aligned16(glogits));
 }
-
-// GO(T, TT) for the (logits, target) storage types given by `dtype`, `tgt_dtype`
-#define BCE_DICE_DISPATCH()                                                      \
-  do {                                                                           \
-    if (dtype == UNETB200_BF16) {                                                \
-      if (tgt_dtype == UNETB200_F32) GO(bf16, float);                            \
-      else if (tgt_dtype == UNETB200_I64) GO(bf16, long long);                   \
-      else GO(bf16, uint8_t);                                                    \
-    } else {                                                                     \
-      if (tgt_dtype == UNETB200_F32) GO(float, float);                           \
-      else if (tgt_dtype == UNETB200_I64) GO(float, long long);                  \
-      else GO(float, uint8_t);                                                   \
-    }                                                                            \
-  } while (0)
 
 int64_t unetb200_bce_dice_work_bytes(int64_t npix) {
   if (npix <= 0) return 0;
@@ -512,10 +504,11 @@ int unetb200_bce_dice_fwd(const void* logits, int dtype, const void* target, int
   const int g = bce_dice_grid(npix);
   const bool vec = bce_dice_vec(logits, target, tgt_dtype, nullptr);
   double* partials = (double*)work;
-#define GO(T, TT) \
-  bce_dice_fwd_kernel<T, TT><<<g, 256, 0, s>>>((const T*)logits, (const TT*)target, npix, vec, partials)
-  BCE_DICE_DISPATCH();
-#undef GO
+  with_bce_dice_types(dtype, tgt_dtype, [&](auto t, auto tt) {
+    using T = decltype(t);
+    using TT = decltype(tt);
+    bce_dice_fwd_kernel<T, TT><<<g, 256, 0, s>>>((const T*)logits, (const TT*)target, npix, vec, partials);
+  });
   bce_dice_finalize_kernel<<<1, 256, 0, s>>>(partials, g, npix, epsilon, out, coefs);
   UB_LAUNCH_CHECK("bce_dice_fwd");
   return 0;
@@ -530,15 +523,15 @@ int unetb200_bce_dice_bwd(const void* logits, int dtype, const void* target, int
   cudaStream_t s = (cudaStream_t)stream;
   const int g = bce_dice_grid(npix);
   const bool vec = bce_dice_vec(logits, target, tgt_dtype, glogits);
-#define GO(T, TT)                                                                                               \
-  bce_dice_bwd_kernel<T, TT><<<g, 256, 0, s>>>((const T*)logits, (const TT*)target, npix, vec, coefs, gscale, \
-                                               (T*)glogits)
-  BCE_DICE_DISPATCH();
-#undef GO
+  with_bce_dice_types(dtype, tgt_dtype, [&](auto t, auto tt) {
+    using T = decltype(t);
+    using TT = decltype(tt);
+    bce_dice_bwd_kernel<T, TT><<<g, 256, 0, s>>>((const T*)logits, (const TT*)target, npix, vec, coefs, gscale,
+                                                 (T*)glogits);
+  });
   UB_LAUNCH_CHECK("bce_dice_bwd");
   return 0;
 }
-#undef BCE_DICE_DISPATCH
 
 int unetb200_dice_fwd(const float* x, const float* t, int64_t G, int64_t L, float epsilon, double* acc, float* out,
                       float* saved, void* stream) {
@@ -594,17 +587,14 @@ int unetb200_boundary_loss(const void* pred, int pred_dtype, int64_t sb, int64_t
   unsigned long long* cnt = (unsigned long long*)work;
   uint32_t* mm = (uint32_t*)((char*)work + 16 * 8);
   int grid = loss_grid((int64_t)B * H * W, 256);
-#define GO(P, TT)                                                                         \
-  do {                                                                                    \
-    BoundaryIO<P, TT> io{(const P*)pred, sb, sh, sw, (const TT*)target, tb, th, tw};      \
-    boundary_counts_kernel<P, TT><<<grid, 256, 0, s>>>(io, g, cnt, mm);                   \
-  } while (0)
-  if (pred_dtype == UNETB200_BF16) {
-    if (tgt_dtype == UNETB200_F32) GO(bf16, float); else GO(bf16, long long);
-  } else {
-    if (tgt_dtype == UNETB200_F32) GO(float, float); else GO(float, long long);
-  }
-#undef GO
+  with_elem(pred_dtype, [&](auto p) {
+    with_type<float, long long>(tgt_dtype, [&](auto tt) {
+      using P = decltype(p);
+      using TT = decltype(tt);
+      BoundaryIO<P, TT> io{(const P*)pred, sb, sh, sw, (const TT*)target, tb, th, tw};
+      boundary_counts_kernel<P, TT><<<grid, 256, 0, s>>>(io, g, cnt, mm);
+    });
+  });
   boundary_finalize_kernel<<<1, 32, 0, s>>>(cnt, mm, g, edge_weight, smooth, out);
   UB_LAUNCH_CHECK("boundary_loss");
   return 0;

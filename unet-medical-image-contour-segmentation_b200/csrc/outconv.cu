@@ -264,7 +264,6 @@ static bool outconv_vec(int C, int64_t ld, const void* p, size_t esz) {
 }  // namespace ub
 
 using namespace ub;
-typedef __nv_bfloat16 bf16;
 
 extern "C" {
 
@@ -277,27 +276,16 @@ int unetb200_outconv_fwd(const void* x, int64_t ld_x, const float* w, const floa
   int blocks = outconv_blocks(npix);
   size_t esz = dtype == UNETB200_BF16 ? 2 : 4;
   size_t smem = sizeof(float) * ((size_t)ncls * C + ncls);
-  if (outconv_vec(C, ld_x, x, esz) && smem <= 48 * 1024) {
-#define UB_OUTCONV_FWD(KK)                                                                                           \
-  case KK:                                                                                                           \
-    if (dtype == UNETB200_BF16)                                                                                      \
-      outconv_fwd_vec_kernel<bf16, KK><<<blocks, 256, smem, s>>>((const bf16*)x, ld_x, w, bias, (bf16*)logits, npix, C, C / 8); \
-    else                                                                                                             \
-      outconv_fwd_vec_kernel<float, KK><<<blocks, 256, smem, s>>>((const float*)x, ld_x, w, bias, (float*)logits, npix, C, C / 8); \
-    break;
-    switch (ncls) {
-      UB_OUTCONV_FWD(1) UB_OUTCONV_FWD(2) UB_OUTCONV_FWD(3) UB_OUTCONV_FWD(4)
-      UB_OUTCONV_FWD(5) UB_OUTCONV_FWD(6) UB_OUTCONV_FWD(7) UB_OUTCONV_FWD(8)
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    if (outconv_vec(C, ld_x, x, esz) && smem <= 48 * 1024) {
+      with_int<1, 2, 3, 4, 5, 6, 7, 8>(ncls, [&](auto KK) {
+        outconv_fwd_vec_kernel<T, KK><<<blocks, 256, smem, s>>>((const T*)x, ld_x, w, bias, (T*)logits, npix, C, C / 8);
+      });
+    } else {
+      outconv_fwd_scalar_kernel<T><<<blocks, 256, 0, s>>>((const T*)x, ld_x, w, bias, (T*)logits, npix, C, ncls);
     }
-#undef UB_OUTCONV_FWD
-  } else {
-    if (dtype == UNETB200_BF16)
-      outconv_fwd_scalar_kernel<bf16><<<blocks, 256, 0, s>>>((const bf16*)x, ld_x, w, bias, (bf16*)logits, npix, C,
-                                                             ncls);
-    else
-      outconv_fwd_scalar_kernel<float><<<blocks, 256, 0, s>>>((const float*)x, ld_x, w, bias, (float*)logits, npix,
-                                                              C, ncls);
-  }
+  });
   UB_LAUNCH_CHECK("outconv_fwd");
   return 0;
 }
@@ -333,34 +321,21 @@ static int outconv_bwd_impl(const void* x, int64_t ld_x, const float* w, const v
   UB_CHECK_ARG(smem_s <= 48 * 1024, "outconv_bwd: n_classes*C too large (%d)", KC);
   bool vec = outconv_bwd_vec_ok(x, ld_x, gx, ld_gx, dtype, C, ncls, bnb);
   UB_CHECK_ARG(!bnb || vec, "outconv_bwd_bnbwd: shape not covered (query _supported first)");
-  if (vec) {
-#define UB_OUTCONV_BWD(KK)                                                                                           \
-  case KK:                                                                                                           \
-    if (dtype == UNETB200_BF16) {                                                                                    \
-      if (bnb) outconv_bwd_vec_kernel<bf16, KK, true><<<blocks, 256, smem_v, s>>>((const bf16*)x, ld_x, w, (const bf16*)glogits, (bf16*)gx, \
-                                                                   ld_gx, workspace, npix, C, C / 8, (const bf16*)yprev, ld_y, bnc); \
-      else outconv_bwd_vec_kernel<bf16, KK, false><<<blocks, 256, smem_v, s>>>((const bf16*)x, ld_x, w, (const bf16*)glogits, (bf16*)gx, \
-                                                                   ld_gx, workspace, npix, C, C / 8, nullptr, 0, nullptr); \
-    } else {                                                                                                         \
-      if (bnb) outconv_bwd_vec_kernel<float, KK, true><<<blocks, 256, smem_v, s>>>((const float*)x, ld_x, w, (const float*)glogits,  \
-                                                                    (float*)gx, ld_gx, workspace, npix, C, C / 8, (const float*)yprev, ld_y, bnc); \
-      else outconv_bwd_vec_kernel<float, KK, false><<<blocks, 256, smem_v, s>>>((const float*)x, ld_x, w, (const float*)glogits,  \
-                                                                    (float*)gx, ld_gx, workspace, npix, C, C / 8, nullptr, 0, nullptr); \
-    }                                                                                                                \
-    break;
-    switch (ncls) {
-      UB_OUTCONV_BWD(1) UB_OUTCONV_BWD(2) UB_OUTCONV_BWD(3) UB_OUTCONV_BWD(4)
-      UB_OUTCONV_BWD(5) UB_OUTCONV_BWD(6) UB_OUTCONV_BWD(7) UB_OUTCONV_BWD(8)
+  with_elem(dtype, [&](auto t) {
+    using T = decltype(t);
+    if (vec) {
+      with_int<1, 2, 3, 4, 5, 6, 7, 8>(ncls, [&](auto KK) {
+        with_bool(bnb, [&](auto BNB) {
+          outconv_bwd_vec_kernel<T, KK, BNB><<<blocks, 256, smem_v, s>>>((const T*)x, ld_x, w, (const T*)glogits,
+                                                                         (T*)gx, ld_gx, workspace, npix, C, C / 8,
+                                                                         (const T*)yprev, ld_y, bnc);
+        });
+      });
+    } else {
+      outconv_bwd_scalar_kernel<T><<<blocks, 256, smem_s, s>>>((const T*)x, ld_x, w, (const T*)glogits, (T*)gx, ld_gx,
+                                                               workspace, npix, C, ncls);
     }
-#undef UB_OUTCONV_BWD
-  } else {
-    if (dtype == UNETB200_BF16)
-      outconv_bwd_scalar_kernel<bf16><<<blocks, 256, smem_s, s>>>((const bf16*)x, ld_x, w, (const bf16*)glogits,
-                                                                  (bf16*)gx, ld_gx, workspace, npix, C, ncls);
-    else
-      outconv_bwd_scalar_kernel<float><<<blocks, 256, smem_s, s>>>((const float*)x, ld_x, w, (const float*)glogits,
-                                                                   (float*)gx, ld_gx, workspace, npix, C, ncls);
-  }
+  });
   outconv_reduce_kernel<<<(KC + ncls + extra + 7) / 8, 256, 0, s>>>(workspace, blocks, KC, ncls, extra, dw, dbias, sums);
   UB_LAUNCH_CHECK("outconv_bwd");
   return 0;
