@@ -74,7 +74,10 @@ __global__ void __launch_bounds__(kHtThreads, HaloTCfg<C1, CUP>::CTAS) halo_t_fp
     if (co < p.cup_real) v = *reinterpret_cast<const uint4*>(p.wp + (size_t)(q * p.cup_real + co) * C1 + c * 8);
     *reinterpret_cast<uint4*>(b_tile + n * P + ((c ^ ((addr >> 7) & CMASK)) << 4)) = v;
   }
-  if (threadIdx.x < 64) sbias[threadIdx.x] = (p.bias && threadIdx.x < p.cup_real) ? p.bias[threadIdx.x] : 0.f;
+  // the bias in the storage dtype, as the other engines add it (conv_tc2.cu, conv_simt.cu) and as autocast's bf16
+  // ConvTranspose2d does
+  if (threadIdx.x < 64)
+    sbias[threadIdx.x] = (p.bias && threadIdx.x < p.cup_real) ? Elem<__nv_bfloat16>::round(p.bias[threadIdx.x]) : 0.f;
   fence_async_smem();
   tc_fence_before();
   __syncthreads();
